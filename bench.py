@@ -65,6 +65,28 @@ def synthetic_crowd(N, M=2000, seed=666, rho=0.5):
     return p.float(), v.float(), ds.float(), dest.float(), obs.float()
 
 
+DUMP_BYTES = 64 << 20
+NPY_HEADER_BYTES = 4096        # per file; a .npy header is 128 bytes for these shapes
+
+
+def dump_outputs(out_dir, arrays):
+    """Write arrays that share their leading (agent) dimension as <out_dir>/<name>.npy in float32, for comparing two
+    builds output for output.  Above 64 MB on disk in all, every array keeps the same seeded sample of agents, whose
+    indices go to rows.npy (float64)."""
+    import numpy as np
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    n = len(next(iter(host.values())))
+    total = sum(x.nbytes for x in host.values())
+    if total + len(host) * NPY_HEADER_BYTES > DUMP_BYTES:
+        budget = DUMP_BYTES - (len(host) + 1) * NPY_HEADER_BYTES
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // (total // n + 8), replace=False))
+        host = {k: x[rows] for k, x in host.items()}
+        host["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, x in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), x)
+
+
 class ClockSampler(threading.Thread):
     """nvidia-smi clocks / throttle reasons sampled DURING the timed region (B200_PROFILING.md recipe)."""
     Q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
@@ -1023,6 +1045,8 @@ def run_ours(a):
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
+        if a.dump_outputs:
+            raise SystemExit("--dump-outputs runs on one GPU")
         dist.init_process_group("nccl", device_id=dev)
     N = a.agents
     if N % world:
@@ -1053,9 +1077,11 @@ def run_ours(a):
             if int(ok) == 0 and crowd is not None:
                 crowd, exchange, exchange_note = None, "nccl", "push unavailable on another rank"
 
+    arrived = None
+
     def advance_step():
         """One step incl. the exchange; returns nothing (state is updated in place / swapped)."""
-        nonlocal pos, vel, pos_next, vel_next
+        nonlocal pos, vel, pos_next, vel_next, arrived
         if crowd is not None:
             crowd.step(model, ds, dest, DT, RADIUS)
             return
@@ -1111,6 +1137,8 @@ def run_ours(a):
         dist.all_reduce(lo, op=dist.ReduceOp.MIN)
         dist.all_reduce(hi, op=dist.ReduceOp.MAX)
         assert float(hi - lo) == 0.0, "ranks disagree on the crowd state after the exchange"
+    if a.dump_outputs:                  # one GPU: pos / vel are what the last timed MLAPM.advance returned
+        dump_outputs(a.dump_outputs, {"action": vel, "new_position": pos, "arrived": arrived})
 
     # ---- end-to-end through the public host-buffer API ------------------------------------------------------------
     act_h = torch.empty(shard, 2).pin_memory()
@@ -1259,7 +1287,15 @@ def main():
     ap.add_argument("--no-config5", action="store_true", help="skip the crowd_1m / scenes_4096 blocks")
     ap.add_argument("--exchange", default="push", choices=["push", "nccl"],
                     help="multi-GPU exchange: fused peer-memory push (default) or NCCL all-gather")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (action, new_position, arrived) "
+                         "as DIR/<name>.npy; inputs are seeded, so runs with the same arguments compare output for "
+                         "output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "mlapm"):
+        ap.error("--dump-outputs applies to the default workload (--impl ours --workload mlapm)")
     if a.impl == "reference":
         run_reference(a)
     elif a.workload == "nn":

@@ -1,6 +1,6 @@
-"""Generate the committed golden vectors by running the UNMODIFIED reference (imported from /root/reference).
+"""Generate the committed golden vectors by running the UNMODIFIED reference (located by tests/golden/_refharness.py).
 
-Run in the build container only:   python tests/golden/make_golden.py [group ...]
+    PIML_REFERENCE=<upstream PIML checkout> python tests/golden/make_golden.py [group ...]
 Groups: features models mlapm sfm rollout sfm_rollout training metrics losses.   Output: tests/golden/*.npz (small, compressed).
 
 The reference ships no tests and no golden vectors (SURVEY.md section 4 / 8c), so these files ARE the pin: they

@@ -28,10 +28,9 @@ def test_library_loads_and_exports_every_declared_symbol():
     assert _lib.launch_count() >= 0
 
 
-def test_no_cpu_fallback():
+def test_no_cpu_fallback(monkeypatch):
     import piml_b200 as P
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)      # a machine without a GPU, also on a GPU box
     x = torch.zeros(1, 4, 2)
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         P.Pedestrians().get_relative_features(x, x.clone(), x.clone(), x, torch.zeros(2, 2), 6, 90, 4, 10, 90, 4)

@@ -5,7 +5,7 @@ import pytest
 import torch
 
 from tests.golden_args import base_args, model_args
-from tests.util import golden, group
+from tests.util import golden, group, reference_available
 
 
 def test_cos_threshold_matches_reference_constant():
@@ -65,7 +65,7 @@ def test_spec_from_module_matches_spec_from_args():
             assert getattr(s1, f) == getattr(s2, f), (kind, f)
 
 
-@pytest.mark.skipif(not __import__("os").path.isdir("/root/reference/src"), reason="reference tree not present")
+@pytest.mark.skipif(not reference_available(), reason="reference tree not present")
 @pytest.mark.parametrize("layers", [16, 3, 1])
 def test_train_mode_dropout_masks_follow_the_reference_rng_stream(layers):
     """ResDNN.forward draws one Dropout mask per block and applies only the last (model.py:115-119).  Under the same
@@ -99,6 +99,23 @@ def test_train_mode_dropout_masks_follow_the_reference_rng_stream(layers):
     assert torch.equal(dp[ok_p], want_p[ok_p]) and torch.equal(do[ok_o], want_o[ok_o])
     assert ok_p.float().mean() > 0.9
     assert torch.equal(after, after_ref)
+
+
+@pytest.mark.parametrize("case,kind", [("pinnsf_bm_train", "pinnsf_bm"), ("pinnsf_m_train", "pinnsf_m")])
+def test_train_mode_dropout_masks_equal_the_recorded_reference_masks(case, kind):
+    """The same draw as above against the masks the reference module applied in train() mode (training_step.npz,
+    16 processor blocks; make_golden.py seeds torch with 666 + 1 right before that forward)."""
+    from piml_b200 import models as M
+    from tests.test_training_ref import drop_masks
+    z = golden("training_step")
+    g = group(z, case)
+    spec = M.spec_from_args(kind, base_args(model=kind, dataset_name=str(g["dataset_name"])))
+    assert spec.n_blocks == 16
+    ped, obs = torch.from_numpy(z["ped"]), torch.from_numpy(z["obs"])
+    torch.manual_seed(667)
+    dp, do = M._dropout_multipliers(spec, True, ped, obs)
+    want_p, want_o = drop_masks(g)
+    assert torch.equal(dp, want_p) and torch.equal(do, want_o)
 
 
 def test_non_relu_single_block_processor_is_rejected():

@@ -1,6 +1,6 @@
-"""Build-container only (skipped where /root/reference is absent, e.g. on the GPU box): the oracle against the
-UNMODIFIED reference imported live, on EVERY frame of the reference's own clips (SURVEY.md A.2b: toy, GC 1000-1060,
-synthetic 1560-1620, UCY 0-54) -- the committed golden vectors hold a subset of these frames."""
+"""Runs where the upstream source tree is available (tests.util.reference_available, skipped elsewhere): the oracle
+against the UNMODIFIED reference imported live, on EVERY frame of the reference's own clips (SURVEY.md A.2b: toy,
+GC 1000-1060, synthetic 1560-1620, UCY 0-54) -- the committed golden vectors hold a subset of these frames."""
 import os
 import sys
 
@@ -9,9 +9,9 @@ import pytest
 import torch
 
 from oracle import oracle as O
-from tests.util import valid_sets
+from tests.util import reference_available, valid_sets
 
-HAVE_REF = os.path.isdir("/root/reference/src")
+HAVE_REF = reference_available()
 pytestmark = pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
 
 

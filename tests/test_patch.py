@@ -4,6 +4,8 @@ import types
 
 import pytest
 
+from tests.util import reference_available
+
 
 def _fake_reference():
     DATA = types.ModuleType("data.data")
@@ -74,7 +76,7 @@ def test_install_swaps_and_uninstall_restores(monkeypatch):
     assert not hasattr(DATA.Pedestrians, "_relative_features_raw")       # helper added by install is removed again
 
 
-@pytest.mark.skipif(not __import__("os").path.isdir("/root/reference/src"), reason="reference tree not present")
+@pytest.mark.skipif(not reference_available(), reason="reference tree not present")
 def test_install_on_the_real_reference_modules():
     """In the build container: the real reference modules expose exactly the attributes the patch replaces."""
     import os
