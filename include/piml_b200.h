@@ -180,11 +180,21 @@ PIML_API int piml_mlapm_advance_f32(const float *pos, const float *vel, const fl
 /* piml_mlapm_advance_f32 with the size of the caller's workspace stated.  With workspace_bytes >=
  * piml_mlapm_workspace_bytes_sym(N) and the whole crowd (row0 = 0, row1 = N) the library may evaluate every UNORDERED
  * pair once for both rows (the smooth part of mlapm.py:25-39 is symmetric under n <-> m; the two gates keep the
- * reference's exact fp32 arithmetic in both directions), which needs room for the column-direction sums
- * (N * N / 64 bytes).  Same results to fp32 summation order (row sums are added in a different, still fixed order).
- * piml_set_mlapm_algorithm: 0 = automatic (symmetric from 16 384 agents), 1 = ordered pairs, 2 = symmetric. */
+ * reference's exact fp32 arithmetic in both directions), which needs room for per-agent fixed-point sums, a spatial
+ * sort of the crowd and a work list (O(N + (N/512)^2) bytes).  The symmetric path skips every pair farther apart than
+ * piml_mlapm_cull_radius, where the fp32 weight is exactly 0.  Same results to fp32 summation order.
+ * piml_set_mlapm_algorithm: 0 = automatic (symmetric, culled, from 16 384 agents), 1 = ordered pairs, 2 = symmetric,
+ * culled, 3 = symmetric, dense (every pair, no culling). */
 PIML_API int64_t piml_mlapm_workspace_bytes_sym(int64_t N);
 PIML_API int piml_set_mlapm_algorithm(int algo);
+/* Distance (m) beyond which the production math's weight of a pair is exactly +0 for these parameters:
+ * (127 + |C log2 e|) / -(B + |D|) log2 e for 'GC', 127 / -(B log2 e) for 'raw' (exp2 of the exponent flushes to 0
+ * below -126), plus 1 % + 0.01 m for approximate rsqrt and fp32 rounding.  +inf where nothing can be skipped:
+ * exact_math, or a weight that does not decay with distance (B + |D| >= 0). */
+PIML_API float piml_mlapm_cull_radius(const piml_mlapm_params *prm);
+/* Diagnostics: the length of the work list (row block x 128-column stage items) that the last culled symmetric step
+ * of N agents built in `workspace`.  Synchronous (waits for the device). */
+PIML_API int piml_mlapm_cull_items(const void *workspace, int64_t N, int64_t *items);
 PIML_API int piml_mlapm_advance_ws_f32(const float *pos, const float *vel, const float *desired_speed, int ds_dim,
                               const float *dest, int64_t N, int64_t row0, int64_t row1,
                               const piml_mlapm_params *prm, float dt, float radius, float *action, float *pos_new,

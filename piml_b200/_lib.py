@@ -85,6 +85,8 @@ SIGNATURES = {
                                      vp, vp, vp]),
     "piml_mlapm_workspace_bytes_sym": (i64, [i64]),
     "piml_set_mlapm_algorithm": (i32, [i32]),
+    "piml_mlapm_cull_radius": (f32, [C.POINTER(MlapmParams)]),
+    "piml_mlapm_cull_items": (i32, [vp, i64, C.POINTER(i64)]),
     "piml_mlapm_advance_ws_f32": (i32, [vp, vp, vp, i32, vp, i64, i64, i64, C.POINTER(MlapmParams), f32, f32, vp, vp,
                                         vp, vp, i64, vp]),
     "piml_scatter_rows_push_f32": (i32, [vp, vp, vp, i64, i64, i32, vp, vp, vp, vp]),

@@ -1,4 +1,8 @@
-// mlapm.cu -- dense all-pairs MLAPM force for sm_100a.
+// mlapm.cu -- all-pairs MLAPM force for sm_100a.
+//
+// The whole-crowd production path (mlapm_sym_list_kernel) evaluates every unordered pair once and skips the pairs
+// farther apart than the radius where the fp32 weight is exactly 0 (a spatial sort, boxes per block and a work list
+// built on the device); the dense kernels below evaluate every pair (row ranges, small crowds, validation).
 //
 // Replaces MLAPM.step (reference src/models/mlapm.py:10-58) and the loop body of src/main_mlapm.py:19-34.
 // The reference materialises (N,N,2)x4 + (N,N,2,2) + (N,N)x6 temporaries (~100 B per ordered pair); here each thread
@@ -13,9 +17,14 @@
 //   EXACT: IEEE div / sqrt / expf in the reference's operation order (validation variant)
 //   fast : rsqrt.approx + ex2.approx, shared 1/r, constant-angle rotation folded into two FMAs (production)
 #include <math_constants.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
+
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_select.cuh>
+#include <cub/iterator/counting_input_iterator.cuh>
 
 #include "common.cuh"
 
@@ -449,11 +458,12 @@ struct MsSmem {
 // far away (their weight underflows to exactly 0 in both directions), so block tails need no masks.
 __global__ void mlapm_prep_sym_kernel(const float2 *__restrict__ pos, const float2 *__restrict__ vel,
                                       const float2 *__restrict__ dest, int N, int Npad, float4 *__restrict__ rec,
-                                      ulonglong2 *__restrict__ colsum) {
+                                      ulonglong2 *__restrict__ colsum, unsigned *__restrict__ bad) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= Npad) return;
     colsum[2 * j] = make_ulonglong2(0ull, 0ull);                   // this step's column-direction accumulators
     colsum[2 * j + 1] = make_ulonglong2(0ull, 0ull);
+    if (bad) bad[j] = 0u;
     if (j >= N) {
         rec[2 * j] = make_float4(MS_FAR, MS_FAR, 0.f, 0.f);
         rec[2 * j + 1] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -531,7 +541,7 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
                                                                          int I0, int per, int sub, M2Const k,
                                                                          float4 *__restrict__ partialR, int nrows_pad,
                                                                          unsigned long long *__restrict__ colsum,
-                                                                         float colscale) {
+                                                                         float colscale, unsigned *__restrict__ bad) {
     constexpr int THREADS = MS_BLOCK / (2 * RPS);
     static_assert(MS_BLOCK % CT == 0 && CT % BATCH == 0 && (BATCH == 8 || BATCH == 4), "bad stage shape");
     constexpr int SPB = MS_BLOCK / CT;                      // stages per block pair
@@ -655,6 +665,8 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
                     const float4 t = sm.colacc[wv][c];
                     a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
                 }
+                // a NaN or inf has no fixed-point value: it poisons the agent through its flag (see SymPartials)
+                if (bad && !isfinite(a.x + a.y + a.z + a.w)) bad[(dst - colsum) / 4 + c] = 1u;
                 atomicAdd(dst + c * 4 + 0, static_cast<unsigned long long>(__float2ll_rn(a.x * colscale)));
                 atomicAdd(dst + c * 4 + 1, static_cast<unsigned long long>(__float2ll_rn(a.y * colscale)));
                 atomicAdd(dst + c * 4 + 2, static_cast<unsigned long long>(__float2ll_rn(a.z * colscale)));
@@ -671,6 +683,308 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
     }
 }
 
+// =====================================================================================================================
+// Culled symmetric evaluation: skip the block pairs whose weight is exactly zero.
+//
+// The production weight is ex2.approx.ftz(arg) / r with arg = Bl r + q (Cl / r + Dl), |q| <= r, so arg <= (Bl + |Dl|) r
+// + |Cl| (raw: arg = Bl r).  sym_params_ok requires Bl + |Dl| < 0, so beyond r_cut = (127 + |Cl|) / -(Bl + |Dl|) every
+// pair has arg < -127: ex2 flushes to +0, every fma(w, r, S) returns S unchanged and every fixed-point column share is
+// 0.  Skipping those pairs changes nothing but the fp32 summation order.
+//
+// Per call: (1) a 32-bit Hilbert key of each agent's 4 m cell, sorted stably (cub::DeviceRadixSort, key + agent
+// index), so that the agents of a 512-block live close together; (2) records in sorted order plus an axis-aligned box
+// per 512-agent block and per 128-agent column stage; (3) the work list: every (row block I, column block J = I + d
+// mod T, stage) item of the circulant schedule whose boxes are within r_cut, compacted in order (cub::DeviceSelect);
+// (4) a persistent pair kernel over the list; (5) the finalize kernel reads each agent's sums through its sorted slot.
+// Row and column directions both go into the crowd-wide int64 fixed-point accumulators, so the result does not depend
+// on how the list is cut over the CTAs.
+// =====================================================================================================================
+constexpr float MC_CELL = 4.0f;                   // metres per cell of the sort key
+constexpr int MC_SPB = MS_BLOCK / MS_CT;          // column stages per block
+constexpr int MC_THREADS = 64;                    // pair kernel: 8 rows per thread (the dense kernel's measured best)
+constexpr unsigned MC_NEAR_ALL = 1u, MC_EMPTY = 2u;   // box flags: holds a NaN / inf, holds no agent
+
+// Hilbert index of cell (x, y) on the 2^16 x 2^16 grid.
+__device__ __forceinline__ uint32_t hilbert16(uint32_t x, uint32_t y) {
+    uint32_t d = 0;
+    for (uint32_t s = 1u << 15; s > 0; s >>= 1) {
+        const uint32_t rx = (x & s) ? 1u : 0u, ry = (y & s) ? 1u : 0u;
+        d += s * s * ((3u * rx) ^ ry);
+        if (ry == 0) {
+            if (rx == 1) { x = 0xFFFFu - x; y = 0xFFFFu - y; }
+            const uint32_t t = x; x = y; y = t;
+        }
+    }
+    return d;
+}
+
+// key[n] = Hilbert index of floor(p_n / MC_CELL) (cell coordinates wrap modulo 2^16: only locality is lost), agent
+// index as the value; a non-finite position sorts last.
+__global__ void mlapm_cull_keys_kernel(const float2 *__restrict__ pos, int N, uint32_t *__restrict__ key,
+                                       int *__restrict__ val) {
+    const int n = blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    const float2 p = pos[n];
+    uint32_t k = 0xFFFFFFFFu;
+    if (isfinite(p.x) && isfinite(p.y)) {
+        const uint32_t cx = static_cast<uint32_t>(__float2int_rd(p.x * (1.0f / MC_CELL))) & 0xFFFFu;
+        const uint32_t cy = static_cast<uint32_t>(__float2int_rd(p.y * (1.0f / MC_CELL))) & 0xFFFFu;
+        k = hilbert16(cx, cy);
+    }
+    key[n] = k;
+    val[n] = n;
+}
+
+// One CTA of MS_BLOCK threads per block of the sorted crowd: rec[j] for the agent perm[j] (j >= N: far-away padding as
+// in mlapm_prep_sym_kernel), slot[agent] = j, zeroed accumulators, and the boxes {min x, min y, max x, max y} of the
+// block and of its MC_SPB column stages.  Agents with a non-finite position or velocity do not enter the min / max (no
+// fminf / fmaxf on NaN); they flag their stage and block MC_NEAR_ALL instead, which keeps every item that touches them.
+__global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
+    const float2 *__restrict__ pos, const float2 *__restrict__ vel, const float2 *__restrict__ dest,
+    const int *__restrict__ perm, int N, float4 *__restrict__ rec, int *__restrict__ slot,
+    ulonglong2 *__restrict__ acc, unsigned *__restrict__ bad, float4 *__restrict__ sbox, unsigned *__restrict__ sflag,
+    float4 *__restrict__ bbox, unsigned *__restrict__ bflag) {
+    __shared__ float4 wbox[MS_BLOCK / 32];
+    __shared__ unsigned wflag[MS_BLOCK / 32];
+    const int j = blockIdx.x * MS_BLOCK + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    acc[2 * j] = make_ulonglong2(0ull, 0ull);
+    acc[2 * j + 1] = make_ulonglong2(0ull, 0ull);
+    bad[j] = 0u;
+    float4 b = make_float4(CUDART_INF_F, CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F);
+    unsigned flag = MC_EMPTY;
+    if (j < N) {
+        const int n = perm[j];
+        slot[n] = j;
+        const float2 p = pos[n], v = vel[n], d = dest[n];
+        const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
+        const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
+        rec[2 * j] = make_float4(p.x, p.y, v.x, v.y);
+        rec[2 * j + 1] = make_float4(__fdiv_rn(dx, dn), __fdiv_rn(dy, dn), 0.f, 0.f);
+        if (isfinite(p.x) && isfinite(p.y) && isfinite(v.x) && isfinite(v.y)) {
+            b = make_float4(p.x, p.y, p.x, p.y);
+            flag = 0u;
+        } else {
+            flag = MC_NEAR_ALL;
+        }
+    } else {
+        rec[2 * j] = make_float4(MS_FAR, MS_FAR, 0.f, 0.f);
+        rec[2 * j + 1] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    // flags combine as: any MC_NEAR_ALL -> MC_NEAR_ALL, else any agent -> 0, else MC_EMPTY
+    auto comb = [](unsigned a, unsigned c) { return (a | c) & MC_NEAR_ALL ? MC_NEAR_ALL : (a & c); };
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        b.x = fminf(b.x, __shfl_xor_sync(0xffffffffu, b.x, o));
+        b.y = fminf(b.y, __shfl_xor_sync(0xffffffffu, b.y, o));
+        b.z = fmaxf(b.z, __shfl_xor_sync(0xffffffffu, b.z, o));
+        b.w = fmaxf(b.w, __shfl_xor_sync(0xffffffffu, b.w, o));
+        flag = comb(flag, __shfl_xor_sync(0xffffffffu, flag, o));
+    }
+    if (lane == 0) { wbox[warp] = b; wflag[warp] = flag; }
+    __syncthreads();
+    if (threadIdx.x < MC_SPB + 1) {
+        // thread s < MC_SPB: stage s (its MS_CT / 32 warps); thread MC_SPB: the whole block
+        const int w0 = threadIdx.x < MC_SPB ? threadIdx.x * (MS_CT / 32) : 0;
+        const int w1 = threadIdx.x < MC_SPB ? w0 + MS_CT / 32 : MS_BLOCK / 32;
+        float4 u = wbox[w0];
+        unsigned f = wflag[w0];
+        for (int w = w0 + 1; w < w1; ++w) {
+            const float4 t = wbox[w];
+            u.x = fminf(u.x, t.x); u.y = fminf(u.y, t.y); u.z = fmaxf(u.z, t.z); u.w = fmaxf(u.w, t.w);
+            f = comb(f, wflag[w]);
+        }
+        if (threadIdx.x < MC_SPB) {
+            sbox[blockIdx.x * MC_SPB + threadIdx.x] = u;
+            sflag[blockIdx.x * MC_SPB + threadIdx.x] = f;
+        } else {
+            bbox[blockIdx.x] = u;
+            bflag[blockIdx.x] = f;
+        }
+    }
+}
+
+// Keep-predicate of the work list over candidate c = ((I * (D + 1) + d) * MC_SPB + stage): rows = block I, columns =
+// stage `stage` of block J = I + d mod T (circulant schedule of mlapm_sym_kernel).  The box gap is rounded down, so a
+// kept-or-not decision never depends on fp32 rounding in the skipping direction.
+struct CullKeep {
+    const float4 *sbox, *bbox;
+    const unsigned *sflag, *bflag;
+    int T, D;
+    float rc;
+    __device__ __forceinline__ bool operator()(int c) const {
+        const int st = c % MC_SPB, pd = c / MC_SPB;
+        const int I = pd / (D + 1), d = pd - I * (D + 1);
+        if (!(T & 1) && d == D && 2 * I >= T) return false;     // even T: the pairs at d = T/2 belong to I < T/2
+        int J = I + d;
+        J = J >= T ? J - T : J;
+        const int s = J * MC_SPB + st;
+        const unsigned fr = bflag[I], fc = sflag[s];
+        if ((fr | fc) & MC_EMPTY) return false;
+        if ((fr | fc) & MC_NEAR_ALL) return true;
+        const float4 a = bbox[I], b = sbox[s];
+        const float gx = fmaxf(fmaxf(__fsub_rd(b.x, a.z), __fsub_rd(a.x, b.z)), 0.f);
+        const float gy = fmaxf(fmaxf(__fsub_rd(b.y, a.w), __fsub_rd(a.y, b.w)), 0.f);
+        return __fadd_rd(__fmul_rd(gx, gx), __fmul_rd(gy, gy)) <= rc * rc;
+    }
+};
+
+// The symmetric pair kernel over the work list.  Persistent: CTA b takes the contiguous items [b n / G, (b+1) n / G)
+// of the n = *nitems on the list (read on the device: no host sync).  Rows stay in registers while consecutive items
+// share the row block; when it changes, and at the end, the row sums go into the fixed-point accumulators with the
+// opposite sign of the column shares (acc = column share - row share; the finalize kernel subtracts acc).  Stage loads
+// (TMA, double buffered), the pair math (pair2 on the diagonal, pair2sym elsewhere) and the warp column reduction are
+// those of mlapm_sym_kernel.
+template <int VERSION>
+__global__ void __launch_bounds__(MC_THREADS, 8) mlapm_sym_list_kernel(const float4 *__restrict__ rec,
+                                                                      const int *__restrict__ items,
+                                                                      const int *__restrict__ nitems, int T, int D,
+                                                                      M2Const k, unsigned long long *__restrict__ acc,
+                                                                      unsigned *__restrict__ bad, float colscale) {
+    constexpr int THREADS = MC_THREADS, RPS = MS_BLOCK / (2 * THREADS), CT = MS_CT, BATCH = MS_BATCH;
+    constexpr int LPC = 32 / BATCH;
+    extern __shared__ __align__(128) unsigned char ms_smem_raw[];
+    MsSmem<CT, BATCH, THREADS> &sm = *reinterpret_cast<MsSmem<CT, BATCH, THREADS> *>(ms_smem_raw);
+    // the item of the stage in tile[buf] (I, d, first column j0 = J * MS_BLOCK + stage * CT), written by the thread
+    // that issues its copy; the loop state lives here too, which keeps the pair loop at 128 registers without spills
+    __shared__ int meta[2][3];
+    __shared__ int s_lo, s_cnt;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int n = *nitems;
+    const int lo = static_cast<int>(static_cast<int64_t>(n) * blockIdx.x / gridDim.x);
+    const int cnt = static_cast<int>(static_cast<int64_t>(n) * (blockIdx.x + 1) / gridDim.x) - lo;
+    if (cnt <= 0) return;
+    constexpr uint32_t STAGE_BYTES = CT * MS_RECF * sizeof(float);
+    auto stage_load = [&](int s, int buf) {                    // thread 0
+        const int c = items[s];
+        const int st = c % MC_SPB, pd = c / MC_SPB;
+        const int I = pd / (D + 1), d = pd - I * (D + 1);
+        const int J = I + d >= T ? I + d - T : I + d;
+        const int j0 = J * MS_BLOCK + st * CT;
+        meta[buf][0] = I; meta[buf][1] = d; meta[buf][2] = j0;
+        mbar_expect_tx(&sm.bars[buf], STAGE_BYTES);
+        tma_bulk_g2s(sm.tile[buf], rec + static_cast<int64_t>(j0) * 2, STAGE_BYTES, &sm.bars[buf]);
+    };
+    if (tid == 0) {
+        mbar_init(&sm.bars[0], 1);
+        mbar_init(&sm.bars[1], 1);
+        mbar_fence_init();
+        s_lo = lo;
+        s_cnt = cnt;
+        stage_load(lo, 0);
+    }
+    __syncthreads();
+
+    float2 npx[RPS], npy[RPS], vx[RPS], vy[RPS], nvx[RPS], nvy[RPS], ex[RPS], ey[RPS], Sx[RPS], Sy[RPS], Tx[RPS],
+        Ty[RPS];
+    const float2 Bl = splat(k.Bl), Cl = splat(k.Cl), Dl = splat(k.Dl);
+    auto flush_rows = [&](int I) {
+#pragma unroll
+        for (int i = 0; i < RPS; ++i) {
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                const int64_t j = static_cast<int64_t>(I) * MS_BLOCK + (2 * i + h) * THREADS + tid;
+                const float a0 = h ? Sx[i].y : Sx[i].x, a1 = h ? Sy[i].y : Sy[i].x;
+                const float a2 = h ? Tx[i].y : Tx[i].x, a3 = h ? Ty[i].y : Ty[i].x;
+                if (!isfinite(a0 + a1 + a2 + a3)) bad[j] = 1u;
+                unsigned long long *dst = acc + j * 4;
+                atomicAdd(dst + 0, static_cast<unsigned long long>(__float2ll_rn(-a0 * colscale)));
+                atomicAdd(dst + 1, static_cast<unsigned long long>(__float2ll_rn(-a1 * colscale)));
+                atomicAdd(dst + 2, static_cast<unsigned long long>(__float2ll_rn(-a2 * colscale)));
+                atomicAdd(dst + 3, static_cast<unsigned long long>(__float2ll_rn(-a3 * colscale)));
+            }
+        }
+    };
+
+    // runs of consecutive items with the same row block: rows loaded once per run, row sums flushed at its end.
+    // meta[t & 1] was written before the barrier that ended item t - 1 and is rewritten only after item t's.
+    int t = 0;
+    while (t < s_cnt) {
+        const int I = meta[t & 1][0];
+#pragma unroll
+        for (int i = 0; i < RPS; ++i) {
+            const int64_t na = static_cast<int64_t>(I) * MS_BLOCK + (2 * i) * THREADS + tid;
+            const int64_t nb = na + THREADS;
+            const float4 a0 = rec[2 * na], a1 = rec[2 * na + 1], b0 = rec[2 * nb], b1 = rec[2 * nb + 1];
+            npx[i] = make_float2(-a0.x, -b0.x); npy[i] = make_float2(-a0.y, -b0.y);
+            vx[i] = make_float2(a0.z, b0.z); vy[i] = make_float2(a0.w, b0.w);
+            nvx[i] = make_float2(-a0.z, -b0.z); nvy[i] = make_float2(-a0.w, -b0.w);
+            ex[i] = make_float2(a1.x, b1.x); ey[i] = make_float2(a1.y, b1.y);
+            Sx[i] = Sy[i] = Tx[i] = Ty[i] = make_float2(0.f, 0.f);
+        }
+        do {
+        const int buf = t & 1;
+        if (tid == 0 && t + 1 < s_cnt) stage_load(s_lo + t + 1, buf ^ 1);   // tile[buf^1] was released by the
+        mbar_wait(&sm.bars[buf], (t >> 1) & 1);                   // the (t/2)-th use of this buffer
+        const float4 *tl = sm.tile[buf];
+        if (meta[buf][1] == 0) {
+            // diagonal block: rows and columns are the same agents, every ordered pair appears -> row direction only
+#pragma unroll 4
+            for (int j = 0; j < CT; ++j) {
+                const float4 cp = tl[2 * j];
+#pragma unroll
+                for (int i = 0; i < RPS; ++i)
+                    pair2<VERSION>(npx[i], npy[i], vx[i], vy[i], nvx[i], nvy[i], ex[i], ey[i], cp, Bl, Cl, Dl, Sx[i],
+                                   Sy[i], Tx[i], Ty[i]);
+            }
+        } else {
+            float4 *red = sm.red[warp];
+            for (int b = 0; b < CT / BATCH; ++b) {
+#pragma unroll
+                for (int c = 0; c < BATCH; ++c) {
+                    const float4 cp = tl[2 * (b * BATCH + c)];
+                    const float4 ce = tl[2 * (b * BATCH + c) + 1];
+                    float2 cSx, cSy, cTx, cTy;
+                    pair2sym<VERSION, true>(npx[0], npy[0], vx[0], vy[0], nvx[0], nvy[0], ex[0], ey[0], cp, ce, Bl, Cl,
+                                            Dl, Sx[0], Sy[0], Tx[0], Ty[0], cSx, cSy, cTx, cTy);
+#pragma unroll
+                    for (int i = 1; i < RPS; ++i)
+                        pair2sym<VERSION, false>(npx[i], npy[i], vx[i], vy[i], nvx[i], nvy[i], ex[i], ey[i], cp, ce,
+                                                 Bl, Cl, Dl, Sx[i], Sy[i], Tx[i], Ty[i], cSx, cSy, cTx, cTy);
+                    red[c * MS_RED_STRIDE + lane] = make_float4(cSx.x + cSx.y, cSy.x + cSy.y, cTx.x + cTx.y,
+                                                                cTy.x + cTy.y);
+                }
+                __syncwarp();
+                const float4 *col = red + (lane / LPC) * MS_RED_STRIDE + (lane % LPC);
+                float4 a = col[0];
+#pragma unroll
+                for (int e = 1; e < 32 / LPC; ++e) {
+                    const float4 t = col[LPC * e];
+                    a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
+                }
+#pragma unroll
+                for (int o = 1; o < LPC; o <<= 1) {
+                    a.x += __shfl_xor_sync(0xffffffffu, a.x, o);
+                    a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
+                    a.z += __shfl_xor_sync(0xffffffffu, a.z, o);
+                    a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
+                }
+                if (lane % LPC == 0) sm.colacc[warp][b * BATCH + lane / LPC] = a;
+                __syncwarp();
+            }
+            __syncthreads();
+            const int64_t j0 = meta[buf][2];
+            for (int c = tid; c < CT; c += THREADS) {
+                float4 a = sm.colacc[0][c];
+#pragma unroll
+                for (int wv = 1; wv < THREADS / 32; ++wv) {
+                    const float4 t = sm.colacc[wv][c];
+                    a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
+                }
+                if (!isfinite(a.x + a.y + a.z + a.w)) bad[j0 + c] = 1u;
+                unsigned long long *dst = acc + (j0 + c) * 4;
+                atomicAdd(dst + 0, static_cast<unsigned long long>(__float2ll_rn(a.x * colscale)));
+                atomicAdd(dst + 1, static_cast<unsigned long long>(__float2ll_rn(a.y * colscale)));
+                atomicAdd(dst + 2, static_cast<unsigned long long>(__float2ll_rn(a.z * colscale)));
+                atomicAdd(dst + 3, static_cast<unsigned long long>(__float2ll_rn(a.w * colscale)));
+            }
+        }
+        __syncthreads();
+        ++t;
+        } while (t < s_cnt && meta[t & 1][0] == I);
+        flush_rows(I);
+    }
+}
+
 // Exchange step of an agent-sharded crowd fused into the finalize kernel: rank g's NEXT-state arrays, mapped into this
 // process over NVLink peer memory.  world == 0: no exchange.
 constexpr int ML_MAX_PEERS = 16;
@@ -679,8 +993,11 @@ struct PeerPush { int world; float2 *pos[ML_MAX_PEERS]; float2 *vel[ML_MAX_PEERS
 // int64 accumulators per agent, value = colsum * inv_colscale.
 // inbox != nullptr (agent-sharded crowd): the column-direction sums were reduced per rank and delivered to the owner
 // of the rows (mlapm_sym_colpush_kernel); inbox[g * inbox_stride + local row] is rank g's share.
+// slot != nullptr (culled evaluation): agent n's accumulators sit at its sorted position slot[n].  bad != nullptr: a
+// flag per accumulator, set where a NaN or inf was added (fixed point has no value for them); the agent's sums then
+// read NaN, as an fp32 sum would.
 struct SymPartials { const long long *colsum; float inv_colscale; int nrows_pad; const float4 *inbox; int world;
-                     int64_t inbox_stride; };
+                     int64_t inbox_stride; const int *slot; const unsigned *bad; };
 // Owners of the 512-agent blocks (rank g owns blocks [Ib[g], Ib[g+1])) and every rank's inbox as mapped here.
 struct PeerInbox { int world, rank; int Ib[ML_MAX_PEERS + 1]; float4 *inbox[ML_MAX_PEERS]; int64_t stride; };
 
@@ -762,13 +1079,16 @@ __global__ void mlapm_finalize2_kernel(const float2 *__restrict__ pos, const flo
     } else if (sym.colsum) {
         // symmetric evaluation: this agent was a COLUMN of T/2 block pairs; their column-direction sums (exact integer
         // total of the per-pair fp32 block sums) enter with the opposite sign (vr[m,n] = -vr[n,m]).
-        const longlong2 c0 = reinterpret_cast<const longlong2 *>(sym.colsum)[2 * n];
-        const longlong2 c1 = reinterpret_cast<const longlong2 *>(sym.colsum)[2 * n + 1];
+        // culled evaluation: the row-direction sums are in the same accumulators, with the opposite sign
+        const int j = sym.slot ? sym.slot[n] : n;
+        const longlong2 c0 = reinterpret_cast<const longlong2 *>(sym.colsum)[2 * j];
+        const longlong2 c1 = reinterpret_cast<const longlong2 *>(sym.colsum)[2 * j + 1];
         const double is = static_cast<double>(sym.inv_colscale);
         s.x -= static_cast<float>(static_cast<double>(c0.x) * is);
         s.y -= static_cast<float>(static_cast<double>(c0.y) * is);
         s.z -= static_cast<float>(static_cast<double>(c1.x) * is);
         s.w -= static_cast<float>(static_cast<double>(c1.y) * is);
+        if (sym.bad && sym.bad[j]) s = make_float4(CUDART_NAN_F, CUDART_NAN_F, CUDART_NAN_F, CUDART_NAN_F);
     }
     float sx, sy;
     if (version == 0) { sx = s.x; sy = s.y; }
@@ -883,7 +1203,7 @@ static void launch_pairs(int R, dim3 grid, cudaStream_t st, const float2 *pos, c
 using namespace piml;
 
 // ---- symmetric evaluation: selection and workspace ------------------------------------------------------------------
-static int g_mlapm_algorithm = 0;                 // 0 automatic, 1 ordered pairs (v2), 2 symmetric (v3)
+static int g_mlapm_algorithm = 0;                 // 0 automatic, 1 ordered pairs (v2), 2 symmetric culled, 3 dense
 constexpr int64_t MS_AUTO_MIN_AGENTS = 16384;     // below this the ordered-pair kernel fills the GPU better
 
 static int64_t sym_blocks(int64_t N) { return (N + MS_BLOCK - 1) / MS_BLOCK; }
@@ -917,14 +1237,67 @@ static int sym_splits(int64_t nI, int64_t T, int *per, int *sub) {
     return static_cast<int>((T / 2 + 1 + *per - 1) / *per) * *sub;
 }
 
-// records (32 B per agent) + row-direction partials (16 B per agent and split) + column-direction fixed-point
-// accumulators (4 x int64 per agent): O(N) -- 0.15 GB at N = 10^6 (the per-pair column partials this replaces: 15.6 GB)
+// Dense symmetric evaluation: records (32 B per agent) + row-direction partials (16 B per agent and split) +
+// column-direction fixed-point accumulators (4 x int64 per agent) + poison flags: O(N) -- 0.15 GB at N = 10^6 (the
+// per-pair column partials this replaces: 15.6 GB)
 static int64_t sym_workspace_bytes(int64_t N) {
     const int64_t T = sym_blocks(N), npad = T * MS_BLOCK;
     int per_, sub_;
     const int64_t S = sym_splits(T, T, &per_, &sub_);
-    return npad * MS_RECF * sizeof(float) + S * npad * 4 * sizeof(float) + npad * 4 * sizeof(long long) + 256;
+    return npad * MS_RECF * sizeof(float) + S * npad * 4 * sizeof(float) + npad * 4 * sizeof(long long) +
+           npad * sizeof(unsigned) + 256;
 }
+
+// Culled symmetric evaluation (mlapm_sym_list_kernel).  Candidates of the work list: T * (floor(T/2) + 1) * MC_SPB,
+// the dense worst case (every item within r_cut); the list index is an int.
+static int64_t cull_candidates(int64_t N) {
+    const int64_t T = sym_blocks(N);
+    return T * (T / 2 + 1) * MC_SPB;
+}
+// Reserved CUB scratch, computable without a device (CUB's own size query needs one).  Radix sort on DoubleBuffers
+// (onesweep): 4 passes x 256 bins of 8 B, and 256 look-back counters of 4 B per tile of >= 256 keys -- at most 4 B
+// per key.  Select: one 16 B tile descriptor per tile of >= 128 candidates -- at most 1 B per candidate.  64 KB for
+// the counters, padding and alignment of both.  The real size is checked against this at every call.
+static int64_t cull_cub_bound(int64_t N) {
+    const int64_t a = 4 * N, b = cull_candidates(N);
+    return (int64_t{1} << 16) + (a > b ? a : b);
+}
+struct CullLayout {
+    float4 *rec; long long *acc; unsigned *bad; uint32_t *key[2]; int *val[2]; int *slot;
+    float4 *sbox, *bbox; unsigned *sflag, *bflag; int *items, *nitems; void *temp; int64_t temp_bytes, total;
+};
+// records, accumulators (4 x int64) and flags per padded agent; keys, values (both double-buffered) and slots per
+// agent; boxes and flags per stage and block; the work list; CUB's scratch.  0.1 GB at N = 10^6.
+static CullLayout cull_layout(int64_t N, void *base) {
+    const int64_t T = sym_blocks(N), npad = T * MS_BLOCK;
+    CullLayout l{};
+    char *p = static_cast<char *>(base);
+    int64_t off = 0;
+    auto take = [&](int64_t bytes) {
+        char *q = p ? p + off : nullptr;
+        off += (bytes + 255) / 256 * 256;
+        return static_cast<void *>(q);
+    };
+    l.rec = static_cast<float4 *>(take(npad * MS_RECF * sizeof(float)));
+    l.acc = static_cast<long long *>(take(npad * 4 * sizeof(long long)));
+    l.bad = static_cast<unsigned *>(take(npad * sizeof(unsigned)));
+    for (int b = 0; b < 2; ++b) {
+        l.key[b] = static_cast<uint32_t *>(take(N * sizeof(uint32_t)));
+        l.val[b] = static_cast<int *>(take(N * sizeof(int)));
+    }
+    l.slot = static_cast<int *>(take(N * sizeof(int)));
+    l.sbox = static_cast<float4 *>(take(T * MC_SPB * sizeof(float4)));
+    l.bbox = static_cast<float4 *>(take(T * sizeof(float4)));
+    l.sflag = static_cast<unsigned *>(take(T * MC_SPB * sizeof(unsigned)));
+    l.bflag = static_cast<unsigned *>(take(T * sizeof(unsigned)));
+    l.items = static_cast<int *>(take(cull_candidates(N) * sizeof(int)));
+    l.nitems = static_cast<int *>(take(sizeof(int)));
+    l.temp_bytes = cull_cub_bound(N);
+    l.temp = take(l.temp_bytes);
+    l.total = off + 256;                                          // + 256: room to align the caller's base
+    return l;
+}
+static int64_t cull_workspace_bytes(int64_t N) { return cull_layout(N, nullptr).total; }
 
 // Fixed-point scale 2^s of the column accumulators: one pair contributes |w r| = exp(arg) <= exp(|C|) (B r + D r cos <= 0
 // is required by sym_params_ok), a column at most N of them; keep two bits of headroom below 2^63.
@@ -935,16 +1308,27 @@ static int sym_colscale_log2(int64_t N, const piml_mlapm_params *prm) {
 }
 
 extern "C" int piml_set_mlapm_algorithm(int algo) {
-    PIML_REQUIRE(algo >= 0 && algo <= 2,
-                 "piml_set_mlapm_algorithm: 0 = automatic, 1 = ordered pairs, 2 = symmetric (unordered pairs)");
+    PIML_REQUIRE(algo >= 0 && algo <= 3,
+                 "piml_set_mlapm_algorithm: 0 = automatic, 1 = ordered pairs, 2 = symmetric (unordered pairs, culled "
+                 "at the radius where the weight is exactly 0), 3 = symmetric, dense (no culling)");
     g_mlapm_algorithm = algo;
     return PIML_OK;
 }
 
 extern "C" int64_t piml_mlapm_workspace_bytes_sym(int64_t N) {
     if (N <= 0) return 0;
-    const int64_t a = piml_mlapm_workspace_bytes(N), b = sym_workspace_bytes(N);
-    return a > b ? a : b;
+    const int64_t a = piml_mlapm_workspace_bytes(N), b = sym_workspace_bytes(N), c = cull_workspace_bytes(N);
+    return a > b ? (a > c ? a : c) : (b > c ? b : c);
+}
+
+extern "C" int piml_mlapm_cull_items(const void *workspace, int64_t N, int64_t *items) {
+    PIML_REQUIRE(workspace && items && N > 0 && N < (1LL << 31), "piml_mlapm_cull_items: bad arguments");
+    const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~static_cast<uintptr_t>(255);
+    const CullLayout l = cull_layout(N, reinterpret_cast<void *>(base));
+    int n = 0;
+    PIML_CUDA(cudaMemcpy(&n, l.nitems, sizeof(int), cudaMemcpyDeviceToHost));
+    *items = n;
+    return PIML_OK;
 }
 
 extern "C" int64_t piml_mlapm_workspace_bytes(int64_t N) {
@@ -975,14 +1359,33 @@ static bool sym_params_ok(const piml_mlapm_params *prm, const MlConst &k, int64_
            sym_colscale_log2(N, prm) >= 30;                        // 2^-30 resolution at the very least (|C| < ~15)
 }
 
+// Distance beyond which every pair's production weight is exactly +0 (see mlapm_sym_list_kernel): arg <= (Bl + |Dl|) r
+// + |Cl| < -127 (raw: Bl r < -127), from the same fp32 constants the kernels use.  The margin (1 % + 0.01 m) covers
+// the rsqrt.approx error in r and q and fp32 rounding of coordinates; ex2.approx.ftz already returns 0 below -126.
+// +inf (no culling) where the symmetric kernels do not run.
+static float cull_radius(const piml_mlapm_params *prm, const MlConst &k) {
+    if (prm->exact_math) return HUGE_VALF;
+    const double slope = prm->version == 0 ? static_cast<double>(k.Bl)
+                                           : static_cast<double>(k.Bl) + fabs(static_cast<double>(k.Dl));
+    if (!(slope < 0.0)) return HUGE_VALF;
+    const double c = prm->version == 0 ? 0.0 : fabs(static_cast<double>(k.Cl));
+    const double r0 = (127.0 + c) / -slope;
+    return static_cast<float>(r0 * 1.01 + 0.01);
+}
+
+extern "C" float piml_mlapm_cull_radius(const piml_mlapm_params *prm) {
+    if (!prm || (prm->version != 0 && prm->version != 1)) return HUGE_VALF;
+    return cull_radius(prm, mlapm_consts(prm));
+}
+
 // prep + symmetric pair kernel for the row blocks [I0, I0 + nI) of a crowd of T blocks.
 static int launch_sym_pairs(int version, const float2 *p2, const float2 *v2, const float2 *d2, int N, int64_t T,
                             int64_t I0, int64_t nI, int per, int sub, int S, const MlConst &k, float4 *rec, float4 *partialR,
-                            long long *colsum, float colscale, cudaStream_t st) {
+                            long long *colsum, float colscale, unsigned *bad, cudaStream_t st) {
     const int64_t D = T / 2, npad = T * MS_BLOCK;
     const int threads = 256;
     mlapm_prep_sym_kernel<<<static_cast<unsigned>((npad + threads - 1) / threads), threads, 0, st>>>(
-        p2, v2, d2, N, static_cast<int>(npad), rec, reinterpret_cast<ulonglong2 *>(colsum));
+        p2, v2, d2, N, static_cast<int>(npad), rec, reinterpret_cast<ulonglong2 *>(colsum), bad);
     count_launch();
     int rc = check_launch("mlapm_prep_sym_kernel");
     if (rc) return rc;
@@ -999,7 +1402,7 @@ static int launch_sym_pairs(int version, const float2 *p2, const float2 *v2, con
                                            static_cast<int>(sizeof(Smem))));                                       \
         mlapm_sym_kernel<V, CT, BATCH, RPS><<<grid, MS_BLOCK / (2 * RPS), sizeof(Smem), st>>>(                     \
             rec, static_cast<int>(T), static_cast<int>(D), static_cast<int>(I0), per, sub, k2, partialR,           \
-            static_cast<int>(nI * MS_BLOCK), reinterpret_cast<unsigned long long *>(colsum), colscale);            \
+            static_cast<int>(nI * MS_BLOCK), reinterpret_cast<unsigned long long *>(colsum), colscale, bad);       \
     } while (0)
     // measured at N = 100k (ms per step): 8 rows per thread (64 threads) 6.81, 4 rows (128 threads) 6.99, 2 rows 7.16
     if (version == 0) PIML_LAUNCH_SYM(0, MS_CT, MS_BATCH, 2);
@@ -1009,6 +1412,75 @@ static int launch_sym_pairs(int version, const float2 *p2, const float2 *v2, con
 #undef PIML_LAUNCH_SYM
     count_launch();
     return check_launch("mlapm_sym_kernel");
+}
+
+// Launches of one CUB radix sort of n 32-bit keys with int values on DoubleBuffers (CUB 2.x, sm_100 policy): one
+// single-tile kernel up to 256 x 19 keys, else histogram + exclusive sum + one onesweep kernel per 8-bit digit.
+static int cub_sort_launches(int64_t n, int bits) { return n <= 256 * 19 ? 1 : 2 + (bits + 7) / 8; }
+
+// Culled symmetric evaluation of the whole crowd: keys, sort, prep + boxes, work list, pair kernel.  The finalize
+// kernel follows in the caller.  No host synchronisation: the list length stays on the device.
+static int launch_sym_culled(int version, const float2 *p2, const float2 *v2, const float2 *d2, int N,
+                             const MlConst &k, float rc, const CullLayout &l, float colscale, cudaStream_t st) {
+    const int64_t T = sym_blocks(N), D = T / 2;
+    const int threads = 256;
+    mlapm_cull_keys_kernel<<<static_cast<unsigned>((N + threads - 1) / threads), threads, 0, st>>>(p2, N, l.key[0],
+                                                                                                     l.val[0]);
+    count_launch();
+    int rc_ = check_launch("mlapm_cull_keys_kernel");
+    if (rc_) return rc_;
+    cub::DoubleBuffer<uint32_t> keys(l.key[0], l.key[1]);
+    cub::DoubleBuffer<int> vals(l.val[0], l.val[1]);
+    size_t need = 0;
+    PIML_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, need, keys, vals, N, 0, 32, st));
+    PIML_REQUIRE(static_cast<int64_t>(need) <= l.temp_bytes,
+                 "piml_mlapm: CUB radix sort needs %lld bytes of scratch, %lld reserved", static_cast<long long>(need),
+                 static_cast<long long>(l.temp_bytes));
+    size_t temp_bytes = static_cast<size_t>(l.temp_bytes);
+    PIML_CUDA(cub::DeviceRadixSort::SortPairs(l.temp, temp_bytes, keys, vals, N, 0, 32, st));
+    count_launch(cub_sort_launches(N, 32));
+    mlapm_prep_cull_kernel<<<static_cast<unsigned>(T), MS_BLOCK, 0, st>>>(
+        p2, v2, d2, vals.Current(), N, l.rec, l.slot, reinterpret_cast<ulonglong2 *>(l.acc), l.bad, l.sbox, l.sflag,
+        l.bbox, l.bflag);
+    count_launch();
+    rc_ = check_launch("mlapm_prep_cull_kernel");
+    if (rc_) return rc_;
+    const CullKeep keep{l.sbox, l.bbox, l.sflag, l.bflag, static_cast<int>(T), static_cast<int>(D), rc};
+    const int ncand = static_cast<int>(cull_candidates(N));
+    cub::CountingInputIterator<int> cand(0);
+    need = 0;
+    PIML_CUDA(cub::DeviceSelect::If(nullptr, need, cand, l.items, l.nitems, ncand, keep, st));
+    PIML_REQUIRE(static_cast<int64_t>(need) <= l.temp_bytes,
+                 "piml_mlapm: CUB select needs %lld bytes of scratch, %lld reserved", static_cast<long long>(need),
+                 static_cast<long long>(l.temp_bytes));
+    temp_bytes = static_cast<size_t>(l.temp_bytes);
+    PIML_CUDA(cub::DeviceSelect::If(l.temp, temp_bytes, cand, l.items, l.nitems, ncand, keep, st));
+    count_launch(2);                                              // tile-state init + select
+    using Smem = MsSmem<MS_CT, MS_BATCH, MC_THREADS>;
+    static_assert(sizeof(Smem) <= 48 * 1024, "mlapm_sym_list_kernel: shared memory above the default limit");
+    const void *kfn = version == 0 ? reinterpret_cast<const void *>(&mlapm_sym_list_kernel<0>)
+                                   : reinterpret_cast<const void *>(&mlapm_sym_list_kernel<1>);
+    static const void *cached_fn = nullptr;
+    static int cached_occ = 0;
+    if (kfn != cached_fn) {
+        int occ = 0;
+        PIML_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kfn, MC_THREADS, sizeof(Smem)));
+        cached_occ = occ < 1 ? 1 : occ;
+        cached_fn = kfn;
+    }
+    // persistent grid: one CTA per resident slot, capped by the largest list (it can never have more items)
+    int64_t grid = static_cast<int64_t>(cached_occ) * sm_count();
+    if (grid > ncand) grid = ncand;
+    M2Const k2{k.Bl, k.Cl, k.Dl};
+    unsigned long long *acc = reinterpret_cast<unsigned long long *>(l.acc);
+    if (version == 0)
+        mlapm_sym_list_kernel<0><<<static_cast<unsigned>(grid), MC_THREADS, sizeof(Smem), st>>>(
+            l.rec, l.items, l.nitems, static_cast<int>(T), static_cast<int>(D), k2, acc, l.bad, colscale);
+    else
+        mlapm_sym_list_kernel<1><<<static_cast<unsigned>(grid), MC_THREADS, sizeof(Smem), st>>>(
+            l.rec, l.items, l.nitems, static_cast<int>(T), static_cast<int>(D), k2, acc, l.bad, colscale);
+    count_launch();
+    return check_launch("mlapm_sym_list_kernel");
 }
 
 static int mlapm_advance_impl(const float *pos, const float *vel, const float *desired_speed, int ds_dim,
@@ -1061,22 +1533,41 @@ static int mlapm_advance_impl(const float *pos, const float *vel, const float *d
     }
     // production, whole crowd: symmetric evaluation (every unordered pair once) when the caller's workspace holds
     // the column-direction sums; row ranges (agent-sharded ranks) and small crowds use the ordered-pair kernel.
-    SymPartials symp{nullptr, 0.f, 0, nullptr, 0, 0};
-    const bool sym_ok = row0 == 0 && row1 == N && workspace_bytes >= sym_workspace_bytes(N) && sym_params_ok(prm, k, N);
-    if (sym_ok && (g_mlapm_algorithm == 2 || (g_mlapm_algorithm == 0 && N >= MS_AUTO_MIN_AGENTS))) {
+    SymPartials symp{nullptr, 0.f, 0, nullptr, 0, 0, nullptr, nullptr};
+    const bool sym_ok = row0 == 0 && row1 == N && sym_params_ok(prm, k, N);
+    const bool want_sym = g_mlapm_algorithm >= 2 || (g_mlapm_algorithm == 0 && N >= MS_AUTO_MIN_AGENTS);
+    // culled (0, 2): skips the work beyond the radius where the weight is exactly 0; the list index is an int
+    if (sym_ok && want_sym && g_mlapm_algorithm != 3 && workspace_bytes >= cull_workspace_bytes(N) &&
+        cull_candidates(N) < (int64_t{1} << 31)) {
+        const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~static_cast<uintptr_t>(255);
+        const CullLayout l = cull_layout(N, reinterpret_cast<void *>(base));
+        const int sl = sym_colscale_log2(N, prm);
+        rc = launch_sym_culled(prm->version, p2, v2, d2, iN, k, cull_radius(prm, k), l, ldexpf(1.0f, sl), st);
+        if (rc) return rc;
+        symp = SymPartials{l.acc, ldexpf(1.0f, -sl), 0, nullptr, 0, 0, l.slot, l.bad};
+        const int threads = 256;
+        mlapm_finalize2_kernel<<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0, st>>>(
+            p2, v2, desired_speed, ds_dim, d2, r0, r1, 0, nullptr, prm->A, k.cos_t, k.sin_t, prm->version, prm->tau,
+            dt, radius, reinterpret_cast<float2 *>(action), reinterpret_cast<float2 *>(pos_new), arrived, push, symp);
+        count_launch();
+        return check_launch("mlapm_finalize2_kernel");
+    }
+    // dense (3, or a workspace without room for the culled path's list)
+    if (sym_ok && want_sym && workspace_bytes >= sym_workspace_bytes(N)) {
         const int64_t T = sym_blocks(N), D = T / 2, npad = T * MS_BLOCK;
         int per, sub;
         const int S = sym_splits(T, T, &per, &sub);
         float4 *rec = reinterpret_cast<float4 *>(workspace);
         float4 *partialR = rec + npad * 2;
         long long *colsum = reinterpret_cast<long long *>(partialR + static_cast<int64_t>(S) * npad);
+        unsigned *bad = reinterpret_cast<unsigned *>(colsum + npad * 4);
         const int sl = sym_colscale_log2(N, prm);
         rc = launch_sym_pairs(prm->version, p2, v2, d2, iN, T, 0, T, per, sub, S, k, rec, partialR, colsum,
-                              ldexpf(1.0f, sl), st);
+                              ldexpf(1.0f, sl), bad, st);
         if (rc) return rc;
         const int threads = 256;
         (void)D;
-        symp = SymPartials{colsum, ldexpf(1.0f, -sl), static_cast<int>(npad), nullptr, 0, 0};
+        symp = SymPartials{colsum, ldexpf(1.0f, -sl), static_cast<int>(npad), nullptr, 0, 0, nullptr, bad};
         mlapm_finalize2_kernel<<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0, st>>>(
             p2, v2, desired_speed, ds_dim, d2, r0, r1, S, partialR, prm->A, k.cos_t, k.sin_t, prm->version, prm->tau,
             dt, radius, reinterpret_cast<float2 *>(action), reinterpret_cast<float2 *>(pos_new), arrived, push, symp);
@@ -1272,7 +1763,7 @@ extern "C" int piml_mlapm_sym_pairs_push_f32(const float *pos, const float *vel,
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     rc = launch_sym_pairs(prm->version, reinterpret_cast<const float2 *>(pos), reinterpret_cast<const float2 *>(vel),
                           reinterpret_cast<const float2 *>(dest), static_cast<int>(N), pl.T, pl.I0, pl.nI, pl.per, pl.sub, pl.S,
-                          k, pl.rec, pl.partialR, pl.colsum, ldexpf(1.0f, sym_colscale_log2(N, prm)), st);
+                          k, pl.rec, pl.partialR, pl.colsum, ldexpf(1.0f, sym_colscale_log2(N, prm)), nullptr, st);
     if (rc) return rc;
     PeerInbox peers;
     peers.world = world;

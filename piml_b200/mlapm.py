@@ -26,8 +26,9 @@ class MLAPM:
                              float(a.get('D', 0.0)), float(a.get('theta', 0.0)), 1 if a.get('exact_math') else 0)
 
     def _workspace(self, N, device, whole_crowd=False):
-        """Caller-owned scratch of the kernels: O(N) for both evaluations (symmetric: 32 B records + 16 B row partials
-        per split + 32 B fixed-point column accumulators per agent -- 0.15 GB at N = 10^6)."""
+        """Caller-owned scratch of the kernels, the largest any path needs: ordered pairs 16 B per agent and split;
+        symmetric dense 32 B records + 16 B row partials per split + 32 B fixed-point accumulators per agent; symmetric
+        culled the same without the row partials, plus the spatial sort and the work list (0.1 GB at N = 10^6)."""
         lib = L.load()
         need = int(lib.piml_mlapm_workspace_bytes(N))
         if whole_crowd and not self.args.get('exact_math'):
