@@ -15,6 +15,9 @@ _lib = None
 
 vp, i32, i64, f32 = C.c_void_p, C.c_int, C.c_int64, C.c_float
 
+# Linears the PINNSF backward's dW launch can take (DW_MAX_JOBS in csrc/mlp_bwd.cu; keep the two equal).
+PINNSF_DW_JOBS = 38
+
 
 class MlapmParams(C.Structure):
     """piml_mlapm_params"""

@@ -286,8 +286,7 @@ static int pinnsf_forward_impl(const piml_net_desc *desc, const float *params, i
                                const float *ped, const float *obs, const float *self, int64_t R, int kp, int ko,
                                int norm_group, const float *drop_ped, const float *drop_obs, float *acc,
                                float *ped_msgs, float *obs_msgs, float *coll, float *stash, void *stream) {
-    PIML_REQUIRE(desc && params && ped && self && acc, "piml_pinnsf_forward_f32: null pointer");
-    PIML_REQUIRE(!has_obs || obs, "piml_pinnsf_forward_f32: has_obs set but obs is null");
+    PIML_REQUIRE(desc && params, "piml_pinnsf_forward_f32: null pointer");
     PIML_REQUIRE(R >= 0 && kp >= 1 && ko >= 0, "piml_pinnsf_forward_f32: bad dimensions R=%lld kp=%d ko=%d",
                  static_cast<long long>(R), kp, ko);
     PIML_REQUIRE(kp <= FT_TR && ko <= FT_TR, "piml_pinnsf_forward_f32: more than %d slots per agent", FT_TR);
@@ -297,7 +296,9 @@ static int pinnsf_forward_impl(const piml_net_desc *desc, const float *params, i
     PackTab PT;
     int rc = build_plan(desc, &P, &PT);
     if (rc) return rc;
-    if (R == 0) return PIML_OK;
+    if (R == 0) return PIML_OK;        // empty batch: the row buffers may be null (torch's empty tensors are)
+    PIML_REQUIRE(ped && self && acc, "piml_pinnsf_forward_f32: null pointer");
+    PIML_REQUIRE(!has_obs || obs, "piml_pinnsf_forward_f32: has_obs set but obs is null");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const SPlan S = make_splan(P, has_obs != 0, R, kp, ko, coll != nullptr);
 
@@ -369,8 +370,8 @@ extern "C" int piml_pinnsf_forward_train_f32(const piml_net_desc *desc, const fl
                                              int ko, int norm_group, const float *drop_ped, const float *drop_obs,
                                              float *acc, float *ped_msgs, float *obs_msgs, float *coll, float *stash,
                                              void *stream) {
-    PIML_REQUIRE(stash, "piml_pinnsf_forward_train_f32: stash is null");
-    PIML_REQUIRE(!desc || desc->n_coll == 0 || coll, "piml_pinnsf_forward_train_f32: coll output is required");
+    PIML_REQUIRE(stash || R == 0, "piml_pinnsf_forward_train_f32: stash is null");
+    PIML_REQUIRE(!desc || desc->n_coll == 0 || coll || R == 0, "piml_pinnsf_forward_train_f32: coll output is required");
     return pinnsf_forward_impl(desc, params, has_obs, tau, ped, obs, self, R, kp, ko, norm_group, drop_ped, drop_obs,
                                acc, ped_msgs, obs_msgs, coll, stash, stream);
 }

@@ -210,7 +210,14 @@ static int build_chunks_bwd(const FPlan &P, int br, bool want_coll, FTab *T) {
 
 // ---- dW / db -----------------------------------------------------------------------------------------------
 struct DwJob { const float *A; const float *G; int64_t rows; int K, OUT; int64_t dst; };
-struct DwTab { int n; DwJob j[24]; };
+// One job per Linear: per branch the encoders, the single processor block, the decoders and the predictor, then the
+// collision head.  The largest net build_plan accepts needs 2 * (8 + 1 + 8 + 1) + 2 = 38 (piml_b200/_lib.py
+// PINNSF_DW_JOBS mirrors this number for the CPU tests).
+constexpr int DW_MAX_JOBS = 38;
+static_assert(DW_MAX_JOBS == 2 * (sizeof(FPlan::enc) / sizeof(FLayer) + 1 + sizeof(FPlan::dec) / sizeof(FLayer) + 1) +
+                                 sizeof(FPlan::coll) / sizeof(FLayer),
+              "DwTab must hold one job per Linear of the largest net build_plan accepts");
+struct DwTab { int n; DwJob j[DW_MAX_JOBS]; };
 constexpr int DW_ROWS = 32;
 constexpr int DW_LD = 132;
 
@@ -406,12 +413,8 @@ extern "C" int piml_pinnsf_backward_f32(const piml_net_desc *desc, const float *
                                         const float *stash, const float *g_acc, const float *g_ped_msgs,
                                         const float *g_obs_msgs, const float *g_coll, float *g_params, float *g_ped,
                                         float *g_obs, float *g_self, float *workspace, void *stream) {
-    PIML_REQUIRE(desc && packed_bwd && ped && self && stash && g_acc && g_params && workspace,
-                 "piml_pinnsf_backward_f32: null pointer");
-    PIML_REQUIRE(!has_obs || obs, "piml_pinnsf_backward_f32: has_obs set but obs is null");
+    PIML_REQUIRE(desc && packed_bwd && g_params, "piml_pinnsf_backward_f32: null pointer");
     PIML_REQUIRE(R >= 0 && kp >= 1 && ko >= 0 && kp <= FT_TR && ko <= FT_TR, "piml_pinnsf_backward_f32: bad dimensions");
-    PIML_REQUIRE(aligned16(packed_bwd) && aligned16(workspace),
-                 "piml_pinnsf_backward_f32: packed_bwd and workspace must be 16-byte aligned");
     if (!has_obs || ko == 0) { has_obs = 0; ko = 0; }
     FPlan P, Pt;
     PackTab PT;
@@ -421,10 +424,14 @@ extern "C" int piml_pinnsf_backward_f32(const piml_net_desc *desc, const float *
     if (rc) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int64_t t_total = P.t_total, t_pad = (t_total + 3) / 4 * 4;
-    if (R == 0) {
+    if (R == 0) {                      // empty batch: the row buffers may be null (torch's empty tensors are)
         PIML_CUDA(cudaMemsetAsync(g_params, 0, sizeof(float) * t_total, st));
         return PIML_OK;
     }
+    PIML_REQUIRE(ped && self && stash && g_acc && workspace, "piml_pinnsf_backward_f32: null pointer");
+    PIML_REQUIRE(!has_obs || obs, "piml_pinnsf_backward_f32: has_obs set but obs is null");
+    PIML_REQUIRE(aligned16(packed_bwd) && aligned16(workspace),
+                 "piml_pinnsf_backward_f32: packed_bwd and workspace must be 16-byte aligned");
     const bool coll = P.n_coll > 0;
     const SPlan S = make_splan(P, has_obs != 0, R, kp, ko, true);
     const SPlan Gp = S;                                            // same shapes
@@ -460,9 +467,11 @@ extern "C" int piml_pinnsf_backward_f32(const piml_net_desc *desc, const float *
     // 2. dW / db of every Linear
     DwTab J;
     J.n = 0;
-    auto job = [&](const float *A, int64_t goff, int64_t rows, const FLayer &L, int64_t tbase) {
+    auto job = [&](const float *A, int64_t goff, int64_t rows, const FLayer &L, int64_t tbase) -> int {
+        PIML_REQUIRE(J.n < DW_MAX_JOBS, "piml_pinnsf_backward_f32: more than %d Linears", DW_MAX_JOBS);
         DwJob &j = J.j[J.n++];
         j.A = A; j.G = G + goff; j.rows = rows; j.K = L.K; j.OUT = L.OUT; j.dst = tbase + L.t_off;
+        return PIML_OK;
     };
     for (int br = 0; br < (has_obs ? 2 : 1); ++br) {
         const int64_t rows = R * (br == 0 ? kp : ko);
@@ -470,26 +479,27 @@ extern "C" int piml_pinnsf_backward_f32(const piml_net_desc *desc, const float *
         const float *feat = br == 0 ? ped : obs;
         const int64_t tb = P.t_branch_off[br];
         for (int l = 0; l < P.n_enc; ++l)
-            job(l == 0 ? feat : stash + S.enc[br][l - 1], Gp.enc[br][l], rows, P.enc[l], tb);
+            rc |= job(l == 0 ? feat : stash + S.enc[br][l - 1], Gp.enc[br][l], rows, P.enc[l], tb);
         const float *proc_out = P.proc_mode == 1 ? stash + S.proc[br] : stash + S.enc[br][P.n_enc - 1];
-        if (P.proc_mode == 1) job(stash + S.enc[br][P.n_enc - 1], Gp.proc[br], rows, P.proc, tb);
+        if (P.proc_mode == 1) rc |= job(stash + S.enc[br][P.n_enc - 1], Gp.proc[br], rows, P.proc, tb);
         for (int l = 0; l < P.n_dec; ++l) {
             const float *A = l > 0 ? stash + S.dec[br][l - 1] : (P.kind == 0 ? proc_out : stash + S.sum[br]);
-            job(A, Gp.dec[br][l], prow, P.dec[l], tb);
+            rc |= job(A, Gp.dec[br][l], prow, P.dec[l], tb);
         }
-        job(stash + S.dec[br][P.n_dec - 1], Gp.pred[br], prow, P.pred, tb);
+        rc |= job(stash + S.dec[br][P.n_dec - 1], Gp.pred[br], prow, P.pred, tb);
     }
     if (coll) {
         const int64_t rows = R * kp;
         const float *A0 = P.kind == 0 ? stash + S.dec[0][P.n_dec - 1]
                                       : (P.proc_mode == 1 ? stash + S.proc[0] : stash + S.enc[0][P.n_enc - 1]);
         if (P.n_coll == 2) {
-            job(A0, Gp.collh, rows, P.coll[0], P.t_coll_off);
-            job(stash + S.collh, Gp.prob, rows, P.coll[1], P.t_coll_off);
+            rc |= job(A0, Gp.collh, rows, P.coll[0], P.t_coll_off);
+            rc |= job(stash + S.collh, Gp.prob, rows, P.coll[1], P.t_coll_off);
         } else {
-            job(A0, Gp.prob, rows, P.coll[0], P.t_coll_off);
+            rc |= job(A0, Gp.prob, rows, P.coll[0], P.t_coll_off);
         }
     }
+    if (rc) return rc;
     PIML_CUDA(cudaMemsetAsync(ws, 0, sizeof(float) * t_pad * nsplit, st));
     pinnsf_dw_kernel<<<dim3(nsplit, J.n), 256, 0, st>>>(J, ws, t_pad);
     count_launch();

@@ -6,12 +6,17 @@ import torch
 import torch.nn.functional as F
 
 
-def _mlp(sd, prefix, x, n, last_act=False):
-    """MLP (reference src/models/model.py:40-65): Linear + ReLU ..., Identity after the last layer."""
+def _relu(x, name):
+    return torch.relu(x)
+
+
+def _mlp(sd, prefix, x, n, last_act=False, relu=_relu):
+    """MLP (reference src/models/model.py:40-65): Linear + ReLU ..., Identity after the last layer.  relu(x, name) gets
+    the pre-activation of Linear `name` (its state_dict prefix)."""
     for l in range(n):
         x = F.linear(x, sd[f"{prefix}.mlp.{2 * l}.weight"], sd[f"{prefix}.mlp.{2 * l}.bias"])
         if l < n - 1 or last_act:
-            x = torch.relu(x)
+            x = relu(x, f"{prefix}.mlp.{2 * l}")
     return x
 
 
@@ -22,27 +27,32 @@ def _count(sd, prefix):
     return n
 
 
-def pinnsf_forward_ref(sd, kind, tau, ped, obs, slf, has_obs=True, drop_ped=None, drop_obs=None, single_block=False):
+def pinnsf_forward_ref(sd, kind, tau, ped, obs, slf, has_obs=True, drop_ped=None, drop_obs=None, single_block=False,
+                       relu=_relu):
     """PINNSF_bottleneck_multitask.forward (model.py:1185-1221, kind='pinnsf_bm'), PINNSF_multitask.forward
     (:1271-1305, 'pinnsf_m'), PINNSF_bottleneck (:1104-1135), PINNSF (:762-792), with processor_hidden_layers > 1 so
-    that ResDNN(x) = dropout(2x) (model.py:115-119, SURVEY.md B-4).  sd: dict of parameter tensors."""
+    that ResDNN(x) = dropout(2x) (model.py:115-119, SURVEY.md B-4).  sd: dict of parameter tensors.  Every ReLU goes
+    through relu(pre_activation, name of its Linear)."""
     per_slot = kind in ("pinnsf_bm", "pinnsf_bottleneck")
 
+    def mlp(prefix, x, n):
+        return _mlp(sd, prefix, x, n, relu=relu)
+
     def branch(name, x, drop):
-        e = _mlp(sd, f"{name}_encoder", x, _count(sd, f"{name}_encoder"))
+        e = mlp(f"{name}_encoder", x, _count(sd, f"{name}_encoder"))
         if single_block:      # ResDNN with one block: relu(W e + b) + e  (model.py:68-79, :115-119)
-            e = torch.relu(F.linear(e, sd[f"{name}_processor.resnet.0.lin.mlp.0.weight"],
-                                    sd[f"{name}_processor.resnet.0.lin.mlp.0.bias"])) + e
+            key = f"{name}_processor.resnet.0.lin.mlp.0"
+            e = relu(F.linear(e, sd[key + ".weight"], sd[key + ".bias"]), key) + e
         else:
             e = 2 * e
         if drop is not None:
             e = e * drop
         if per_slot:
-            d = _mlp(sd, f"{name}_decoder", e, _count(sd, f"{name}_decoder"))
-            msg = _mlp(sd, f"{name}_predictor", d, 1)
+            d = mlp(f"{name}_decoder", e, _count(sd, f"{name}_decoder"))
+            msg = mlp(f"{name}_predictor", d, 1)
             return msg.sum(-2), msg, d
-        d = _mlp(sd, f"{name}_decoder", e.sum(-2), _count(sd, f"{name}_decoder"))
-        return _mlp(sd, f"{name}_predictor", d, 1), e, e
+        d = mlp(f"{name}_decoder", e.sum(-2), _count(sd, f"{name}_decoder"))
+        return mlp(f"{name}_predictor", d, 1), e, e
 
     acc, pmsg, phead = branch("ped", ped, drop_ped)
     out = [None, pmsg]
@@ -55,7 +65,7 @@ def pinnsf_forward_ref(sd, kind, tau, ped, obs, slf, has_obs=True, drop_ped=None
     n_[n_ == 0] = n_[n_ == 0] + 0.1
     out[0] = acc + (slf[..., -1:] * (slf[..., :2] / n_) - slf[..., 2:4]) / tau
     if kind in ("pinnsf_bm", "pinnsf_m"):
-        c = _mlp(sd, "ped_collision_predictor", phead, _count(sd, "ped_collision_predictor"))
+        c = mlp("ped_collision_predictor", phead, _count(sd, "ped_collision_predictor"))
         out.append(torch.sigmoid(c).squeeze())
     return out
 
