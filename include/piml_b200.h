@@ -200,6 +200,21 @@ PIML_API int piml_mlapm_advance_ws_f32(const float *pos, const float *vel, const
                               const piml_mlapm_params *prm, float dt, float radius, float *action, float *pos_new,
                               uint8_t *arrived, void *workspace, int64_t workspace_bytes, void *stream);
 
+/* Many independent crowds (scenes) in one launch: for every scene s, piml_mlapm_advance_f32 on the scene's active
+ * agents alone, with the scene's own constants.  Padded layout: pos, vel, dest, action, pos_new (S,N,2);
+ * desired_speed (S,N,ds_dim), ds_dim 1 or 2; active, arrived (S,N) uint8.  Inactive slots take part in no pair (their
+ * inputs may hold anything, NaN included) and get action = pos_new = NaN, arrived = 0.
+ * prm: version and exact_math for the whole call, and the constants when scene_params is NULL.
+ * scene_params: NULL, or device (S,6) float = tau, A, B, C, D, theta_deg per scene.
+ * Each active agent sums over its scene's active agents in ascending slot order in one thread: a scene's result does
+ * not depend on the other scenes, on S or on the launch shape, and is deterministic.  No workspace, no allocation.
+ * 1 <= N <= PIML_MLAPM_SCENES_MAX_N (a scene's columns stay in shared memory), S >= 1, S*N < 2^31. */
+#define PIML_MLAPM_SCENES_MAX_N 8192
+PIML_API int piml_mlapm_scenes_advance_f32(const float *pos, const float *vel, const float *desired_speed, int ds_dim,
+                                  const float *dest, const uint8_t *active, int64_t S, int64_t N,
+                                  const piml_mlapm_params *prm, const float *scene_params, float dt, float radius,
+                                  float *action, float *pos_new, uint8_t *arrived, void *stream);
+
 /* piml_mlapm_advance_f32 for an agent-sharded crowd with the path's one exchange FUSED into it (SURVEY.md 8e): the
  * finalize kernel stores the new position and velocity of its rows [row0,row1) straight into every rank's next-state
  * arrays over NVLink / NVSwitch peer memory, instead of a separate all-gather.

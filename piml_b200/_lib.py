@@ -92,6 +92,8 @@ SIGNATURES = {
     "piml_mlapm_cull_items": (i32, [vp, i64, C.POINTER(i64)]),
     "piml_mlapm_advance_ws_f32": (i32, [vp, vp, vp, i32, vp, i64, i64, i64, C.POINTER(MlapmParams), f32, f32, vp, vp,
                                         vp, vp, i64, vp]),
+    "piml_mlapm_scenes_advance_f32": (i32, [vp, vp, vp, i32, vp, vp, i64, i64, C.POINTER(MlapmParams), vp, f32, f32,
+                                            vp, vp, vp, vp]),
     "piml_scatter_rows_push_f32": (i32, [vp, vp, vp, i64, i64, i32, vp, vp, vp, vp]),
     "piml_mlapm_sym_shard_rows": (i32, [i64, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
     "piml_mlapm_sym_inbox_bytes": (i64, [i64, i32]),

@@ -41,6 +41,48 @@ struct MlConst {
     float inv_tau, tau;
 };
 
+// The kernels' constants from the reference's six (host: mlapm_consts; device: one set per scene of
+// mlapm_scenes_kernel).  One derivation, so a scene's constants do not depend on where they were formed.
+__host__ __device__ __forceinline__ MlConst mlapm_derive(int version, float tau, float A, float B, float C, float D,
+                                                         float theta_deg) {
+    MlConst k;
+    k.version = version;
+    k.A = A; k.B = B; k.C = C; k.D = D;
+    const double log2e = 1.4426950408889634;
+    k.Bl = static_cast<float>(B * log2e); k.Cl = static_cast<float>(C * log2e);
+    k.Dl = static_cast<float>(D * log2e);
+    // theta tensor as the reference builds it in fp32: ((+-1 * theta) / 180) * pi   (mlapm.py:33)
+    const float th = (theta_deg / 180.0f) * 3.14159274101257324f;
+    k.cos_t = static_cast<float>(cos(static_cast<double>(th)));
+    k.sin_t = static_cast<float>(sin(static_cast<double>(th)));
+    k.tau = tau; k.inv_tau = 1.0f / tau;
+    return k;
+}
+
+// The rest of the loop body main_mlapm.py:19-34 for one agent, shared by every kernel that finishes a step.  Split so
+// that a kernel forms the destination term before it gathers the pair sum (sx, sy), and the new position and the
+// arrival test only where they are stored (the finalize kernels keep their register counts):
+//   fd = (desired_speed * ed - v) / tau                                (mlapm.py:21-22)
+//   force = fd - (sx, sy) (mlapm.py:29/39);  action = v + force*dt     (mlapm.py:57)
+//   p' = p + action*dt;  arrived = |p' - dest| < radius                (main_mlapm.py:26,34)
+__device__ __forceinline__ float2 mlapm_dest_term(float2 p, float2 v, float2 d, float dsx, float dsy, float tau) {
+    const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
+    const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
+    const float ex = __fdiv_rn(dx, dn), ey = __fdiv_rn(dy, dn);
+    return make_float2(__fdiv_rn(__fsub_rn(__fmul_rn(dsx, ex), v.x), tau),
+                       __fdiv_rn(__fsub_rn(__fmul_rn(dsy, ey), v.y), tau));
+}
+__device__ __forceinline__ float2 mlapm_action(float2 v, float2 fd, float sx, float sy, float dt) {
+    const float fx = __fsub_rn(fd.x, sx), fy = __fsub_rn(fd.y, sy);
+    return make_float2(__fadd_rn(v.x, __fmul_rn(fx, dt)), __fadd_rn(v.y, __fmul_rn(fy, dt)));
+}
+__device__ __forceinline__ float2 mlapm_move(float2 p, float2 a, float dt) {
+    return make_float2(__fadd_rn(p.x, __fmul_rn(a.x, dt)), __fadd_rn(p.y, __fmul_rn(a.y, dt)));
+}
+__device__ __forceinline__ bool mlapm_arrived(float2 q, float2 d, float radius) {
+    return norm2_rn(__fsub_rn(q.x, d.x), __fsub_rn(q.y, d.y)) < radius;
+}
+
 __device__ __forceinline__ float ex2_approx(float x) {            // one MUFU.EX2
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -221,29 +263,20 @@ __global__ void mlapm_finalize_kernel(const float2 *__restrict__ pos, const floa
     if (rl >= nrows) return;
     const int n = row0 + rl;
     const float2 p = pos[n], v = vel[n], d = dest[n];
-    const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
-    const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
-    const float ex = __fdiv_rn(dx, dn), ey = __fdiv_rn(dy, dn);
     const float dsx = ds[static_cast<int64_t>(n) * ds_dim];
     const float dsy = ds[static_cast<int64_t>(n) * ds_dim + (ds_dim > 1 ? 1 : 0)];
-    // force += (desired_speed * ed - velocity) / tau      (mlapm.py:22)
-    float fx = __fdiv_rn(__fsub_rn(__fmul_rn(dsx, ex), v.x), tau);
-    float fy = __fdiv_rn(__fsub_rn(__fmul_rn(dsy, ey), v.y), tau);
+    const float2 fd = mlapm_dest_term(p, v, d, dsx, dsy, tau);
     float sx = 0.f, sy = 0.f;
     for (int s = 0; s < nsplit; ++s) {
         const float2 q = partial[static_cast<int64_t>(s) * nrows + rl];
         sx = __fadd_rn(sx, q.x); sy = __fadd_rn(sy, q.y);
     }
-    fx = __fsub_rn(fx, sx); fy = __fsub_rn(fy, sy);               // force -= (...).sum(dim=1)   (mlapm.py:29/39)
-    const float ax = __fadd_rn(v.x, __fmul_rn(fx, dt));           // action = velocity + force*dt (mlapm.py:57)
-    const float ay = __fadd_rn(v.y, __fmul_rn(fy, dt));
-    action[rl] = make_float2(ax, ay);
+    const float2 a = mlapm_action(v, fd, sx, sy, dt);
+    action[rl] = a;
     if (pos_new || arrived) {
-        const float qx = __fadd_rn(p.x, __fmul_rn(ax, dt));       // p = position + v*dt          (main_mlapm.py:26)
-        const float qy = __fadd_rn(p.y, __fmul_rn(ay, dt));
-        if (pos_new) pos_new[rl] = make_float2(qx, qy);
-        if (arrived)                                              // ||p - destination|| < radius (main_mlapm.py:34)
-            arrived[rl] = norm2_rn(__fsub_rn(qx, d.x), __fsub_rn(qy, d.y)) < radius ? 1 : 0;
+        const float2 q = mlapm_move(p, a, dt);
+        if (pos_new) pos_new[rl] = q;
+        if (arrived) arrived[rl] = mlapm_arrived(q, d, radius) ? 1 : 0;
     }
 }
 
@@ -1060,14 +1093,9 @@ __global__ void mlapm_finalize2_kernel(const float2 *__restrict__ pos, const flo
     float qx = 0.f, qy = 0.f, ax = 0.f, ay = 0.f;
     if (live && sub == 0) {
     const float2 p = pos[n], v = vel[n], d = dest[n];
-    const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
-    const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
-    const float ex = __fdiv_rn(dx, dn), ey = __fdiv_rn(dy, dn);
     const float dsx = ds[static_cast<int64_t>(n) * ds_dim];
     const float dsy = ds[static_cast<int64_t>(n) * ds_dim + (ds_dim > 1 ? 1 : 0)];
-    // force += (desired_speed * ed - velocity) / tau      (mlapm.py:22)
-    float fx = __fdiv_rn(__fsub_rn(__fmul_rn(dsx, ex), v.x), tau);
-    float fy = __fdiv_rn(__fsub_rn(__fmul_rn(dsy, ey), v.y), tau);
+    const float2 fd = mlapm_dest_term(p, v, d, dsx, dsy, tau);
     if (sym.inbox) {
         // agent-sharded symmetric evaluation: one pre-reduced share per rank, added in rank order
         float4 u = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1096,17 +1124,14 @@ __global__ void mlapm_finalize2_kernel(const float2 *__restrict__ pos, const flo
         sx = fmaf(cos_t, s.x, -(sin_t * s.w));
         sy = fmaf(sin_t, s.z, cos_t * s.y);
     }
-    fx = __fsub_rn(fx, __fmul_rn(A, sx));                         // force -= (...).sum(dim=1)   (mlapm.py:29/39)
-    fy = __fsub_rn(fy, __fmul_rn(A, sy));
-    ax = __fadd_rn(v.x, __fmul_rn(fx, dt));                       // action = velocity + force*dt (mlapm.py:57)
-    ay = __fadd_rn(v.y, __fmul_rn(fy, dt));
-    if (action) action[rl] = make_float2(ax, ay);
+    const float2 a = mlapm_action(v, fd, __fmul_rn(A, sx), __fmul_rn(A, sy), dt);
+    ax = a.x; ay = a.y;
+    if (action) action[rl] = a;
     if (pos_new || arrived || push.world > 0) {
-        qx = __fadd_rn(p.x, __fmul_rn(ax, dt));                   // p = position + v*dt          (main_mlapm.py:26)
-        qy = __fadd_rn(p.y, __fmul_rn(ay, dt));
-        if (pos_new) pos_new[rl] = make_float2(qx, qy);
-        if (arrived)                                              // ||p - destination|| < radius (main_mlapm.py:34)
-            arrived[rl] = norm2_rn(__fsub_rn(qx, d.x), __fsub_rn(qy, d.y)) < radius ? 1 : 0;
+        const float2 q = mlapm_move(p, a, dt);
+        qx = q.x; qy = q.y;
+        if (pos_new) pos_new[rl] = q;
+        if (arrived) arrived[rl] = mlapm_arrived(q, d, radius) ? 1 : 0;
     }
     }
     if (push.world > 0) {
@@ -1125,6 +1150,118 @@ __global__ void mlapm_finalize2_kernel(const float2 *__restrict__ pos, const flo
         __syncthreads();
         if (threadIdx.x == 0) __threadfence_system();
     }
+}
+
+// =====================================================================================================================
+// Many independent scenes in one launch (piml_mlapm_scenes_advance_f32).  Layout padded (S, N): a scene's active slots
+// are its agents, the inactive ones take part in nothing.
+//
+// One thread owns one row and sums its scene's active columns in ascending slot order (pair_fast / pair_exact), so a
+// scene's result does not depend on the batch, on S or on the launch shape.  A "chunk" is C lanes of one scene:
+//   N <= 32    C = the power of two >= N, 256 / C scenes per CTA (8 scenes of 32 lanes ... 256 of 1)
+//   N <= 256   C = N rounded up to whole warps, floor(256 / C) scenes per CTA
+//   N  > 256   the rows split over ceil(N / 256) CTAs of C <= 256 lanes each (balanced, whole warps)
+// Every CTA stages the columns of its scenes (position, velocity: TMA bulk copies where 16 B aligned, like the dense
+// kernel's tiles; activity flags) and their constants in shared memory: 17 B per column, 139 KB at N = 8192.
+// =====================================================================================================================
+constexpr int MSC_THREADS = 256;
+static_assert(PIML_MLAPM_SCENES_MAX_N * 17 + 1024 <= 227 * 1024, "mlapm_scenes_kernel: columns exceed shared memory");
+
+struct MscShape { int C, k, nchunk; };       // lanes per chunk, scenes per CTA, chunks (CTAs) per scene
+struct MscSmem { int pv, cst, act, total; }; // byte offsets: positions + velocities, constants, flags; total
+
+static MscShape msc_shape(int N) {
+    MscShape sh;
+    sh.nchunk = (N + MSC_THREADS - 1) / MSC_THREADS;
+    if (N <= 32) {
+        sh.C = 1;
+        while (sh.C < N) sh.C *= 2;
+    } else {
+        const int rows = (N + sh.nchunk - 1) / sh.nchunk;
+        sh.C = (rows + 31) / 32 * 32;
+    }
+    sh.k = sh.nchunk == 1 ? MSC_THREADS / sh.C : 1;
+    return sh;
+}
+
+__host__ __device__ __forceinline__ MscSmem msc_smem(int ncol, int k) {
+    MscSmem m;
+    m.pv = 16;                                                    // after the mbarrier
+    const int pv_bytes = (ncol + 1) / 2 * 16;                     // each array a whole number of 16 B
+    m.cst = m.pv + 2 * pv_bytes;
+    m.act = m.cst + k * static_cast<int>(sizeof(MlConst));
+    m.total = m.act + ncol;
+    return m;
+}
+
+template <int VERSION, bool EXACT>
+__global__ void __launch_bounds__(MSC_THREADS) mlapm_scenes_kernel(
+    const float2 *__restrict__ pos, const float2 *__restrict__ vel, const float *__restrict__ ds, int ds_dim,
+    const float2 *__restrict__ dest, const uint8_t *__restrict__ active, int S, int N, MscShape sh, MlConst k0,
+    const float *__restrict__ scene_params, float dt, float radius, float2 *__restrict__ action,
+    float2 *__restrict__ pos_new, uint8_t *__restrict__ arrived) {
+    extern __shared__ __align__(128) unsigned char msc_raw[];
+    const int group = blockIdx.x / sh.nchunk, chunk = blockIdx.x % sh.nchunk;
+    const int s0 = group * sh.k;
+    const int ks = min(sh.k, S - s0);                             // scenes this CTA holds
+    const int ncol = ks * N;
+    const MscSmem lay = msc_smem(ncol, sh.k);
+    uint64_t *bar = reinterpret_cast<uint64_t *>(msc_raw);
+    float2 *sp = reinterpret_cast<float2 *>(msc_raw + lay.pv);
+    float2 *sv = sp + (ncol + 1) / 2 * 2;
+    MlConst *sk = reinterpret_cast<MlConst *>(msc_raw + lay.cst);
+    uint8_t *sa = msc_raw + lay.act;
+    if (threadIdx.x == 0) {
+        mbar_init(bar, 1);
+        mbar_fence_init();
+    }
+    __syncthreads();
+    const int64_t base = static_cast<int64_t>(s0) * N;
+    const bool tma = stage_tile_pv(sp, sv, pos + base, vel + base, ncol, bar);
+    for (int i = threadIdx.x; i < ncol; i += blockDim.x) sa[i] = active[base + i];
+    if (static_cast<int>(threadIdx.x) < ks) {
+        MlConst c = k0;
+        if (scene_params) {
+            const float *q = scene_params + 6 * static_cast<int64_t>(s0 + threadIdx.x);
+            c = mlapm_derive(VERSION, q[0], q[1], q[2], q[3], q[4], q[5]);
+        }
+        sk[threadIdx.x] = c;
+    }
+    if (tma) mbar_wait(bar, 0);
+    __syncthreads();
+
+    const int ls = threadIdx.x / sh.C, row = chunk * sh.C + threadIdx.x % sh.C;
+    if (ls >= ks || row >= N) return;
+    const int c0 = ls * N;
+    const int64_t n = base + c0 + row;
+    if (!sa[c0 + row]) {
+        action[n] = make_float2(CUDART_NAN_F, CUDART_NAN_F);
+        pos_new[n] = make_float2(CUDART_NAN_F, CUDART_NAN_F);
+        arrived[n] = 0;
+        return;
+    }
+    const MlConst k = sk[ls];
+    const float2 p = sp[c0 + row], v = sv[c0 + row], d = dest[n];
+    // ed = F.normalize(destination - position)   (mlapm.py:21)
+    const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
+    const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
+    const float ex = __fdiv_rn(dx, dn), ey = __fdiv_rn(dy, dn);
+    float fx = 0.f, fy = 0.f;
+    const float2 *cp = sp + c0, *cv = sv + c0;
+    const uint8_t *ca = sa + c0;
+#pragma unroll 4
+    for (int j = 0; j < N; ++j) {
+        if (!ca[j]) continue;
+        if (EXACT) pair_exact<VERSION>(p.x, p.y, v.x, v.y, ex, ey, cp[j], cv[j], k, fx, fy);
+        else pair_fast<VERSION>(p.x, p.y, v.x, v.y, ex, ey, cp[j], cv[j], k, fx, fy);
+    }
+    const float dsx = ds[n * ds_dim];
+    const float dsy = ds[n * ds_dim + (ds_dim > 1 ? 1 : 0)];
+    const float2 a = mlapm_action(v, mlapm_dest_term(p, v, d, dsx, dsy, k.tau), fx, fy, dt);
+    const float2 q = mlapm_move(p, a, dt);
+    action[n] = a;
+    pos_new[n] = q;
+    arrived[n] = mlapm_arrived(q, d, radius) ? 1 : 0;
 }
 
 constexpr int ML_MAX_SPLIT = 64;
@@ -1339,18 +1476,7 @@ extern "C" int64_t piml_mlapm_workspace_bytes(int64_t N) {
 }
 
 static MlConst mlapm_consts(const piml_mlapm_params *prm) {
-    MlConst k;
-    k.version = prm->version;
-    k.A = prm->A; k.B = prm->B; k.C = prm->C; k.D = prm->D;
-    const double log2e = 1.4426950408889634;
-    k.Bl = static_cast<float>(prm->B * log2e); k.Cl = static_cast<float>(prm->C * log2e);
-    k.Dl = static_cast<float>(prm->D * log2e);
-    // theta tensor as the reference builds it in fp32: ((+-1 * theta) / 180) * pi   (mlapm.py:33)
-    const float th = (prm->theta_deg / 180.0f) * 3.14159274101257324f;
-    k.cos_t = static_cast<float>(cos(static_cast<double>(th)));
-    k.sin_t = static_cast<float>(sin(static_cast<double>(th)));
-    k.tau = prm->tau; k.inv_tau = 1.0f / prm->tau;
-    return k;
+    return mlapm_derive(prm->version, prm->tau, prm->A, prm->B, prm->C, prm->D, prm->theta_deg);
 }
 
 // The padding agents of the symmetric kernel need a weight that underflows to 0 at large r.
@@ -1621,6 +1747,50 @@ static int mlapm_advance_impl(const float *pos, const float *vel, const float *d
         dt, radius, reinterpret_cast<float2 *>(action), reinterpret_cast<float2 *>(pos_new), arrived, push, symp);
     count_launch();
     return check_launch("mlapm_finalize2_kernel");
+}
+
+extern "C" int piml_mlapm_scenes_advance_f32(const float *pos, const float *vel, const float *desired_speed,
+                                             int ds_dim, const float *dest, const uint8_t *active, int64_t S,
+                                             int64_t N, const piml_mlapm_params *prm, const float *scene_params,
+                                             float dt, float radius, float *action, float *pos_new, uint8_t *arrived,
+                                             void *stream) {
+    PIML_REQUIRE(pos && vel && desired_speed && dest && active && prm && action && pos_new && arrived,
+                 "piml_mlapm_scenes_advance_f32: null pointer");
+    PIML_REQUIRE(S >= 1 && N >= 1 && S * N < (int64_t{1} << 31),
+                 "piml_mlapm_scenes_advance_f32: S=%lld, N=%lld out of range (S, N >= 1, S*N < 2^31)",
+                 static_cast<long long>(S), static_cast<long long>(N));
+    PIML_REQUIRE(N <= PIML_MLAPM_SCENES_MAX_N,
+                 "piml_mlapm_scenes_advance_f32: N=%lld slots per scene, at most %d are supported (a scene's columns "
+                 "stay in shared memory); step a larger crowd with piml_mlapm_advance_ws_f32 (MLAPM.advance)",
+                 static_cast<long long>(N), PIML_MLAPM_SCENES_MAX_N);
+    PIML_REQUIRE(ds_dim == 1 || ds_dim == 2, "piml_mlapm_scenes_advance_f32: ds_dim=%d, must be 1 or 2", ds_dim);
+    PIML_REQUIRE(prm->version == 0 || prm->version == 1,
+                 "piml_mlapm_scenes_advance_f32: version %d unsupported (0='raw', 1='GC')", prm->version);
+    PIML_REQUIRE(((reinterpret_cast<uintptr_t>(pos) | reinterpret_cast<uintptr_t>(vel) |
+                   reinterpret_cast<uintptr_t>(dest) | reinterpret_cast<uintptr_t>(action) |
+                   reinterpret_cast<uintptr_t>(pos_new)) & 7u) == 0,
+                 "piml_mlapm_scenes_advance_f32: pointers must be 8-byte aligned");
+    int iS = static_cast<int>(S), iN = static_cast<int>(N);
+    MscShape sh = msc_shape(iN);
+    const int64_t grid = (S + sh.k - 1) / sh.k * sh.nchunk;
+    const int smem = msc_smem(sh.k * iN, sh.k).total;
+    MlConst k0 = mlapm_consts(prm);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const void *kfn = prm->version == 0 ? (prm->exact_math ? reinterpret_cast<const void *>(&mlapm_scenes_kernel<0, true>)
+                                                           : reinterpret_cast<const void *>(&mlapm_scenes_kernel<0, false>))
+                                        : (prm->exact_math ? reinterpret_cast<const void *>(&mlapm_scenes_kernel<1, true>)
+                                                           : reinterpret_cast<const void *>(&mlapm_scenes_kernel<1, false>));
+    if (smem > 48 * 1024)                                         // per device: a process may drive several GPUs
+        PIML_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    const float2 *p2 = reinterpret_cast<const float2 *>(pos), *v2 = reinterpret_cast<const float2 *>(vel);
+    const float2 *d2 = reinterpret_cast<const float2 *>(dest);
+    float2 *a2 = reinterpret_cast<float2 *>(action), *q2 = reinterpret_cast<float2 *>(pos_new);
+    void *args[] = {&p2, &v2, &desired_speed, &ds_dim, &d2, &active, &iS, &iN, &sh, &k0, &scene_params, &dt, &radius,
+                    &a2, &q2, &arrived};
+    PIML_CUDA(cudaLaunchKernel(kfn, dim3(static_cast<unsigned>(grid)), dim3(sh.k * sh.C), args,
+                               static_cast<size_t>(smem), st));
+    count_launch();
+    return check_launch("mlapm_scenes_kernel");
 }
 
 extern "C" int piml_mlapm_advance_f32(const float *pos, const float *vel, const float *desired_speed, int ds_dim,
