@@ -455,6 +455,40 @@ typedef struct {
 /* Enqueues the whole loop (3-4 launches per step, no host synchronisation) on `stream`. */
 PIML_API int piml_rollout_f32(const piml_rollout_args *args, void *stream);
 
+/* ---- social-force constants sweep: one clip rolled out under S constant sets ------------------------------------- */
+
+/* The pure social-force rollout of piml_rollout_f32 (sfm mode) of ONE clip from t_start to T, under S constant sets at
+ * once.  The clip's ground truth, waypoints and obstacles are shared by all sets (no scene axis).  For each set s the
+ * trajectory equals piml_rollout_f32 on the clip alone with params[s], bit for bit, on either route (persistent kernel
+ * or per-step launches, chosen as piml_rollout_f32 chooses them).  Score per set, over t in [t_start, T) and the slots n
+ * whose simulated position at t is not NaN and mask_p[t][n] == 1:
+ *   err_sum[s] = sum ||p_sim[t][s][n] - pos_tm[t][n]||_2 (float64),  err_count[s] = number of terms.
+ * Each slot sums its own terms in time order, then the slots of a set are added in slot order: the score does not
+ * depend on S, on the set's position in the batch or on the route.  All pointers are device pointers. */
+typedef struct {
+    int S, N, M, D, T, t_start; float dt;
+    int kp; float cos_p, thr_p; int ko; float cos_o, thr_o;            /* topk / cos(sight angle) / distance threshold */
+    const float *obstacles;                                             /* (M,2), NULL when M == 0 */
+    const float *pos_tm, *vel_tm, *acc_tm, *dest_tm;                    /* (T,N,2) */
+    const int64_t *dest_idx_tm;                                         /* (T,N) */
+    const int64_t *entry_tm;                                            /* (T,N) mask_p - mask_p_pred (simulators.py:593) */
+    const float *mask_p;                                                /* (T,N): the slots the score compares */
+    const int64_t *dest_num;                                            /* (N) */
+    const float *waypoints;                                             /* (D,N,2) */
+    const float *desired_speed;                                         /* (N) */
+    const float *p, *v, *a, *dest; const int64_t *dest_idx;             /* (N,..) state at t_start (read only) */
+    const float *ped_f, *obs_f, *self_f;                                /* (N,kp',6), (N,ko',6), (N,7) its features */
+    const piml_sfm_params *params;                                      /* (S) constant sets */
+    double *err_sum; int64_t *err_count;                                /* (S) out */
+    float *rec_p, *rec_v, *rec_a, *rec_mask;  /* (T,S,N,2) x3, (T,S,N): rows t >= t_start written as piml_rollout_f32
+                                                 writes them; all four NULL for a score-only sweep */
+    void *workspace; int64_t workspace_bytes;                           /* >= piml_sfm_sweep_workspace_bytes(args) */
+} piml_sfm_sweep_args;
+
+/* Workspace bytes piml_sfm_sweep_f32 needs for these sizes and the route it will take: O(S N), never O(S T N). */
+PIML_API int64_t piml_sfm_sweep_workspace_bytes(const piml_sfm_sweep_args *args);
+PIML_API int piml_sfm_sweep_f32(const piml_sfm_sweep_args *args, void *stream);
+
 /* ---- one NN-augmented rollout step, fused: src/models/simulators.py:595-652 ----------------------------------------- */
 
 /* The loop body of get_multiple_rollouts re-ordered around the state: features of the current state

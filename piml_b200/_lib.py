@@ -44,6 +44,18 @@ class RolloutArgs(C.Structure):
                 ("rec_p", vp), ("rec_v", vp), ("rec_a", vp), ("rec_mask", vp), ("sfm", vp)]
 
 
+class SfmSweepArgs(C.Structure):
+    """piml_sfm_sweep_args"""
+    _fields_ = [("S", i32), ("N", i32), ("M", i32), ("D", i32), ("T", i32), ("t_start", i32), ("dt", f32),
+                ("kp", i32), ("cos_p", f32), ("thr_p", f32), ("ko", i32), ("cos_o", f32), ("thr_o", f32),
+                ("obstacles", vp), ("pos_tm", vp), ("vel_tm", vp), ("acc_tm", vp), ("dest_tm", vp),
+                ("dest_idx_tm", vp), ("entry_tm", vp), ("mask_p", vp), ("dest_num", vp), ("waypoints", vp),
+                ("desired_speed", vp), ("p", vp), ("v", vp), ("a", vp), ("dest", vp), ("dest_idx", vp),
+                ("ped_f", vp), ("obs_f", vp), ("self_f", vp), ("params", vp), ("err_sum", vp), ("err_count", vp),
+                ("rec_p", vp), ("rec_v", vp), ("rec_a", vp), ("rec_mask", vp), ("workspace", vp),
+                ("workspace_bytes", i64)]
+
+
 class NnStepArgs(C.Structure):
     """piml_nn_step_args"""
     _fields_ = [("desc", C.POINTER(NetDesc)), ("packed_tc", vp), ("has_obs", i32), ("tau", f32),
@@ -134,6 +146,8 @@ SIGNATURES = {
     "piml_relative_features_backward_f32": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp]),
     "piml_collision_detection_f32": (i32, [vp, vp, i32, i32, i32, f32, i32, vp, vp, vp]),
     "piml_rollout_f32": (i32, [C.POINTER(RolloutArgs), vp]),
+    "piml_sfm_sweep_workspace_bytes": (i64, [C.POINTER(SfmSweepArgs)]),
+    "piml_sfm_sweep_f32": (i32, [C.POINTER(SfmSweepArgs), vp]),
     "piml_nn_step_supported": (i32, [C.POINTER(NetDesc)]),
     "piml_nn_step_f32": (i32, [C.POINTER(NnStepArgs), vp]),
     "piml_nn_step_shard_f32": (i32, [C.POINTER(NnStepArgs), i64, i64, i32, vp, vp, vp, vp]),

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libpiml_b200.so")
-SOURCES = ["api.cu", "features.cu", "features_cells.cu", "mlapm.cu", "mlp.cu", "mlp_bwd.cu", "mlp_tc.cu", "mlp_tc16.cu", "integrate.cu", "nn_step.cu", "losses.cu", "metrics.cu", "rollout.cu", "rollout_sfm.cu", "sfm.cu"]
+SOURCES = ["api.cu", "features.cu", "features_cells.cu", "mlapm.cu", "mlp.cu", "mlp_bwd.cu", "mlp_tc.cu", "mlp_tc16.cu", "integrate.cu", "nn_step.cu", "losses.cu", "metrics.cu", "rollout.cu", "rollout_sfm.cu", "sfm.cu", "sfm_sweep.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC,-fvisibility=hidden", "--expt-relaxed-constexpr", "-cudart", "static"]
 

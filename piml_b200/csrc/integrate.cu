@@ -8,13 +8,18 @@
 
 namespace piml {
 
+template <bool SWEEP = false>
 __device__ __forceinline__ void integrate_body(const IntArgs &g) {
     const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i >= static_cast<int64_t>(g.S) * g.N) return;
-    integrate_agent(g, i, g.a_next[i]);
+    integrate_agent<SWEEP>(g, i, g.a_next[i]);
 }
 
 __global__ void integrate_kernel(IntArgs g) { integrate_body(g); }
+
+// The step of a constants sweep (sfm_sweep.cu): S sets of one clip, whose ground truth has no scene axis; the
+// recorded position is added to the slot's score.
+__global__ void integrate_sweep_kernel(IntArgs g) { integrate_body<true>(g); }
 
 // The same step with the frame index read from device memory: `g` carries the BASE pointers of the time-major
 // ground-truth / record arrays, frame t = *t_dev selects the slices (record into frame t, entries from frame t + 1).
@@ -48,6 +53,14 @@ int integrate_step_indirect(const piml_rollout_args *r, const int *t_dev, cudaSt
     integrate_indirect_kernel<<<static_cast<unsigned>((tot + threads - 1) / threads), threads, 0, st>>>(g, t_dev);
     count_launch();
     return check_launch("integrate_indirect_kernel");
+}
+
+int integrate_sweep_launch(const IntArgs &g, cudaStream_t st) {
+    const int64_t tot = static_cast<int64_t>(g.S) * g.N;
+    const int threads = 128;
+    integrate_sweep_kernel<<<static_cast<unsigned>((tot + threads - 1) / threads), threads, 0, st>>>(g);
+    count_launch();
+    return check_launch("integrate_sweep_kernel");
 }
 
 int advance_counter(int *t_dev, cudaStream_t st) {

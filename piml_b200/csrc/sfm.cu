@@ -35,12 +35,10 @@ __global__ void calc_acceleration_kernel(const float *__restrict__ rel, int64_t 
 
 // Pure social-force "model" (BASELINE config 2): v0 repulsion per ped / obstacle slot (utils.py:53-58), slot sums,
 // destination term (model.py:1205-1210).  One thread per agent: 16 slots x 8 B + 28 B read, 8 B written (+ messages).
-__global__ void sfm_forward_kernel(const float *__restrict__ ped, const float *__restrict__ obs,
-                                   const float *__restrict__ self, int64_t R, int kp, int ko, piml_sfm_params c,
-                                   float2 *__restrict__ acc, float2 *__restrict__ ped_msgs,
-                                   float2 *__restrict__ obs_msgs) {
-    const int64_t r = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-    if (r >= R) return;
+__device__ __forceinline__ void sfm_forward_row(const float *__restrict__ ped, const float *__restrict__ obs,
+                                                const float *__restrict__ self, int64_t r, int kp, int ko,
+                                                const piml_sfm_params &c, float2 *__restrict__ acc,
+                                                float2 *__restrict__ ped_msgs, float2 *__restrict__ obs_msgs) {
     float ax = 0.f, ay = 0.f, ox = 0.f, oy = 0.f;
     for (int j = 0; j < kp; ++j) {
         const float2 d = *reinterpret_cast<const float2 *>(ped + (r * kp + j) * 6);
@@ -56,6 +54,34 @@ __global__ void sfm_forward_kernel(const float *__restrict__ ped, const float *_
     }
     const float *s = self + r * 7;
     acc[r] = sfm_total(ax, ay, ox, oy, s[0], s[1], s[2], s[3], s[6], c.tau);
+}
+
+__global__ void sfm_forward_kernel(const float *__restrict__ ped, const float *__restrict__ obs,
+                                   const float *__restrict__ self, int64_t R, int kp, int ko, piml_sfm_params c,
+                                   float2 *__restrict__ acc, float2 *__restrict__ ped_msgs,
+                                   float2 *__restrict__ obs_msgs) {
+    const int64_t r = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (r >= R) return;
+    sfm_forward_row(ped, obs, self, r, kp, ko, c, acc, ped_msgs, obs_msgs);
+}
+
+// The same per row with the constants of the row's set (row r belongs to set r / N): the forward of a constants sweep.
+__global__ void sfm_forward_sets_kernel(const float *__restrict__ ped, const float *__restrict__ obs,
+                                        const float *__restrict__ self, int64_t R, int kp, int ko,
+                                        const piml_sfm_params *__restrict__ sets, int N, float2 *__restrict__ acc) {
+    const int64_t r = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (r >= R) return;
+    const piml_sfm_params c = sets[r / N];
+    sfm_forward_row(ped, obs, self, r, kp, ko, c, acc, nullptr, nullptr);
+}
+
+int sfm_forward_sets_launch(const piml_sfm_params *sets, int N, const float *ped_f, const float *obs_f,
+                            const float *self_f, int64_t R, int kp, int ko, float *acc, cudaStream_t st) {
+    const int threads = 128;
+    sfm_forward_sets_kernel<<<static_cast<unsigned>((R + threads - 1) / threads), threads, 0, st>>>(
+        ped_f, obs_f, self_f, R, kp, ko, sets, N, reinterpret_cast<float2 *>(acc));
+    count_launch();
+    return check_launch("sfm_forward_sets_kernel");
 }
 
 }  // namespace piml
