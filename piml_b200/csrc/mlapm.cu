@@ -65,12 +65,16 @@ __host__ __device__ __forceinline__ MlConst mlapm_derive(int version, float tau,
 //   fd = (desired_speed * ed - v) / tau                                (mlapm.py:21-22)
 //   force = fd - (sx, sy) (mlapm.py:29/39);  action = v + force*dt     (mlapm.py:57)
 //   p' = p + action*dt;  arrived = |p' - dest| < radius                (main_mlapm.py:26,34)
-__device__ __forceinline__ float2 mlapm_dest_term(float2 p, float2 v, float2 d, float dsx, float dsy, float tau) {
+// ed = F.normalize(destination - position)                             (mlapm.py:21)
+__device__ __forceinline__ float2 mlapm_dest_dir(float2 p, float2 d) {
     const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
     const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
-    const float ex = __fdiv_rn(dx, dn), ey = __fdiv_rn(dy, dn);
-    return make_float2(__fdiv_rn(__fsub_rn(__fmul_rn(dsx, ex), v.x), tau),
-                       __fdiv_rn(__fsub_rn(__fmul_rn(dsy, ey), v.y), tau));
+    return make_float2(__fdiv_rn(dx, dn), __fdiv_rn(dy, dn));
+}
+__device__ __forceinline__ float2 mlapm_dest_term(float2 p, float2 v, float2 d, float dsx, float dsy, float tau) {
+    const float2 e = mlapm_dest_dir(p, d);
+    return make_float2(__fdiv_rn(__fsub_rn(__fmul_rn(dsx, e.x), v.x), tau),
+                       __fdiv_rn(__fsub_rn(__fmul_rn(dsy, e.y), v.y), tau));
 }
 __device__ __forceinline__ float2 mlapm_action(float2 v, float2 fd, float sx, float sy, float dt) {
     const float fx = __fsub_rn(fd.x, sx), fy = __fsub_rn(fd.y, sy);
@@ -199,12 +203,9 @@ __global__ void __launch_bounds__(ML_THREADS) mlapm_pairs_kernel(const float2 *_
         int rl = rbase + i * ML_THREADS + threadIdx.x;
         rl = rl < nrows ? rl : nrows - 1;
         const int n = row0 + rl;
-        const float2 p = pos[n], v = vel[n], d = dest[n];
+        const float2 p = pos[n], v = vel[n], e = mlapm_dest_dir(p, dest[n]);
         px[i] = p.x; py[i] = p.y; vx[i] = v.x; vy[i] = v.y;
-        // ed = F.normalize(destination - position)   (mlapm.py:21)
-        const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
-        const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
-        ex[i] = __fdiv_rn(dx, dn); ey[i] = __fdiv_rn(dy, dn);
+        ex[i] = e.x; ey[i] = e.y;
         fx[i] = 0.f; fy[i] = 0.f;
     }
 
@@ -364,7 +365,7 @@ __device__ __forceinline__ void pair2(const float2 npx, const float2 npy, const 
 }
 
 // partial[split][row - row0] = (Sx, Sy, Tx', Ty') over this split's columns.  Each thread owns 2*RP rows.
-template <int VERSION, int RP, int UNROLL>
+template <int VERSION, int RP>
 __global__ void __launch_bounds__(M2_THREADS) mlapm_pairs2_kernel(const float2 *__restrict__ pos,
                                                                   const float2 *__restrict__ vel,
                                                                   const float2 *__restrict__ dest,
@@ -391,12 +392,9 @@ __global__ void __launch_bounds__(M2_THREADS) mlapm_pairs2_kernel(const float2 *
             int rl = rbase + (2 * i + h) * M2_THREADS + threadIdx.x;
             rl = rl < nrows ? rl : nrows - 1;
             const int n = row0 + rl;
-            const float2 p = pos[n], v = vel[n], d = dest[n];
-            // ed = F.normalize(destination - position)   (mlapm.py:21)
-            const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
-            const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
+            const float2 p = pos[n], v = vel[n], e = mlapm_dest_dir(p, dest[n]);
             t[h][0] = p.x; t[h][1] = p.y; t[h][2] = v.x; t[h][3] = v.y;
-            t[h][4] = __fdiv_rn(dx, dn); t[h][5] = __fdiv_rn(dy, dn);
+            t[h][4] = e.x; t[h][5] = e.y;
         }
         npx[i] = make_float2(-t[0][0], -t[1][0]); npy[i] = make_float2(-t[0][1], -t[1][1]);
         vx[i] = make_float2(t[0][2], t[1][2]); vy[i] = make_float2(t[0][3], t[1][3]);
@@ -426,7 +424,7 @@ __global__ void __launch_bounds__(M2_THREADS) mlapm_pairs2_kernel(const float2 *
         phase_bits ^= (1u << buf);
         const int tn = min(c1 - (c0 + t * M2_TILE), M2_TILE);
         const float4 *tl = tile[buf];
-#pragma unroll(UNROLL)
+#pragma unroll 4
         for (int j = 0; j < tn; ++j) {
             const float4 cp = tl[j];
 #pragma unroll
@@ -466,47 +464,58 @@ __global__ void __launch_bounds__(M2_THREADS) mlapm_pairs2_kernel(const float2 *
 // shared memory (TMA bulk copies, double buffered), so the row direction accumulates in registers as before.  The
 // column direction needs, per column, the sum over all 512 rows of the CTA: the two packed lanes are added, each lane
 // parks its 4 sums for a batch of 8 columns in a per-warp shared-memory scratch, the warp transposes (lane -> column
-// lane/4, every 4th entry) and finishes with two shuffle stages; the 4 warps' column sums are added in a fixed order
-// and written to partialC[(I, d)][column] -- deterministic, no atomics.  Cost of the reduction per column and warp:
-// 9 FADD + 1 SHFL + 2 x 128-bit shared accesses against 64 packed instructions of pair work.
+// lane/4, every 4th entry) and finishes with two shuffle stages; the warps' column sums are added in a fixed order and
+// go into int64 fixed-point accumulators per agent (ms_add_columns) -- deterministic.  Cost of the reduction per column
+// and warp: 9 FADD + 1 SHFL + 2 x 128-bit shared accesses against 64 packed instructions of pair work.
 // The finalize kernel subtracts the column-direction sums (vr' = -vr) from the row-direction sums.
 // =====================================================================================================================
-constexpr int MS_THREADS = 128;
-constexpr int MS_BLOCK = 512;                     // agents per block of the schedule = rows per CTA (4 per thread)
-constexpr int MS_CT = 128;                        // default columns per shared-memory stage (4 KB; 35 KB per CTA)
-constexpr int MS_BATCH = 8;                       // default columns per warp-level reduction
+constexpr int MS_BLOCK = 512;                     // agents per block of the schedule = rows per CTA
+constexpr int MS_CT = 128;                        // columns per shared-memory stage (4 KB)
+constexpr int MS_BATCH = 8;                       // columns per warp-level reduction
 constexpr int MS_RED_STRIDE = 36;                 // float4 per column of the scratch: 32 lanes + 64 B skew (no conflicts)
 constexpr int MS_RECF = 8;                        // floats per agent record {px,py,vx,vy, ex,ey,0,0}
 constexpr float MS_FAR = 1.0e18f;                 // padding agents sit here: exp(B r) == 0 exactly, nothing overflows
+static_assert(MS_BLOCK % MS_CT == 0 && MS_CT % MS_BATCH == 0 && (MS_BATCH == 8 || MS_BATCH == 4), "bad stage shape");
 
-template <int CT, int BATCH, int THREADS = MS_THREADS>
+template <int THREADS>
 struct MsSmem {
-    float4 tile[2][CT * 2];
-    float4 red[THREADS / 32][BATCH * MS_RED_STRIDE];
-    float4 colacc[THREADS / 32][CT];
+    float4 tile[2][MS_CT * 2];
+    float4 red[THREADS / 32][MS_BATCH * MS_RED_STRIDE];
+    float4 colacc[THREADS / 32][MS_CT];
     uint64_t bars[2];
 };
 
-// rec[j] = {px,py,vx,vy},{ex,ey,0,0}, e = F.normalize(destination - position) (mlapm.py:21); j >= N: padding agents
-// far away (their weight underflows to exactly 0 in both directions), so block tails need no masks.
+// Slot j of the symmetric kernels' inputs for this step: zeroed fixed-point accumulators, a cleared NaN flag (bad may
+// be null) and the record rec[j] = {px,py,vx,vy},{ex,ey,0,0} of agent n; returns its {px,py,vx,vy}.  agent == false: a
+// padding slot, an agent far away whose weight underflows to exactly 0 in both directions, so block tails need no masks.
+__device__ __forceinline__ float4 ms_prep_slot(int j, bool agent, int n, const float2 *__restrict__ pos,
+                                               const float2 *__restrict__ vel, const float2 *__restrict__ dest,
+                                               float4 *__restrict__ rec, ulonglong2 *__restrict__ acc,
+                                               unsigned *__restrict__ bad) {
+    acc[2 * j] = make_ulonglong2(0ull, 0ull);
+    acc[2 * j + 1] = make_ulonglong2(0ull, 0ull);
+    if (bad) bad[j] = 0u;
+    if (!agent) {
+        const float4 far = make_float4(MS_FAR, MS_FAR, 0.f, 0.f);
+        rec[2 * j] = far;
+        rec[2 * j + 1] = make_float4(0.f, 0.f, 0.f, 0.f);
+        return far;
+    }
+    const float2 p = pos[n], v = vel[n], d = dest[n];
+    const float4 pv = make_float4(p.x, p.y, v.x, v.y);
+    rec[2 * j] = pv;
+    const float2 e = mlapm_dest_dir(p, d);
+    rec[2 * j + 1] = make_float4(e.x, e.y, 0.f, 0.f);
+    return pv;
+}
+
+// The slots of the dense symmetric evaluation: agent j in slot j, padding from N up to Npad.
 __global__ void mlapm_prep_sym_kernel(const float2 *__restrict__ pos, const float2 *__restrict__ vel,
                                       const float2 *__restrict__ dest, int N, int Npad, float4 *__restrict__ rec,
                                       ulonglong2 *__restrict__ colsum, unsigned *__restrict__ bad) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= Npad) return;
-    colsum[2 * j] = make_ulonglong2(0ull, 0ull);                   // this step's column-direction accumulators
-    colsum[2 * j + 1] = make_ulonglong2(0ull, 0ull);
-    if (bad) bad[j] = 0u;
-    if (j >= N) {
-        rec[2 * j] = make_float4(MS_FAR, MS_FAR, 0.f, 0.f);
-        rec[2 * j + 1] = make_float4(0.f, 0.f, 0.f, 0.f);
-        return;
-    }
-    const float2 p = pos[j], v = vel[j], d = dest[j];
-    const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
-    const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
-    rec[2 * j] = make_float4(p.x, p.y, v.x, v.y);
-    rec[2 * j + 1] = make_float4(__fdiv_rn(dx, dn), __fdiv_rn(dy, dn), 0.f, 0.f);
+    ms_prep_slot(j, j < N, j, pos, vel, dest, rec, colsum, bad);
 }
 
 // Two rows (packed lanes) against one column, both directions.  Row sums accumulate in S/T; the column's share is
@@ -566,21 +575,125 @@ __device__ __forceinline__ void pair2sym(const float2 npx, const float2 npy, con
     }
 }
 
-// partialR[split][local row] = row-direction (Sx,Sy,Tx',Ty') over the split's block pairs;
-// partialC[(I - I0) * D + d - 1][column of block J] = column-direction sums of block pair (I, J = I + d mod T).
+// A thread's 2 * RPS rows of one row block, two per packed lane pair, and their row-direction sums.
+template <int RPS>
+struct MsRows {
+    float2 npx[RPS], npy[RPS], vx[RPS], vy[RPS], nvx[RPS], nvy[RPS], ex[RPS], ey[RPS], Sx[RPS], Sy[RPS], Tx[RPS],
+        Ty[RPS];
+};
+
+// Rows of block I: lanes x / y of pair i are the block's rows (2i) THREADS + tid and (2i + 1) THREADS + tid, with the
+// CTA's THREADS = MS_BLOCK / (2 RPS) threads; the sums start at 0.
+template <int RPS>
+__device__ __forceinline__ void ms_load_rows(MsRows<RPS> &r, const float4 *__restrict__ rec, int I, int tid) {
+    constexpr int THREADS = MS_BLOCK / (2 * RPS);
+#pragma unroll
+    for (int i = 0; i < RPS; ++i) {
+        const int64_t na = static_cast<int64_t>(I) * MS_BLOCK + (2 * i) * THREADS + tid;
+        const int64_t nb = na + THREADS;
+        const float4 a0 = rec[2 * na], a1 = rec[2 * na + 1], b0 = rec[2 * nb], b1 = rec[2 * nb + 1];
+        r.npx[i] = make_float2(-a0.x, -b0.x); r.npy[i] = make_float2(-a0.y, -b0.y);
+        r.vx[i] = make_float2(a0.z, b0.z); r.vy[i] = make_float2(a0.w, b0.w);
+        r.nvx[i] = make_float2(-a0.z, -b0.z); r.nvy[i] = make_float2(-a0.w, -b0.w);
+        r.ex[i] = make_float2(a1.x, b1.x); r.ey[i] = make_float2(a1.y, b1.y);
+        r.Sx[i] = r.Sy[i] = r.Tx[i] = r.Ty[i] = make_float2(0.f, 0.f);
+    }
+}
+
+// One staged tile of MS_CT column records `tl` of the rows' own (diagonal) block: every ordered pair appears, so each
+// is evaluated in the row direction only (pair2).
+template <int VERSION, int RPS>
+__device__ __forceinline__ void ms_diag_tile(MsRows<RPS> &r, const float4 *tl, float2 Bl, float2 Cl, float2 Dl) {
+#pragma unroll 4
+    for (int j = 0; j < MS_CT; ++j) {
+        const float4 cp = tl[2 * j];
+#pragma unroll
+        for (int i = 0; i < RPS; ++i)
+            pair2<VERSION>(r.npx[i], r.npy[i], r.vx[i], r.vy[i], r.nvx[i], r.nvy[i], r.ex[i], r.ey[i], cp, Bl, Cl, Dl,
+                           r.Sx[i], r.Sy[i], r.Tx[i], r.Ty[i]);
+    }
+}
+
+// One staged tile of MS_CT column records `tl` of another block: every pair feeds both directions (pair2sym).  The
+// warp's column-direction sums go to colacc[column]: the two packed lanes are added, each lane parks its sums of a
+// batch of MS_BATCH columns in the warp's scratch `red`, the warp transposes (lane -> column lane/LPC, every LPC-th
+// entry) and finishes with shuffles.
+template <int VERSION, int RPS>
+__device__ __forceinline__ void ms_pair_tile(MsRows<RPS> &r, const float4 *tl, float4 *red, float4 *colacc, int lane,
+                                             float2 Bl, float2 Cl, float2 Dl) {
+    constexpr int LPC = 32 / MS_BATCH;                      // lanes that share a column in the transposed sum
+    for (int b = 0; b < MS_CT / MS_BATCH; ++b) {
+#pragma unroll
+        for (int c = 0; c < MS_BATCH; ++c) {
+            const float4 cp = tl[2 * (b * MS_BATCH + c)];
+            const float4 ce = tl[2 * (b * MS_BATCH + c) + 1];
+            float2 cSx, cSy, cTx, cTy;
+            pair2sym<VERSION, true>(r.npx[0], r.npy[0], r.vx[0], r.vy[0], r.nvx[0], r.nvy[0], r.ex[0], r.ey[0], cp, ce,
+                                    Bl, Cl, Dl, r.Sx[0], r.Sy[0], r.Tx[0], r.Ty[0], cSx, cSy, cTx, cTy);
+#pragma unroll
+            for (int i = 1; i < RPS; ++i)
+                pair2sym<VERSION, false>(r.npx[i], r.npy[i], r.vx[i], r.vy[i], r.nvx[i], r.nvy[i], r.ex[i], r.ey[i], cp,
+                                         ce, Bl, Cl, Dl, r.Sx[i], r.Sy[i], r.Tx[i], r.Ty[i], cSx, cSy, cTx, cTy);
+            red[c * MS_RED_STRIDE + lane] = make_float4(cSx.x + cSx.y, cSy.x + cSy.y, cTx.x + cTx.y, cTy.x + cTy.y);
+        }
+        __syncwarp();
+        const float4 *col = red + (lane / LPC) * MS_RED_STRIDE + (lane % LPC);
+        float4 a = col[0];
+#pragma unroll
+        for (int e = 1; e < 32 / LPC; ++e) {
+            const float4 t = col[LPC * e];
+            a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
+        }
+#pragma unroll
+        for (int o = 1; o < LPC; o <<= 1) {
+            a.x += __shfl_xor_sync(0xffffffffu, a.x, o);
+            a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
+            a.z += __shfl_xor_sync(0xffffffffu, a.z, o);
+            a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
+        }
+        if (lane % LPC == 0) colacc[b * MS_BATCH + lane / LPC] = a;
+        __syncwarp();
+    }
+}
+
+// The column-direction sums of one stage over the CTA's rows (the warps' colacc, added in warp order) into the
+// crowd-wide FIXED-POINT accumulators acc[slot][4] (int64, 2^-s resolution) of the stage's slots j0 .. j0 + MS_CT - 1,
+// with fire-and-forget 64-bit atomics.  Integer addition is associative, so the total does not depend on the order in
+// which the block pairs that share a column arrive: deterministic like per-pair partial arrays, with O(N) instead of
+// O(N^2 / 64) workspace and DRAM traffic.  A NaN or inf has no fixed-point value: it poisons the slot through its flag
+// in bad, unless bad is null (see SymPartials).
+template <int THREADS>
+__device__ __forceinline__ void ms_add_columns(const float4 (*colacc)[MS_CT], unsigned long long *acc, unsigned *bad,
+                                               int64_t j0, float colscale, int tid) {
+    for (int c = tid; c < MS_CT; c += THREADS) {
+        float4 a = colacc[0][c];
+#pragma unroll
+        for (int wv = 1; wv < THREADS / 32; ++wv) {
+            const float4 t = colacc[wv][c];
+            a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
+        }
+        if (bad && !isfinite(a.x + a.y + a.z + a.w)) bad[j0 + c] = 1u;
+        unsigned long long *dst = acc + (j0 + c) * 4;
+        atomicAdd(dst + 0, static_cast<unsigned long long>(__float2ll_rn(a.x * colscale)));
+        atomicAdd(dst + 1, static_cast<unsigned long long>(__float2ll_rn(a.y * colscale)));
+        atomicAdd(dst + 2, static_cast<unsigned long long>(__float2ll_rn(a.z * colscale)));
+        atomicAdd(dst + 3, static_cast<unsigned long long>(__float2ll_rn(a.w * colscale)));
+    }
+}
+
+// partialR[split][local row] = row-direction (Sx,Sy,Tx',Ty') over the split's block pairs; the column-direction sums
+// of block pair (I, J = I + d mod T) go into colsum (ms_add_columns).
 // RPS = packed row pairs per thread (2 * RPS rows): the CTA's 512 rows are spread over THREADS = 256 / RPS threads.
-template <int VERSION, int CT, int BATCH, int RPS = 2>
+template <int VERSION, int RPS>
 __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const float4 *__restrict__ rec, int T, int D,
                                                                          int I0, int per, int sub, M2Const k,
                                                                          float4 *__restrict__ partialR, int nrows_pad,
                                                                          unsigned long long *__restrict__ colsum,
                                                                          float colscale, unsigned *__restrict__ bad) {
     constexpr int THREADS = MS_BLOCK / (2 * RPS);
-    static_assert(MS_BLOCK % CT == 0 && CT % BATCH == 0 && (BATCH == 8 || BATCH == 4), "bad stage shape");
-    constexpr int SPB = MS_BLOCK / CT;                      // stages per block pair
-    constexpr int LPC = 32 / BATCH;                         // lanes that share a column in the transposed sum
+    constexpr int SPB = MS_BLOCK / MS_CT;                   // stages per block pair
     extern __shared__ __align__(128) unsigned char ms_smem_raw[];
-    MsSmem<CT, BATCH, THREADS> &sm = *reinterpret_cast<MsSmem<CT, BATCH, THREADS> *>(ms_smem_raw);
+    MsSmem<THREADS> &sm = *reinterpret_cast<MsSmem<THREADS> *>(ms_smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid == 0) {
         mbar_init(&sm.bars[0], 1);
@@ -599,120 +712,45 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
     const int d_lo = sy * per;
     const int d_hi = min(d_lo + per, L);
 
-    float2 npx[RPS], npy[RPS], vx[RPS], vy[RPS], nvx[RPS], nvy[RPS], ex[RPS], ey[RPS], Sx[RPS], Sy[RPS], Tx[RPS],
-        Ty[RPS];
-#pragma unroll
-    for (int i = 0; i < RPS; ++i) {
-        const int64_t na = static_cast<int64_t>(I) * MS_BLOCK + (2 * i) * THREADS + tid;
-        const int64_t nb = na + THREADS;
-        const float4 a0 = rec[2 * na], a1 = rec[2 * na + 1], b0 = rec[2 * nb], b1 = rec[2 * nb + 1];
-        npx[i] = make_float2(-a0.x, -b0.x); npy[i] = make_float2(-a0.y, -b0.y);
-        vx[i] = make_float2(a0.z, b0.z); vy[i] = make_float2(a0.w, b0.w);
-        nvx[i] = make_float2(-a0.z, -b0.z); nvy[i] = make_float2(-a0.w, -b0.w);
-        ex[i] = make_float2(a1.x, b1.x); ey[i] = make_float2(a1.y, b1.y);
-        Sx[i] = Sy[i] = Tx[i] = Ty[i] = make_float2(0.f, 0.f);
-    }
+    MsRows<RPS> rw;
+    ms_load_rows(rw, rec, I, tid);
     const float2 Bl = splat(k.Bl), Cl = splat(k.Cl), Dl = splat(k.Dl);
 
     const int nst = d_hi > d_lo ? (d_hi - d_lo) * spc : 0;
-    constexpr uint32_t STAGE_BYTES = CT * MS_RECF * sizeof(float);
-    auto stage_src = [&](int s) {
+    constexpr uint32_t STAGE_BYTES = MS_CT * MS_RECF * sizeof(float);
+    auto stage_j0 = [&](int s) {                             // first slot of stage s
         int J = I + d_lo + s / spc;
         J = J >= T ? J - T : J;
-        return rec + (static_cast<int64_t>(J) * MS_BLOCK + (su * spc + s % spc) * CT) * 2;
+        return static_cast<int64_t>(J) * MS_BLOCK + (su * spc + s % spc) * MS_CT;
     };
     if (tid == 0 && nst > 0) {
         mbar_expect_tx(&sm.bars[0], STAGE_BYTES);
-        tma_bulk_g2s(sm.tile[0], stage_src(0), STAGE_BYTES, &sm.bars[0]);
+        tma_bulk_g2s(sm.tile[0], rec + stage_j0(0) * 2, STAGE_BYTES, &sm.bars[0]);
     }
     uint32_t phase_bits = 0;
     for (int s = 0; s < nst; ++s) {
         const int buf = s & 1;
         if (tid == 0 && s + 1 < nst) {                      // tile[buf^1] was released by the barrier below
             mbar_expect_tx(&sm.bars[buf ^ 1], STAGE_BYTES);
-            tma_bulk_g2s(sm.tile[buf ^ 1], stage_src(s + 1), STAGE_BYTES, &sm.bars[buf ^ 1]);
+            tma_bulk_g2s(sm.tile[buf ^ 1], rec + stage_j0(s + 1) * 2, STAGE_BYTES, &sm.bars[buf ^ 1]);
         }
         mbar_wait(&sm.bars[buf], (phase_bits >> buf) & 1u);
         phase_bits ^= (1u << buf);
-        const float4 *tl = sm.tile[buf];
-        const int d = d_lo + s / spc;
-        if (d == 0) {
-            // diagonal block: rows and columns are the same agents, every ordered pair appears -> one direction each
-#pragma unroll 4
-            for (int j = 0; j < CT; ++j) {
-                const float4 cp = tl[2 * j];
-#pragma unroll
-                for (int i = 0; i < RPS; ++i)
-                    pair2<VERSION>(npx[i], npy[i], vx[i], vy[i], nvx[i], nvy[i], ex[i], ey[i], cp, Bl, Cl, Dl, Sx[i],
-                                   Sy[i], Tx[i], Ty[i]);
-            }
-        } else {
-            float4 *red = sm.red[warp];
-            for (int b = 0; b < CT / BATCH; ++b) {
-#pragma unroll
-                for (int c = 0; c < BATCH; ++c) {
-                    const float4 cp = tl[2 * (b * BATCH + c)];
-                    const float4 ce = tl[2 * (b * BATCH + c) + 1];
-                    float2 cSx, cSy, cTx, cTy;
-                    pair2sym<VERSION, true>(npx[0], npy[0], vx[0], vy[0], nvx[0], nvy[0], ex[0], ey[0], cp, ce, Bl, Cl,
-                                            Dl, Sx[0], Sy[0], Tx[0], Ty[0], cSx, cSy, cTx, cTy);
-#pragma unroll
-                    for (int i = 1; i < RPS; ++i)
-                        pair2sym<VERSION, false>(npx[i], npy[i], vx[i], vy[i], nvx[i], nvy[i], ex[i], ey[i], cp, ce,
-                                                 Bl, Cl, Dl, Sx[i], Sy[i], Tx[i], Ty[i], cSx, cSy, cTx, cTy);
-                    red[c * MS_RED_STRIDE + lane] = make_float4(cSx.x + cSx.y, cSy.x + cSy.y, cTx.x + cTx.y,
-                                                                cTy.x + cTy.y);
-                }
-                __syncwarp();
-                // lane -> column lane/LPC, entries (lane%LPC), (lane%LPC)+LPC, ...: 32/LPC of the 32 row lanes each
-                const float4 *col = red + (lane / LPC) * MS_RED_STRIDE + (lane % LPC);
-                float4 acc = col[0];
-#pragma unroll
-                for (int e = 1; e < 32 / LPC; ++e) {
-                    const float4 t = col[LPC * e];
-                    acc.x += t.x; acc.y += t.y; acc.z += t.z; acc.w += t.w;
-                }
-#pragma unroll
-                for (int o = 1; o < LPC; o <<= 1) {
-                    acc.x += __shfl_xor_sync(0xffffffffu, acc.x, o);
-                    acc.y += __shfl_xor_sync(0xffffffffu, acc.y, o);
-                    acc.z += __shfl_xor_sync(0xffffffffu, acc.z, o);
-                    acc.w += __shfl_xor_sync(0xffffffffu, acc.w, o);
-                }
-                if (lane % LPC == 0) sm.colacc[warp][b * BATCH + lane / LPC] = acc;
-                __syncwarp();
-            }
+        // the off-diagonal branch first: in the other order ptxas emits the diagonal loop twice
+        if (d_lo + s / spc != 0) {
+            ms_pair_tile<VERSION>(rw, sm.tile[buf], sm.red[warp], sm.colacc[warp], lane, Bl, Cl, Dl);
             __syncthreads();
-            // Column-direction sums of this stage's columns (block J), over the CTA's 512 rows: added into the crowd-wide
-            // FIXED-POINT accumulators colsum[agent][4] (int64, 2^-s resolution) with fire-and-forget 64-bit atomics.
-            // Integer addition is associative, so the total does not depend on the order in which the T/2 block pairs
-            // that share a column arrive: deterministic like the per-pair partial arrays this replaces, with O(N)
-            // instead of O(N^2 / 64) workspace and DRAM traffic.
-            int J = I + d;
-            J = J >= T ? J - T : J;
-            unsigned long long *dst = colsum + (static_cast<int64_t>(J) * MS_BLOCK + (su * spc + s % spc) * CT) * 4;
-            for (int c = tid; c < CT; c += THREADS) {
-                float4 a = sm.colacc[0][c];
-#pragma unroll
-                for (int wv = 1; wv < THREADS / 32; ++wv) {
-                    const float4 t = sm.colacc[wv][c];
-                    a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
-                }
-                // a NaN or inf has no fixed-point value: it poisons the agent through its flag (see SymPartials)
-                if (bad && !isfinite(a.x + a.y + a.z + a.w)) bad[(dst - colsum) / 4 + c] = 1u;
-                atomicAdd(dst + c * 4 + 0, static_cast<unsigned long long>(__float2ll_rn(a.x * colscale)));
-                atomicAdd(dst + c * 4 + 1, static_cast<unsigned long long>(__float2ll_rn(a.y * colscale)));
-                atomicAdd(dst + c * 4 + 2, static_cast<unsigned long long>(__float2ll_rn(a.z * colscale)));
-                atomicAdd(dst + c * 4 + 3, static_cast<unsigned long long>(__float2ll_rn(a.w * colscale)));
-            }
+            ms_add_columns<THREADS>(sm.colacc, colsum, bad, stage_j0(s), colscale, tid);
+        } else {
+            ms_diag_tile<VERSION>(rw, sm.tile[buf], Bl, Cl, Dl);
         }
         __syncthreads();
     }
     float4 *out = partialR + static_cast<int64_t>(blockIdx.y) * nrows_pad + static_cast<int64_t>(blockIdx.x) * MS_BLOCK;
 #pragma unroll
     for (int i = 0; i < RPS; ++i) {
-        out[(2 * i) * THREADS + tid] = make_float4(Sx[i].x, Sy[i].x, Tx[i].x, Ty[i].x);
-        out[(2 * i + 1) * THREADS + tid] = make_float4(Sx[i].y, Sy[i].y, Tx[i].y, Ty[i].y);
+        out[(2 * i) * THREADS + tid] = make_float4(rw.Sx[i].x, rw.Sy[i].x, rw.Tx[i].x, rw.Ty[i].x);
+        out[(2 * i + 1) * THREADS + tid] = make_float4(rw.Sx[i].y, rw.Sy[i].y, rw.Tx[i].y, rw.Ty[i].y);
     }
 }
 
@@ -768,8 +806,8 @@ __global__ void mlapm_cull_keys_kernel(const float2 *__restrict__ pos, int N, ui
     val[n] = n;
 }
 
-// One CTA of MS_BLOCK threads per block of the sorted crowd: rec[j] for the agent perm[j] (j >= N: far-away padding as
-// in mlapm_prep_sym_kernel), slot[agent] = j, zeroed accumulators, and the boxes {min x, min y, max x, max y} of the
+// One CTA of MS_BLOCK threads per block of the sorted crowd: slot j holds the agent perm[j] (ms_prep_slot; j >= N:
+// padding), slot[agent] = j, and the boxes {min x, min y, max x, max y} of the
 // block and of its MC_SPB column stages.  Agents with a non-finite position or velocity do not enter the min / max (no
 // fminf / fmaxf on NaN); they flag their stage and block MC_NEAR_ALL instead, which keeps every item that touches them.
 __global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
@@ -780,28 +818,19 @@ __global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
     __shared__ float4 wbox[MS_BLOCK / 32];
     __shared__ unsigned wflag[MS_BLOCK / 32];
     const int j = blockIdx.x * MS_BLOCK + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    acc[2 * j] = make_ulonglong2(0ull, 0ull);
-    acc[2 * j + 1] = make_ulonglong2(0ull, 0ull);
-    bad[j] = 0u;
+    const bool agent = j < N;
+    const int n = agent ? perm[j] : 0;
+    if (agent) slot[n] = j;
+    const float4 pv = ms_prep_slot(j, agent, n, pos, vel, dest, rec, acc, bad);
     float4 b = make_float4(CUDART_INF_F, CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F);
     unsigned flag = MC_EMPTY;
-    if (j < N) {
-        const int n = perm[j];
-        slot[n] = j;
-        const float2 p = pos[n], v = vel[n], d = dest[n];
-        const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
-        const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
-        rec[2 * j] = make_float4(p.x, p.y, v.x, v.y);
-        rec[2 * j + 1] = make_float4(__fdiv_rn(dx, dn), __fdiv_rn(dy, dn), 0.f, 0.f);
-        if (isfinite(p.x) && isfinite(p.y) && isfinite(v.x) && isfinite(v.y)) {
-            b = make_float4(p.x, p.y, p.x, p.y);
+    if (agent) {
+        if (isfinite(pv.x) && isfinite(pv.y) && isfinite(pv.z) && isfinite(pv.w)) {
+            b = make_float4(pv.x, pv.y, pv.x, pv.y);
             flag = 0u;
         } else {
             flag = MC_NEAR_ALL;
         }
-    } else {
-        rec[2 * j] = make_float4(MS_FAR, MS_FAR, 0.f, 0.f);
-        rec[2 * j + 1] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
     // flags combine as: any MC_NEAR_ALL -> MC_NEAR_ALL, else any agent -> 0, else MC_EMPTY
     auto comb = [](unsigned a, unsigned c) { return (a | c) & MC_NEAR_ALL ? MC_NEAR_ALL : (a & c); };
@@ -864,35 +893,34 @@ struct CullKeep {
 // The symmetric pair kernel over the work list.  Persistent: CTA b takes the contiguous items [b n / G, (b+1) n / G)
 // of the n = *nitems on the list (read on the device: no host sync).  Rows stay in registers while consecutive items
 // share the row block; when it changes, and at the end, the row sums go into the fixed-point accumulators with the
-// opposite sign of the column shares (acc = column share - row share; the finalize kernel subtracts acc).  Stage loads
-// (TMA, double buffered), the pair math (pair2 on the diagonal, pair2sym elsewhere) and the warp column reduction are
-// those of mlapm_sym_kernel.
+// opposite sign of the column shares (acc = column share - row share; the finalize kernel subtracts acc).  The stages
+// are evaluated as in mlapm_sym_kernel (ms_diag_tile, ms_pair_tile, ms_add_columns).
 template <int VERSION>
 __global__ void __launch_bounds__(MC_THREADS, 8) mlapm_sym_list_kernel(const float4 *__restrict__ rec,
                                                                       const int *__restrict__ items,
                                                                       const int *__restrict__ nitems, int T, int D,
                                                                       M2Const k, unsigned long long *__restrict__ acc,
                                                                       unsigned *__restrict__ bad, float colscale) {
-    constexpr int THREADS = MC_THREADS, RPS = MS_BLOCK / (2 * THREADS), CT = MS_CT, BATCH = MS_BATCH;
-    constexpr int LPC = 32 / BATCH;
+    constexpr int THREADS = MC_THREADS, RPS = MS_BLOCK / (2 * THREADS);
     extern __shared__ __align__(128) unsigned char ms_smem_raw[];
-    MsSmem<CT, BATCH, THREADS> &sm = *reinterpret_cast<MsSmem<CT, BATCH, THREADS> *>(ms_smem_raw);
-    // the item of the stage in tile[buf] (I, d, first column j0 = J * MS_BLOCK + stage * CT), written by the thread
+    MsSmem<THREADS> &sm = *reinterpret_cast<MsSmem<THREADS> *>(ms_smem_raw);
+    // the item of the stage in tile[buf] (I, d, first column j0 = J * MS_BLOCK + stage * MS_CT), written by the thread
     // that issues its copy; the loop state lives here too, which keeps the pair loop at 128 registers without spills
     __shared__ int meta[2][3];
     __shared__ int s_lo, s_cnt;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    __builtin_assume(bad != nullptr);                          // never null here: one copy of ms_add_columns' loop
     const int n = *nitems;
     const int lo = static_cast<int>(static_cast<int64_t>(n) * blockIdx.x / gridDim.x);
     const int cnt = static_cast<int>(static_cast<int64_t>(n) * (blockIdx.x + 1) / gridDim.x) - lo;
     if (cnt <= 0) return;
-    constexpr uint32_t STAGE_BYTES = CT * MS_RECF * sizeof(float);
+    constexpr uint32_t STAGE_BYTES = MS_CT * MS_RECF * sizeof(float);
     auto stage_load = [&](int s, int buf) {                    // thread 0
         const int c = items[s];
         const int st = c % MC_SPB, pd = c / MC_SPB;
         const int I = pd / (D + 1), d = pd - I * (D + 1);
         const int J = I + d >= T ? I + d - T : I + d;
-        const int j0 = J * MS_BLOCK + st * CT;
+        const int j0 = J * MS_BLOCK + st * MS_CT;
         meta[buf][0] = I; meta[buf][1] = d; meta[buf][2] = j0;
         mbar_expect_tx(&sm.bars[buf], STAGE_BYTES);
         tma_bulk_g2s(sm.tile[buf], rec + static_cast<int64_t>(j0) * 2, STAGE_BYTES, &sm.bars[buf]);
@@ -907,8 +935,7 @@ __global__ void __launch_bounds__(MC_THREADS, 8) mlapm_sym_list_kernel(const flo
     }
     __syncthreads();
 
-    float2 npx[RPS], npy[RPS], vx[RPS], vy[RPS], nvx[RPS], nvy[RPS], ex[RPS], ey[RPS], Sx[RPS], Sy[RPS], Tx[RPS],
-        Ty[RPS];
+    MsRows<RPS> rw;
     const float2 Bl = splat(k.Bl), Cl = splat(k.Cl), Dl = splat(k.Dl);
     auto flush_rows = [&](int I) {
 #pragma unroll
@@ -916,8 +943,8 @@ __global__ void __launch_bounds__(MC_THREADS, 8) mlapm_sym_list_kernel(const flo
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
                 const int64_t j = static_cast<int64_t>(I) * MS_BLOCK + (2 * i + h) * THREADS + tid;
-                const float a0 = h ? Sx[i].y : Sx[i].x, a1 = h ? Sy[i].y : Sy[i].x;
-                const float a2 = h ? Tx[i].y : Tx[i].x, a3 = h ? Ty[i].y : Ty[i].x;
+                const float a0 = h ? rw.Sx[i].y : rw.Sx[i].x, a1 = h ? rw.Sy[i].y : rw.Sy[i].x;
+                const float a2 = h ? rw.Tx[i].y : rw.Tx[i].x, a3 = h ? rw.Ty[i].y : rw.Ty[i].x;
                 if (!isfinite(a0 + a1 + a2 + a3)) bad[j] = 1u;
                 unsigned long long *dst = acc + j * 4;
                 atomicAdd(dst + 0, static_cast<unsigned long long>(__float2ll_rn(-a0 * colscale)));
@@ -933,83 +960,18 @@ __global__ void __launch_bounds__(MC_THREADS, 8) mlapm_sym_list_kernel(const flo
     int t = 0;
     while (t < s_cnt) {
         const int I = meta[t & 1][0];
-#pragma unroll
-        for (int i = 0; i < RPS; ++i) {
-            const int64_t na = static_cast<int64_t>(I) * MS_BLOCK + (2 * i) * THREADS + tid;
-            const int64_t nb = na + THREADS;
-            const float4 a0 = rec[2 * na], a1 = rec[2 * na + 1], b0 = rec[2 * nb], b1 = rec[2 * nb + 1];
-            npx[i] = make_float2(-a0.x, -b0.x); npy[i] = make_float2(-a0.y, -b0.y);
-            vx[i] = make_float2(a0.z, b0.z); vy[i] = make_float2(a0.w, b0.w);
-            nvx[i] = make_float2(-a0.z, -b0.z); nvy[i] = make_float2(-a0.w, -b0.w);
-            ex[i] = make_float2(a1.x, b1.x); ey[i] = make_float2(a1.y, b1.y);
-            Sx[i] = Sy[i] = Tx[i] = Ty[i] = make_float2(0.f, 0.f);
-        }
+        ms_load_rows(rw, rec, I, tid);
         do {
         const int buf = t & 1;
         if (tid == 0 && t + 1 < s_cnt) stage_load(s_lo + t + 1, buf ^ 1);   // tile[buf^1] was released by the
         mbar_wait(&sm.bars[buf], (t >> 1) & 1);                   // the (t/2)-th use of this buffer
-        const float4 *tl = sm.tile[buf];
-        if (meta[buf][1] == 0) {
-            // diagonal block: rows and columns are the same agents, every ordered pair appears -> row direction only
-#pragma unroll 4
-            for (int j = 0; j < CT; ++j) {
-                const float4 cp = tl[2 * j];
-#pragma unroll
-                for (int i = 0; i < RPS; ++i)
-                    pair2<VERSION>(npx[i], npy[i], vx[i], vy[i], nvx[i], nvy[i], ex[i], ey[i], cp, Bl, Cl, Dl, Sx[i],
-                                   Sy[i], Tx[i], Ty[i]);
-            }
-        } else {
-            float4 *red = sm.red[warp];
-            for (int b = 0; b < CT / BATCH; ++b) {
-#pragma unroll
-                for (int c = 0; c < BATCH; ++c) {
-                    const float4 cp = tl[2 * (b * BATCH + c)];
-                    const float4 ce = tl[2 * (b * BATCH + c) + 1];
-                    float2 cSx, cSy, cTx, cTy;
-                    pair2sym<VERSION, true>(npx[0], npy[0], vx[0], vy[0], nvx[0], nvy[0], ex[0], ey[0], cp, ce, Bl, Cl,
-                                            Dl, Sx[0], Sy[0], Tx[0], Ty[0], cSx, cSy, cTx, cTy);
-#pragma unroll
-                    for (int i = 1; i < RPS; ++i)
-                        pair2sym<VERSION, false>(npx[i], npy[i], vx[i], vy[i], nvx[i], nvy[i], ex[i], ey[i], cp, ce,
-                                                 Bl, Cl, Dl, Sx[i], Sy[i], Tx[i], Ty[i], cSx, cSy, cTx, cTy);
-                    red[c * MS_RED_STRIDE + lane] = make_float4(cSx.x + cSx.y, cSy.x + cSy.y, cTx.x + cTx.y,
-                                                                cTy.x + cTy.y);
-                }
-                __syncwarp();
-                const float4 *col = red + (lane / LPC) * MS_RED_STRIDE + (lane % LPC);
-                float4 a = col[0];
-#pragma unroll
-                for (int e = 1; e < 32 / LPC; ++e) {
-                    const float4 t = col[LPC * e];
-                    a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
-                }
-#pragma unroll
-                for (int o = 1; o < LPC; o <<= 1) {
-                    a.x += __shfl_xor_sync(0xffffffffu, a.x, o);
-                    a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
-                    a.z += __shfl_xor_sync(0xffffffffu, a.z, o);
-                    a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
-                }
-                if (lane % LPC == 0) sm.colacc[warp][b * BATCH + lane / LPC] = a;
-                __syncwarp();
-            }
+        // the off-diagonal branch first: in the other order ptxas emits the diagonal loop twice
+        if (meta[buf][1] != 0) {
+            ms_pair_tile<VERSION>(rw, sm.tile[buf], sm.red[warp], sm.colacc[warp], lane, Bl, Cl, Dl);
             __syncthreads();
-            const int64_t j0 = meta[buf][2];
-            for (int c = tid; c < CT; c += THREADS) {
-                float4 a = sm.colacc[0][c];
-#pragma unroll
-                for (int wv = 1; wv < THREADS / 32; ++wv) {
-                    const float4 t = sm.colacc[wv][c];
-                    a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
-                }
-                if (!isfinite(a.x + a.y + a.z + a.w)) bad[j0 + c] = 1u;
-                unsigned long long *dst = acc + (j0 + c) * 4;
-                atomicAdd(dst + 0, static_cast<unsigned long long>(__float2ll_rn(a.x * colscale)));
-                atomicAdd(dst + 1, static_cast<unsigned long long>(__float2ll_rn(a.y * colscale)));
-                atomicAdd(dst + 2, static_cast<unsigned long long>(__float2ll_rn(a.z * colscale)));
-                atomicAdd(dst + 3, static_cast<unsigned long long>(__float2ll_rn(a.w * colscale)));
-            }
+            ms_add_columns<THREADS>(sm.colacc, acc, bad, meta[buf][2], colscale, tid);
+        } else {
+            ms_diag_tile<VERSION>(rw, sm.tile[buf], Bl, Cl, Dl);
         }
         __syncthreads();
         ++t;
@@ -1242,18 +1204,15 @@ __global__ void __launch_bounds__(MSC_THREADS) mlapm_scenes_kernel(
     }
     const MlConst k = sk[ls];
     const float2 p = sp[c0 + row], v = sv[c0 + row], d = dest[n];
-    // ed = F.normalize(destination - position)   (mlapm.py:21)
-    const float dx = __fsub_rn(d.x, p.x), dy = __fsub_rn(d.y, p.y);
-    const float dn = fmaxf(norm2_rn(dx, dy), 1e-12f);
-    const float ex = __fdiv_rn(dx, dn), ey = __fdiv_rn(dy, dn);
+    const float2 e = mlapm_dest_dir(p, d);
     float fx = 0.f, fy = 0.f;
     const float2 *cp = sp + c0, *cv = sv + c0;
     const uint8_t *ca = sa + c0;
 #pragma unroll 4
     for (int j = 0; j < N; ++j) {
         if (!ca[j]) continue;
-        if (EXACT) pair_exact<VERSION>(p.x, p.y, v.x, v.y, ex, ey, cp[j], cv[j], k, fx, fy);
-        else pair_fast<VERSION>(p.x, p.y, v.x, v.y, ex, ey, cp[j], cv[j], k, fx, fy);
+        if (EXACT) pair_exact<VERSION>(p.x, p.y, v.x, v.y, e.x, e.y, cp[j], cv[j], k, fx, fy);
+        else pair_fast<VERSION>(p.x, p.y, v.x, v.y, e.x, e.y, cp[j], cv[j], k, fx, fy);
     }
     const float dsx = ds[n * ds_dim];
     const float dsy = ds[n * ds_dim + (ds_dim > 1 ? 1 : 0)];
@@ -1294,34 +1253,19 @@ static void pick_split(int64_t nrows, int64_t N, int rows_per_cta, int tile, int
     *nsplit = static_cast<int>((N + cps - 1) / cps);
 }
 
-// Column splits for the packed kernel: enough CTAs for >= 8 waves over the resident slots (occupancy x SMs), each
-// split a whole number of tiles.  Measured at N = 100k (profiles/r01_mlapm_experiments.md): 27-36 splits (6-8 waves)
-// are ~2% faster than the exact 2- or 4-wave fits (9, 18), 4 splits (1 wave) 18% slower.  PIML_MLAPM_SPLIT overrides.
-static int pick_split2(const void *kernel, int64_t nrows, int64_t N, int rows_per_cta, int *nsplit,
-                       int *cols_per_split) {
-    static const void *cached_kernel = nullptr;
-    static int cached_occ = 0;
-    if (kernel != cached_kernel) {
-        int occ = 0;
-        PIML_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, M2_THREADS, 0));
-        cached_occ = occ < 1 ? 1 : occ;
-        cached_kernel = kernel;
-    }
-    (void)nrows; (void)rows_per_cta;
-    // The column partition depends on N ONLY: a row's sum is then evaluated in the same order whichever row range
-    // (rank) it is computed in, so an agent-sharded crowd is bit-identical to the unsharded one (SURVEY.md A.2b).
-    // As many splits as allowed also gives every rank of an 8-way shard enough CTAs to fill its GPU.
+// Column splits for the packed kernel, each a whole number of tiles: one tile per split up to ML_MAX_SPLIT.  Measured
+// at N = 100k (profiles/r01_mlapm_experiments.md): 27-36 splits (6-8 waves) are ~2% faster than the exact 2- or 4-wave
+// fits (9, 18), 4 splits (1 wave) 18% slower.
+// The column partition depends on N ONLY: a row's sum is then evaluated in the same order whichever row range (rank) it
+// is computed in, so an agent-sharded crowd is bit-identical to the unsharded one (SURVEY.md A.2b).  As many splits as
+// allowed also gives every rank of an 8-way shard enough CTAs to fill its GPU.
+static void pick_split2(int64_t N, int *nsplit, int *cols_per_split) {
     const int64_t tiles = (N + M2_TILE - 1) / M2_TILE;
     int64_t s = tiles < ML_MAX_SPLIT ? tiles : ML_MAX_SPLIT;
     if (s < 1) s = 1;
-    if (const char *e = getenv("PIML_MLAPM_SPLIT")) {
-        const int64_t f = atoll(e);
-        if (f >= 1 && f <= ML_MAX_SPLIT && f <= tiles) s = f;
-    }
     const int64_t per = (tiles + s - 1) / s;
     *cols_per_split = static_cast<int>(per * M2_TILE);
     *nsplit = static_cast<int>((tiles + per - 1) / per);
-    return PIML_OK;
 }
 
 template <int VERSION, bool EXACT>
@@ -1333,6 +1277,15 @@ static void launch_pairs(int R, dim3 grid, cudaStream_t st, const float2 *pos, c
         mlapm_pairs_kernel<VERSION, 2, EXACT><<<grid, ML_THREADS, 0, st>>>(pos, vel, dest, N, row0, row1, cps, k, partial);
     else
         mlapm_pairs_kernel<VERSION, 1, EXACT><<<grid, ML_THREADS, 0, st>>>(pos, vel, dest, N, row0, row1, cps, k, partial);
+}
+
+template <int VERSION>
+static void launch_pairs2(int RP, dim3 grid, cudaStream_t st, const float2 *pos, const float2 *vel, const float2 *dest,
+                          const float4 *col8, int N, int row0, int row1, int cps, const M2Const &k, float4 *partial) {
+    if (RP == 2)
+        mlapm_pairs2_kernel<VERSION, 2><<<grid, M2_THREADS, 0, st>>>(pos, vel, dest, col8, N, row0, row1, cps, k, partial);
+    else
+        mlapm_pairs2_kernel<VERSION, 1><<<grid, M2_THREADS, 0, st>>>(pos, vel, dest, col8, N, row0, row1, cps, k, partial);
 }
 
 }  // namespace piml
@@ -1347,10 +1300,6 @@ static int64_t sym_blocks(int64_t N) { return (N + MS_BLOCK - 1) / MS_BLOCK; }
 // Block pairs per CTA for nI row blocks of a crowd of T blocks: >= 64 CTAs per SM (measured best at N = 100k on one
 // GPU: 2; an 8-way shard of the same crowd gets 1).
 static int sym_per(int64_t nI, int64_t T) {
-    if (const char *e = getenv("PIML_MLAPM_SYM_PER")) {
-        const int f = atoi(e);
-        if (f >= 1) return f;
-    }
     const int64_t pairs = nI * (T / 2 + 1), want = 64LL * sm_count();
     const int64_t per = pairs / want;
     return per < 1 ? 1 : static_cast<int>(per);
@@ -1358,10 +1307,6 @@ static int sym_per(int64_t nI, int64_t T) {
 // CTAs per block pair (1, 2 or 4 = the 4 column stages of a pair split over that many CTAs): a shard with few row
 // blocks (8 ranks at N = 100k: 25 blocks x 99 pairs) would otherwise run ~2 waves of CTAs with a nearly empty last one.
 static int sym_sub(int64_t nI, int64_t T, int per) {
-    if (const char *e = getenv("PIML_MLAPM_SYM_SUB")) {
-        const int f = atoi(e);
-        if (f == 1 || f == 2 || f == 4) return f;
-    }
     const int64_t ctas = nI * ((T / 2 + 1 + per - 1) / per), wave = 8LL * sm_count();
     int sub = 1;
     while (sub < MS_BLOCK / MS_CT && ctas * sub < 6 * wave) sub *= 2;
@@ -1374,15 +1319,37 @@ static int sym_splits(int64_t nI, int64_t T, int *per, int *sub) {
     return static_cast<int>((T / 2 + 1 + *per - 1) / *per) * *sub;
 }
 
-// Dense symmetric evaluation: records (32 B per agent) + row-direction partials (16 B per agent and split) +
-// column-direction fixed-point accumulators (4 x int64 per agent) + poison flags: O(N) -- 0.15 GB at N = 10^6 (the
-// per-pair column partials this replaces: 15.6 GB)
-static int64_t sym_workspace_bytes(int64_t N) {
-    const int64_t T = sym_blocks(N), npad = T * MS_BLOCK;
-    int per_, sub_;
-    const int64_t S = sym_splits(T, T, &per_, &sub_);
-    return npad * MS_RECF * sizeof(float) + S * npad * 4 * sizeof(float) + npad * 4 * sizeof(long long) +
-           npad * sizeof(unsigned) + 256;
+// Consecutive 256-byte aligned regions of a workspace; base == nullptr only adds up their sizes.
+struct WsCarve {
+    char *base;
+    int64_t off;
+    void *take(int64_t bytes) {
+        char *q = base ? base + off : nullptr;
+        off += (bytes + 255) / 256 * 256;
+        return q;
+    }
+};
+// The caller's workspace rounded up to 256 bytes (every layout's total has room for it).
+static void *ws_align(const void *ws) {
+    return reinterpret_cast<void *>((reinterpret_cast<uintptr_t>(ws) + 255) & ~static_cast<uintptr_t>(255));
+}
+
+// Dense symmetric evaluation (mlapm_sym_kernel) of a crowd split over `world` ranks (1: the whole crowd): records (32 B
+// per agent), the row-direction partials of the largest shard (16 B per row and split, so that every rank's layout is
+// the same), column-direction fixed-point accumulators (4 x int64 per agent) and poison flags: O(N) -- 0.15 GB at
+// N = 10^6 (the per-pair column partials this replaces: 15.6 GB).
+struct SymLayout { int per, sub, S; float4 *rec, *partialR; long long *colsum; unsigned *bad; int64_t total; };
+static SymLayout sym_layout(int64_t N, int world, void *base) {
+    const int64_t T = sym_blocks(N), npad = T * MS_BLOCK, nI = (T + world - 1) / world;
+    SymLayout l{};
+    l.S = sym_splits(nI, T, &l.per, &l.sub);
+    WsCarve c{static_cast<char *>(base), 0};
+    l.rec = static_cast<float4 *>(c.take(npad * MS_RECF * sizeof(float)));
+    l.partialR = static_cast<float4 *>(c.take(l.S * nI * MS_BLOCK * sizeof(float4)));
+    l.colsum = static_cast<long long *>(c.take(npad * 4 * sizeof(long long)));
+    l.bad = static_cast<unsigned *>(c.take(npad * sizeof(unsigned)));
+    l.total = c.off + 256;                                        // + 256: room to align the caller's base
+    return l;
 }
 
 // Culled symmetric evaluation (mlapm_sym_list_kernel).  Candidates of the work list: T * (floor(T/2) + 1) * MC_SPB,
@@ -1408,30 +1375,24 @@ struct CullLayout {
 static CullLayout cull_layout(int64_t N, void *base) {
     const int64_t T = sym_blocks(N), npad = T * MS_BLOCK;
     CullLayout l{};
-    char *p = static_cast<char *>(base);
-    int64_t off = 0;
-    auto take = [&](int64_t bytes) {
-        char *q = p ? p + off : nullptr;
-        off += (bytes + 255) / 256 * 256;
-        return static_cast<void *>(q);
-    };
-    l.rec = static_cast<float4 *>(take(npad * MS_RECF * sizeof(float)));
-    l.acc = static_cast<long long *>(take(npad * 4 * sizeof(long long)));
-    l.bad = static_cast<unsigned *>(take(npad * sizeof(unsigned)));
+    WsCarve c{static_cast<char *>(base), 0};
+    l.rec = static_cast<float4 *>(c.take(npad * MS_RECF * sizeof(float)));
+    l.acc = static_cast<long long *>(c.take(npad * 4 * sizeof(long long)));
+    l.bad = static_cast<unsigned *>(c.take(npad * sizeof(unsigned)));
     for (int b = 0; b < 2; ++b) {
-        l.key[b] = static_cast<uint32_t *>(take(N * sizeof(uint32_t)));
-        l.val[b] = static_cast<int *>(take(N * sizeof(int)));
+        l.key[b] = static_cast<uint32_t *>(c.take(N * sizeof(uint32_t)));
+        l.val[b] = static_cast<int *>(c.take(N * sizeof(int)));
     }
-    l.slot = static_cast<int *>(take(N * sizeof(int)));
-    l.sbox = static_cast<float4 *>(take(T * MC_SPB * sizeof(float4)));
-    l.bbox = static_cast<float4 *>(take(T * sizeof(float4)));
-    l.sflag = static_cast<unsigned *>(take(T * MC_SPB * sizeof(unsigned)));
-    l.bflag = static_cast<unsigned *>(take(T * sizeof(unsigned)));
-    l.items = static_cast<int *>(take(cull_candidates(N) * sizeof(int)));
-    l.nitems = static_cast<int *>(take(sizeof(int)));
+    l.slot = static_cast<int *>(c.take(N * sizeof(int)));
+    l.sbox = static_cast<float4 *>(c.take(T * MC_SPB * sizeof(float4)));
+    l.bbox = static_cast<float4 *>(c.take(T * sizeof(float4)));
+    l.sflag = static_cast<unsigned *>(c.take(T * MC_SPB * sizeof(unsigned)));
+    l.bflag = static_cast<unsigned *>(c.take(T * sizeof(unsigned)));
+    l.items = static_cast<int *>(c.take(cull_candidates(N) * sizeof(int)));
+    l.nitems = static_cast<int *>(c.take(sizeof(int)));
     l.temp_bytes = cull_cub_bound(N);
-    l.temp = take(l.temp_bytes);
-    l.total = off + 256;                                          // + 256: room to align the caller's base
+    l.temp = c.take(l.temp_bytes);
+    l.total = c.off + 256;                                          // + 256: room to align the caller's base
     return l;
 }
 static int64_t cull_workspace_bytes(int64_t N) { return cull_layout(N, nullptr).total; }
@@ -1454,14 +1415,13 @@ extern "C" int piml_set_mlapm_algorithm(int algo) {
 
 extern "C" int64_t piml_mlapm_workspace_bytes_sym(int64_t N) {
     if (N <= 0) return 0;
-    const int64_t a = piml_mlapm_workspace_bytes(N), b = sym_workspace_bytes(N), c = cull_workspace_bytes(N);
+    const int64_t a = piml_mlapm_workspace_bytes(N), b = sym_layout(N, 1, nullptr).total, c = cull_workspace_bytes(N);
     return a > b ? (a > c ? a : c) : (b > c ? b : c);
 }
 
 extern "C" int piml_mlapm_cull_items(const void *workspace, int64_t N, int64_t *items) {
     PIML_REQUIRE(workspace && items && N > 0 && N < (1LL << 31), "piml_mlapm_cull_items: bad arguments");
-    const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~static_cast<uintptr_t>(255);
-    const CullLayout l = cull_layout(N, reinterpret_cast<void *>(base));
+    const CullLayout l = cull_layout(N, ws_align(workspace));
     int n = 0;
     PIML_CUDA(cudaMemcpy(&n, l.nitems, sizeof(int), cudaMemcpyDeviceToHost));
     *items = n;
@@ -1504,38 +1464,31 @@ extern "C" float piml_mlapm_cull_radius(const piml_mlapm_params *prm) {
     return cull_radius(prm, mlapm_consts(prm));
 }
 
-// prep + symmetric pair kernel for the row blocks [I0, I0 + nI) of a crowd of T blocks.
+// prep + symmetric pair kernel for the row blocks [I0, I0 + nI) of a crowd of T blocks, in workspace l; bad: the NaN
+// flags, or null.
 static int launch_sym_pairs(int version, const float2 *p2, const float2 *v2, const float2 *d2, int N, int64_t T,
-                            int64_t I0, int64_t nI, int per, int sub, int S, const MlConst &k, float4 *rec, float4 *partialR,
-                            long long *colsum, float colscale, unsigned *bad, cudaStream_t st) {
-    const int64_t D = T / 2, npad = T * MS_BLOCK;
+                            int64_t I0, int64_t nI, const SymLayout &l, const MlConst &k, float colscale,
+                            unsigned *bad, cudaStream_t st) {
+    const int64_t npad = T * MS_BLOCK;
     const int threads = 256;
     mlapm_prep_sym_kernel<<<static_cast<unsigned>((npad + threads - 1) / threads), threads, 0, st>>>(
-        p2, v2, d2, N, static_cast<int>(npad), rec, reinterpret_cast<ulonglong2 *>(colsum), bad);
+        p2, v2, d2, N, static_cast<int>(npad), l.rec, reinterpret_cast<ulonglong2 *>(l.colsum), bad);
     count_launch();
     int rc = check_launch("mlapm_prep_sym_kernel");
     if (rc) return rc;
-    M2Const k2{k.Bl, k.Cl, k.Dl};
-    dim3 grid(static_cast<unsigned>(nI), static_cast<unsigned>(S));
-    int cfg = 0;                                               // tuning: PIML_MLAPM_SYM_CFG = 0..3
-    if (const char *e = getenv("PIML_MLAPM_SYM_CFG")) cfg = atoi(e);
-#define PIML_LAUNCH_SYM(V, CT, BATCH, RPS)                                                                         \
-    do {                                                                                                           \
-        using Smem = MsSmem<CT, BATCH, MS_BLOCK / (2 * RPS)>;                                                      \
-        if (sizeof(Smem) > 48 * 1024)                    /* per device: a process may drive several GPUs */        \
-            PIML_CUDA(cudaFuncSetAttribute(mlapm_sym_kernel<V, CT, BATCH, RPS>,                                    \
-                                           cudaFuncAttributeMaxDynamicSharedMemorySize,                            \
-                                           static_cast<int>(sizeof(Smem))));                                       \
-        mlapm_sym_kernel<V, CT, BATCH, RPS><<<grid, MS_BLOCK / (2 * RPS), sizeof(Smem), st>>>(                     \
-            rec, static_cast<int>(T), static_cast<int>(D), static_cast<int>(I0), per, sub, k2, partialR,           \
-            static_cast<int>(nI * MS_BLOCK), reinterpret_cast<unsigned long long *>(colsum), colscale, bad);       \
-    } while (0)
+    const M2Const k2{k.Bl, k.Cl, k.Dl};
+    const dim3 grid(static_cast<unsigned>(nI), static_cast<unsigned>(l.S));
+    const int iT = static_cast<int>(T), iI0 = static_cast<int>(I0), nrows_pad = static_cast<int>(nI * MS_BLOCK);
+    unsigned long long *colsum = reinterpret_cast<unsigned long long *>(l.colsum);
+    static_assert(sizeof(MsSmem<MS_BLOCK / 4>) <= 48 * 1024 && sizeof(MsSmem<MS_BLOCK / 8>) <= 48 * 1024,
+                  "mlapm_sym_kernel: shared memory above the default limit");
     // measured at N = 100k (ms per step): 8 rows per thread (64 threads) 6.81, 4 rows (128 threads) 6.99, 2 rows 7.16
-    if (version == 0) PIML_LAUNCH_SYM(0, MS_CT, MS_BATCH, 2);
-    else if (cfg == 2) PIML_LAUNCH_SYM(1, 128, 8, 2);
-    else if (cfg == 4) PIML_LAUNCH_SYM(1, 128, 8, 1);
-    else PIML_LAUNCH_SYM(1, MS_CT, MS_BATCH, 4);
-#undef PIML_LAUNCH_SYM
+    if (version == 0)
+        mlapm_sym_kernel<0, 2><<<grid, MS_BLOCK / 4, sizeof(MsSmem<MS_BLOCK / 4>), st>>>(
+            l.rec, iT, iT / 2, iI0, l.per, l.sub, k2, l.partialR, nrows_pad, colsum, colscale, bad);
+    else
+        mlapm_sym_kernel<1, 4><<<grid, MS_BLOCK / 8, sizeof(MsSmem<MS_BLOCK / 8>), st>>>(
+            l.rec, iT, iT / 2, iI0, l.per, l.sub, k2, l.partialR, nrows_pad, colsum, colscale, bad);
     count_launch();
     return check_launch("mlapm_sym_kernel");
 }
@@ -1582,7 +1535,7 @@ static int launch_sym_culled(int version, const float2 *p2, const float2 *v2, co
     temp_bytes = static_cast<size_t>(l.temp_bytes);
     PIML_CUDA(cub::DeviceSelect::If(l.temp, temp_bytes, cand, l.items, l.nitems, ncand, keep, st));
     count_launch(2);                                              // tile-state init + select
-    using Smem = MsSmem<MS_CT, MS_BATCH, MC_THREADS>;
+    using Smem = MsSmem<MC_THREADS>;
     static_assert(sizeof(Smem) <= 48 * 1024, "mlapm_sym_list_kernel: shared memory above the default limit");
     const void *kfn = version == 0 ? reinterpret_cast<const void *>(&mlapm_sym_list_kernel<0>)
                                    : reinterpret_cast<const void *>(&mlapm_sym_list_kernel<1>);
@@ -1659,91 +1612,56 @@ static int mlapm_advance_impl(const float *pos, const float *vel, const float *d
     }
     // production, whole crowd: symmetric evaluation (every unordered pair once) when the caller's workspace holds
     // the column-direction sums; row ranges (agent-sharded ranks) and small crowds use the ordered-pair kernel.
+    int nsplit = 0;                                                // row-direction partials of the finalize kernel
+    const float4 *partial = nullptr;
     SymPartials symp{nullptr, 0.f, 0, nullptr, 0, 0, nullptr, nullptr};
     const bool sym_ok = row0 == 0 && row1 == N && sym_params_ok(prm, k, N);
     const bool want_sym = g_mlapm_algorithm >= 2 || (g_mlapm_algorithm == 0 && N >= MS_AUTO_MIN_AGENTS);
-    // culled (0, 2): skips the work beyond the radius where the weight is exactly 0; the list index is an int
     if (sym_ok && want_sym && g_mlapm_algorithm != 3 && workspace_bytes >= cull_workspace_bytes(N) &&
         cull_candidates(N) < (int64_t{1} << 31)) {
-        const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~static_cast<uintptr_t>(255);
-        const CullLayout l = cull_layout(N, reinterpret_cast<void *>(base));
+        // culled (0, 2): skips the work beyond the radius where the weight is exactly 0; the list index is an int
+        const CullLayout l = cull_layout(N, ws_align(workspace));
         const int sl = sym_colscale_log2(N, prm);
         rc = launch_sym_culled(prm->version, p2, v2, d2, iN, k, cull_radius(prm, k), l, ldexpf(1.0f, sl), st);
         if (rc) return rc;
         symp = SymPartials{l.acc, ldexpf(1.0f, -sl), 0, nullptr, 0, 0, l.slot, l.bad};
-        const int threads = 256;
-        mlapm_finalize2_kernel<<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0, st>>>(
-            p2, v2, desired_speed, ds_dim, d2, r0, r1, 0, nullptr, prm->A, k.cos_t, k.sin_t, prm->version, prm->tau,
-            dt, radius, reinterpret_cast<float2 *>(action), reinterpret_cast<float2 *>(pos_new), arrived, push, symp);
-        count_launch();
-        return check_launch("mlapm_finalize2_kernel");
-    }
-    // dense (3, or a workspace without room for the culled path's list)
-    if (sym_ok && want_sym && workspace_bytes >= sym_workspace_bytes(N)) {
-        const int64_t T = sym_blocks(N), D = T / 2, npad = T * MS_BLOCK;
-        int per, sub;
-        const int S = sym_splits(T, T, &per, &sub);
-        float4 *rec = reinterpret_cast<float4 *>(workspace);
-        float4 *partialR = rec + npad * 2;
-        long long *colsum = reinterpret_cast<long long *>(partialR + static_cast<int64_t>(S) * npad);
-        unsigned *bad = reinterpret_cast<unsigned *>(colsum + npad * 4);
+    } else if (sym_ok && want_sym && workspace_bytes >= sym_layout(N, 1, nullptr).total) {
+        // dense (3, or a workspace without room for the culled path's list)
+        const int64_t T = sym_blocks(N);
+        const SymLayout l = sym_layout(N, 1, ws_align(workspace));
         const int sl = sym_colscale_log2(N, prm);
-        rc = launch_sym_pairs(prm->version, p2, v2, d2, iN, T, 0, T, per, sub, S, k, rec, partialR, colsum,
-                              ldexpf(1.0f, sl), bad, st);
+        rc = launch_sym_pairs(prm->version, p2, v2, d2, iN, T, 0, T, l, k, ldexpf(1.0f, sl), l.bad, st);
         if (rc) return rc;
-        const int threads = 256;
-        (void)D;
-        symp = SymPartials{colsum, ldexpf(1.0f, -sl), static_cast<int>(npad), nullptr, 0, 0, nullptr, bad};
-        mlapm_finalize2_kernel<<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0, st>>>(
-            p2, v2, desired_speed, ds_dim, d2, r0, r1, S, partialR, prm->A, k.cos_t, k.sin_t, prm->version, prm->tau,
-            dt, radius, reinterpret_cast<float2 *>(action), reinterpret_cast<float2 *>(pos_new), arrived, push, symp);
-        count_launch();
-        return check_launch("mlapm_finalize2_kernel");
-    }
-    // ordered pairs: packed-FP32 kernel on 16 B column records
-    const int64_t npad = (N + M2_TILE - 1) / M2_TILE * M2_TILE;
-    float4 *col8 = reinterpret_cast<float4 *>(workspace);
-    float4 *partial4 = col8 + npad;
-    {
+        nsplit = l.S;
+        partial = l.partialR;
+        symp = SymPartials{l.colsum, ldexpf(1.0f, -sl), static_cast<int>(T * MS_BLOCK), nullptr, 0, 0, nullptr, l.bad};
+    } else {
+        // ordered pairs: packed-FP32 kernel on 16 B column records
+        const int64_t npad = (N + M2_TILE - 1) / M2_TILE * M2_TILE;
+        float4 *col8 = reinterpret_cast<float4 *>(workspace);
+        float4 *partial4 = col8 + npad;
         const int threads = 256;
         mlapm_prep_kernel<<<static_cast<unsigned>((npad + threads - 1) / threads), threads, 0, st>>>(
             p2, v2, iN, static_cast<int>(npad), col8);
         count_launch();
         rc = check_launch("mlapm_prep_kernel");
         if (rc) return rc;
+        const int RP = pick_row_pairs(nrows, N);
+        int cps;
+        pick_split2(N, &nsplit, &cps);
+        const dim3 grid(static_cast<unsigned>((nrows + M2_THREADS * 2 * RP - 1) / (M2_THREADS * 2 * RP)),
+                        static_cast<unsigned>(nsplit));
+        const M2Const k2{k.Bl, k.Cl, k.Dl};
+        if (prm->version == 0) launch_pairs2<0>(RP, grid, st, p2, v2, d2, col8, iN, r0, r1, cps, k2, partial4);
+        else launch_pairs2<1>(RP, grid, st, p2, v2, d2, col8, iN, r0, r1, cps, k2, partial4);
+        count_launch();
+        rc = check_launch("mlapm_pairs2_kernel");
+        if (rc) return rc;
+        partial = partial4;
     }
-    int RP = pick_row_pairs(nrows, N), unroll = 4;
-    if (const char *e = getenv("PIML_MLAPM_EXP")) sscanf(e, "%d,%d", &RP, &unroll);            // tuning experiments
-    M2Const k2{k.Bl, k.Cl, k.Dl};
-    dim3 grid;
-    int nsplit = 1, cps = 0, rc2 = PIML_OK;
-#define PIML_LAUNCH_PAIRS2(V, RPV, UN)                                                                             \
-    do {                                                                                                           \
-        rc2 = pick_split2(reinterpret_cast<const void *>(&mlapm_pairs2_kernel<V, RPV, UN>), nrows, N,              \
-                          M2_THREADS * 2 * RPV, &nsplit, &cps);                                                    \
-        grid = dim3(static_cast<unsigned>((nrows + M2_THREADS * 2 * RPV - 1) / (M2_THREADS * 2 * RPV)),            \
-                    static_cast<unsigned>(nsplit));                                                                \
-        if (rc2 == PIML_OK)                                                                                        \
-            mlapm_pairs2_kernel<V, RPV, UN><<<grid, M2_THREADS, 0, st>>>(p2, v2, d2, col8, iN, r0, r1, cps, k2,    \
-                                                                         partial4);                                \
-    } while (0)
-    if (prm->version == 0) {
-        if (RP == 2) PIML_LAUNCH_PAIRS2(0, 2, 4); else PIML_LAUNCH_PAIRS2(0, 1, 4);
-    } else if (RP == 4) {
-        PIML_LAUNCH_PAIRS2(1, 4, 2);
-    } else if (RP == 2) {
-        if (unroll == 2) PIML_LAUNCH_PAIRS2(1, 2, 2); else PIML_LAUNCH_PAIRS2(1, 2, 4);
-    } else {
-        if (unroll == 2) PIML_LAUNCH_PAIRS2(1, 1, 2); else PIML_LAUNCH_PAIRS2(1, 1, 4);
-    }
-    if (rc2) return rc2;
-#undef PIML_LAUNCH_PAIRS2
-    count_launch();
-    rc = check_launch("mlapm_pairs2_kernel");
-    if (rc) return rc;
     const int threads = 256;
     mlapm_finalize2_kernel<<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0, st>>>(
-        p2, v2, desired_speed, ds_dim, d2, r0, r1, nsplit, partial4, prm->A, k.cos_t, k.sin_t, prm->version, prm->tau,
+        p2, v2, desired_speed, ds_dim, d2, r0, r1, nsplit, partial, prm->A, k.cos_t, k.sin_t, prm->version, prm->tau,
         dt, radius, reinterpret_cast<float2 *>(action), reinterpret_cast<float2 *>(pos_new), arrived, push, symp);
     count_launch();
     return check_launch("mlapm_finalize2_kernel");
@@ -1886,14 +1804,10 @@ extern "C" int64_t piml_mlapm_sym_inbox_bytes(int64_t N, int world) {
 
 extern "C" int64_t piml_mlapm_sym_shard_workspace_bytes(int64_t N, int world) {
     if (N <= 0 || world < 1 || world > ML_MAX_PEERS) return 0;
-    const int64_t T = sym_blocks(N), npad = T * MS_BLOCK;
-    const int64_t nI = (T + world - 1) / world;
-    int per_, sub_;
-    const int64_t S = sym_splits(nI, T, &per_, &sub_);
-    return npad * MS_RECF * sizeof(float) + S * nI * MS_BLOCK * 4 * sizeof(float) + npad * 4 * sizeof(long long) + 256;
+    return sym_layout(N, world, nullptr).total;
 }
 
-struct SymShardPlan { int64_t T, D, npad, I0, nI; int per, sub, S; float4 *rec, *partialR; long long *colsum; };
+struct SymShardPlan { int64_t T, I0, nI; SymLayout l; };
 
 static int sym_shard_plan(int64_t N, int world, int rank, void *workspace, int64_t workspace_bytes, SymShardPlan *pl) {
     PIML_REQUIRE(N > 0 && N < (1LL << 31) && world >= 1 && world <= ML_MAX_PEERS && rank >= 0 && rank < world,
@@ -1903,17 +1817,11 @@ static int sym_shard_plan(int64_t N, int world, int rank, void *workspace, int64
                  static_cast<long long>(piml_mlapm_sym_shard_workspace_bytes(N, world)));
     pl->T = sym_blocks(N);
     PIML_REQUIRE(pl->T >= world, "piml_mlapm_sym: fewer blocks than ranks");
-    pl->D = pl->T / 2;
-    pl->npad = pl->T * MS_BLOCK;
     int Ib[ML_MAX_PEERS + 1];
     sym_block_bounds(pl->T, world, Ib);
     pl->I0 = Ib[rank];
     pl->nI = Ib[rank + 1] - Ib[rank];
-    pl->S = sym_splits((pl->T + world - 1) / world, pl->T, &pl->per, &pl->sub);
-    pl->rec = reinterpret_cast<float4 *>(workspace);
-    pl->partialR = pl->rec + pl->npad * 2;
-    // the largest shard's row partials, so that every rank's layout is the same
-    pl->colsum = reinterpret_cast<long long *>(pl->partialR + static_cast<int64_t>(pl->S) * ((pl->T + world - 1) / world) * MS_BLOCK);
+    pl->l = sym_layout(N, world, ws_align(workspace));
     return PIML_OK;
 }
 
@@ -1932,8 +1840,8 @@ extern "C" int piml_mlapm_sym_pairs_push_f32(const float *pos, const float *vel,
     if (rc) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     rc = launch_sym_pairs(prm->version, reinterpret_cast<const float2 *>(pos), reinterpret_cast<const float2 *>(vel),
-                          reinterpret_cast<const float2 *>(dest), static_cast<int>(N), pl.T, pl.I0, pl.nI, pl.per, pl.sub, pl.S,
-                          k, pl.rec, pl.partialR, pl.colsum, ldexpf(1.0f, sym_colscale_log2(N, prm)), nullptr, st);
+                          reinterpret_cast<const float2 *>(dest), static_cast<int>(N), pl.T, pl.I0, pl.nI, pl.l, k,
+                          ldexpf(1.0f, sym_colscale_log2(N, prm)), nullptr, st);
     if (rc) return rc;
     PeerInbox peers;
     peers.world = world;
@@ -1948,7 +1856,7 @@ extern "C" int piml_mlapm_sym_pairs_push_f32(const float *pos, const float *vel,
     }
     const int threads = 256;
     mlapm_sym_colpush_kernel<<<static_cast<unsigned>((N + threads - 1) / threads), threads, 0, st>>>(
-        pl.colsum, ldexpf(1.0f, -sym_colscale_log2(N, prm)), static_cast<int>(N), peers);
+        pl.l.colsum, ldexpf(1.0f, -sym_colscale_log2(N, prm)), static_cast<int>(N), peers);
     count_launch();
     return check_launch("mlapm_sym_colpush_kernel");
 }
@@ -1984,7 +1892,7 @@ extern "C" int piml_mlapm_sym_finalize_push_f32(const float *pos, const float *v
     mlapm_finalize2_kernel<<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0,
                              static_cast<cudaStream_t>(stream)>>>(
         reinterpret_cast<const float2 *>(pos), reinterpret_cast<const float2 *>(vel), desired_speed, ds_dim,
-        reinterpret_cast<const float2 *>(dest), static_cast<int>(row0), static_cast<int>(row1), pl.S, pl.partialR,
+        reinterpret_cast<const float2 *>(dest), static_cast<int>(row0), static_cast<int>(row1), pl.l.S, pl.l.partialR,
         prm->A, k.cos_t, k.sin_t, prm->version, prm->tau, dt, radius, nullptr, nullptr, arrived, push, symp);
     count_launch();
     return check_launch("mlapm_finalize2_kernel");

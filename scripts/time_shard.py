@@ -8,4 +8,4 @@ p, v, ds, dest, _ = [x.to(dev) for x in bench.synthetic_crowd(N)]
 model = P.MLAPM(**bench.MLAPM_KW)
 for rows in (12500, 25000, 50000, 100000):
     ms = timeit(lambda: model.advance(p, v, ds, dest, bench.DT, bench.RADIUS, rows=(0, rows)), iters=10)
-    print(f"EXP={os.environ.get('PIML_MLAPM_EXP','auto')} rows={rows}: {ms:.3f} ms  ({rows*N/ms/1e9:.1f} Gpairs/s, ideal share of 9.49 ms: {9.49*rows/N:.3f})")
+    print(f"rows={rows}: {ms:.3f} ms  ({rows*N/ms/1e9:.1f} Gpairs/s, ideal share of 9.49 ms: {9.49*rows/N:.3f})")
