@@ -192,8 +192,8 @@ PIML_API int piml_set_mlapm_algorithm(int algo);
  * below -126), plus 1 % + 0.01 m for approximate rsqrt and fp32 rounding.  +inf where nothing can be skipped:
  * exact_math, or a weight that does not decay with distance (B + |D| >= 0). */
 PIML_API float piml_mlapm_cull_radius(const piml_mlapm_params *prm);
-/* Diagnostics: the length of the work list (row block x 128-column stage items) that the last culled symmetric step
- * of N agents built in `workspace`.  Synchronous (waits for the device). */
+/* Diagnostics: the number of live (128-row tile x 32-column tile) units that the last culled symmetric step of N
+ * agents evaluated from `workspace`.  Synchronous (waits for the device). */
 PIML_API int piml_mlapm_cull_items(const void *workspace, int64_t N, int64_t *items);
 PIML_API int piml_mlapm_advance_ws_f32(const float *pos, const float *vel, const float *desired_speed, int ds_dim,
                               const float *dest, int64_t N, int64_t row0, int64_t row1,

@@ -1,7 +1,7 @@
 // mlapm.cu -- all-pairs MLAPM force for sm_100a.
 //
-// The whole-crowd production path (mlapm_sym_list_kernel) evaluates every unordered pair once and skips the pairs
-// farther apart than the radius where the fp32 weight is exactly 0 (a spatial sort, boxes per block and a work list
+// The whole-crowd production path (mlapm_sym_tiles_kernel) evaluates every unordered pair once and skips the pairs
+// farther apart than the radius where the fp32 weight is exactly 0 (a spatial sort, boxes per tile and a work list
 // built on the device); the dense kernels below evaluate every pair (row ranges, small crowds, validation).
 //
 // Replaces MLAPM.step (reference src/models/mlapm.py:10-58) and the loop body of src/main_mlapm.py:19-34.
@@ -23,8 +23,11 @@
 #include <stdlib.h>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 #include <cub/iterator/counting_input_iterator.cuh>
+#include <thrust/iterator/counting_iterator.h>
+#include <thrust/iterator/transform_iterator.h>
 
 #include "common.cuh"
 
@@ -582,14 +585,13 @@ struct MsRows {
         Ty[RPS];
 };
 
-// Rows of block I: lanes x / y of pair i are the block's rows (2i) THREADS + tid and (2i + 1) THREADS + tid, with the
-// CTA's THREADS = MS_BLOCK / (2 RPS) threads; the sums start at 0.
-template <int RPS>
-__device__ __forceinline__ void ms_load_rows(MsRows<RPS> &r, const float4 *__restrict__ rec, int I, int tid) {
-    constexpr int THREADS = MS_BLOCK / (2 * RPS);
+// The 2 * RPS * THREADS rows from slot j0: lanes x / y of pair i are the rows j0 + (2i) THREADS + tid and
+// j0 + (2i + 1) THREADS + tid; the sums start at 0.
+template <int RPS, int THREADS>
+__device__ __forceinline__ void ms_load_rows(MsRows<RPS> &r, const float4 *__restrict__ rec, int64_t j0, int tid) {
 #pragma unroll
     for (int i = 0; i < RPS; ++i) {
-        const int64_t na = static_cast<int64_t>(I) * MS_BLOCK + (2 * i) * THREADS + tid;
+        const int64_t na = j0 + (2 * i) * THREADS + tid;
         const int64_t nb = na + THREADS;
         const float4 a0 = rec[2 * na], a1 = rec[2 * na + 1], b0 = rec[2 * nb], b1 = rec[2 * nb + 1];
         r.npx[i] = make_float2(-a0.x, -b0.x); r.npy[i] = make_float2(-a0.y, -b0.y);
@@ -600,12 +602,12 @@ __device__ __forceinline__ void ms_load_rows(MsRows<RPS> &r, const float4 *__res
     }
 }
 
-// One staged tile of MS_CT column records `tl` of the rows' own (diagonal) block: every ordered pair appears, so each
-// is evaluated in the row direction only (pair2).
-template <int VERSION, int RPS>
+// One staged tile of CT column records `tl` of the rows' own columns: every ordered pair appears, so each is evaluated
+// in the row direction only (pair2).
+template <int VERSION, int RPS, int CT>
 __device__ __forceinline__ void ms_diag_tile(MsRows<RPS> &r, const float4 *tl, float2 Bl, float2 Cl, float2 Dl) {
 #pragma unroll 4
-    for (int j = 0; j < MS_CT; ++j) {
+    for (int j = 0; j < CT; ++j) {
         const float4 cp = tl[2 * j];
 #pragma unroll
         for (int i = 0; i < RPS; ++i)
@@ -614,15 +616,16 @@ __device__ __forceinline__ void ms_diag_tile(MsRows<RPS> &r, const float4 *tl, f
     }
 }
 
-// One staged tile of MS_CT column records `tl` of another block: every pair feeds both directions (pair2sym).  The
-// warp's column-direction sums go to colacc[column]: the two packed lanes are added, each lane parks its sums of a
-// batch of MS_BATCH columns in the warp's scratch `red`, the warp transposes (lane -> column lane/LPC, every LPC-th
-// entry) and finishes with shuffles.
-template <int VERSION, int RPS>
-__device__ __forceinline__ void ms_pair_tile(MsRows<RPS> &r, const float4 *tl, float4 *red, float4 *colacc, int lane,
-                                             float2 Bl, float2 Cl, float2 Dl) {
+// One staged tile of CT column records `tl` of other rows: every pair feeds both directions (pair2sym).  The warp's
+// column-direction sum of column c goes to sink(c, sum), called by one lane per column: the two packed lanes are
+// added, each lane parks its sums of a batch of MS_BATCH columns in the warp's scratch `red`, the warp transposes
+// (lane -> column lane/LPC, every LPC-th entry) and finishes with shuffles.
+template <int VERSION, int RPS, int CT, class Sink>
+__device__ __forceinline__ void ms_pair_tile(MsRows<RPS> &r, const float4 *tl, float4 *red, int lane, float2 Bl,
+                                             float2 Cl, float2 Dl, Sink sink) {
+    static_assert(CT % MS_BATCH == 0, "bad stage shape");
     constexpr int LPC = 32 / MS_BATCH;                      // lanes that share a column in the transposed sum
-    for (int b = 0; b < MS_CT / MS_BATCH; ++b) {
+    for (int b = 0; b < CT / MS_BATCH; ++b) {
 #pragma unroll
         for (int c = 0; c < MS_BATCH; ++c) {
             const float4 cp = tl[2 * (b * MS_BATCH + c)];
@@ -651,7 +654,7 @@ __device__ __forceinline__ void ms_pair_tile(MsRows<RPS> &r, const float4 *tl, f
             a.z += __shfl_xor_sync(0xffffffffu, a.z, o);
             a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
         }
-        if (lane % LPC == 0) colacc[b * MS_BATCH + lane / LPC] = a;
+        if (lane % LPC == 0) sink(b * MS_BATCH + lane / LPC, a);
         __syncwarp();
     }
 }
@@ -713,7 +716,7 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
     const int d_hi = min(d_lo + per, L);
 
     MsRows<RPS> rw;
-    ms_load_rows(rw, rec, I, tid);
+    ms_load_rows<RPS, THREADS>(rw, rec, static_cast<int64_t>(I) * MS_BLOCK, tid);
     const float2 Bl = splat(k.Bl), Cl = splat(k.Cl), Dl = splat(k.Dl);
 
     const int nst = d_hi > d_lo ? (d_hi - d_lo) * spc : 0;
@@ -738,11 +741,13 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
         phase_bits ^= (1u << buf);
         // the off-diagonal branch first: in the other order ptxas emits the diagonal loop twice
         if (d_lo + s / spc != 0) {
-            ms_pair_tile<VERSION>(rw, sm.tile[buf], sm.red[warp], sm.colacc[warp], lane, Bl, Cl, Dl);
+            float4 *colacc = sm.colacc[warp];
+            ms_pair_tile<VERSION, RPS, MS_CT>(rw, sm.tile[buf], sm.red[warp], lane, Bl, Cl, Dl,
+                                              [colacc](int c, float4 a) { colacc[c] = a; });
             __syncthreads();
             ms_add_columns<THREADS>(sm.colacc, colsum, bad, stage_j0(s), colscale, tid);
         } else {
-            ms_diag_tile<VERSION>(rw, sm.tile[buf], Bl, Cl, Dl);
+            ms_diag_tile<VERSION, RPS, MS_CT>(rw, sm.tile[buf], Bl, Cl, Dl);
         }
         __syncthreads();
     }
@@ -764,16 +769,24 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
 //
 // Per call: (1) a 32-bit Hilbert key of each agent's 4 m cell, sorted stably (cub::DeviceRadixSort, key + agent
 // index), so that the agents of a 512-block live close together; (2) records in sorted order plus an axis-aligned box
-// per 512-agent block and per 128-agent column stage; (3) the work list: every (row block I, column block J = I + d
-// mod T, stage) item of the circulant schedule whose boxes are within r_cut, compacted in order (cub::DeviceSelect);
-// (4) a persistent pair kernel over the list; (5) the finalize kernel reads each agent's sums through its sorted slot.
-// Row and column directions both go into the crowd-wide int64 fixed-point accumulators, so the result does not depend
-// on how the list is cut over the CTAs.
+// per 512-agent block, per 128-agent row tile and per 32-agent column tile; (3) the work list: every (row tile R of
+// block I, column block J = I + d mod T) item of the circulant schedule whose boxes are within r_cut, compacted in
+// order (cub::DeviceSelect), the mask of its column tiles within r_cut, and the exclusive scan of the masks' popcounts
+// (cub::DeviceScan): the live (row tile, column tile) units; (4) a persistent pair kernel over the units; (5) the
+// finalize kernel reads each agent's sums through its sorted slot.  Row and column directions both go into the
+// crowd-wide int64 fixed-point accumulators, so the result does not depend on how the units are cut over the CTAs.
+// Every unordered pair once: d >= 1 takes the 16 column tiles of block J in both directions; d = 0 takes the column
+// tiles of the row tiles r' > r of the own block in both directions and the row tile's own 4 column tiles in the row
+// direction only (every ordered pair of the row tile appears there); r' < r belongs to row tile r'.
 // =====================================================================================================================
 constexpr float MC_CELL = 4.0f;                   // metres per cell of the sort key
-constexpr int MC_SPB = MS_BLOCK / MS_CT;          // column stages per block
-constexpr int MC_THREADS = 64;                    // pair kernel: 8 rows per thread (the dense kernel's measured best)
+constexpr int MC_RT = 128;                        // rows per row tile
+constexpr int MC_CT = 32;                         // columns per column tile: one warp of the prep kernel, 1 KB
+constexpr int MC_RPB = MS_BLOCK / MC_RT;          // row tiles per block
+constexpr int MC_CPB = MS_BLOCK / MC_CT;          // column tiles per block: one bit each in a uint16_t mask
+constexpr int MC_THREADS = 32;                    // pair kernel: one warp per row tile, 4 rows per thread
 constexpr unsigned MC_NEAR_ALL = 1u, MC_EMPTY = 2u;   // box flags: holds a NaN / inf, holds no agent
+static_assert(MC_CPB <= 16 && MC_RT % (2 * MC_THREADS) == 0, "bad tile shape");
 
 // Hilbert index of cell (x, y) on the 2^16 x 2^16 grid.
 __device__ __forceinline__ uint32_t hilbert16(uint32_t x, uint32_t y) {
@@ -807,14 +820,15 @@ __global__ void mlapm_cull_keys_kernel(const float2 *__restrict__ pos, int N, ui
 }
 
 // One CTA of MS_BLOCK threads per block of the sorted crowd: slot j holds the agent perm[j] (ms_prep_slot; j >= N:
-// padding), slot[agent] = j, and the boxes {min x, min y, max x, max y} of the
-// block and of its MC_SPB column stages.  Agents with a non-finite position or velocity do not enter the min / max (no
-// fminf / fmaxf on NaN); they flag their stage and block MC_NEAR_ALL instead, which keeps every item that touches them.
+// padding), slot[agent] = j, and the boxes {min x, min y, max x, max y} of its MC_CPB column tiles (one warp each), its
+// MC_RPB row tiles and the block.  Agents with a non-finite position or velocity do not enter the min / max (no
+// fminf / fmaxf on NaN); they flag their tiles and block MC_NEAR_ALL instead, which keeps every unit that touches them.
 __global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
     const float2 *__restrict__ pos, const float2 *__restrict__ vel, const float2 *__restrict__ dest,
     const int *__restrict__ perm, int N, float4 *__restrict__ rec, int *__restrict__ slot,
-    ulonglong2 *__restrict__ acc, unsigned *__restrict__ bad, float4 *__restrict__ sbox, unsigned *__restrict__ sflag,
-    float4 *__restrict__ bbox, unsigned *__restrict__ bflag) {
+    ulonglong2 *__restrict__ acc, unsigned *__restrict__ bad, float4 *__restrict__ cbox, unsigned *__restrict__ cflag,
+    float4 *__restrict__ rbox, unsigned *__restrict__ rflag, float4 *__restrict__ bbox, unsigned *__restrict__ bflag) {
+    static_assert(MC_CT == 32, "a column tile is one warp");
     __shared__ float4 wbox[MS_BLOCK / 32];
     __shared__ unsigned wflag[MS_BLOCK / 32];
     const int j = blockIdx.x * MS_BLOCK + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -842,12 +856,16 @@ __global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
         b.w = fmaxf(b.w, __shfl_xor_sync(0xffffffffu, b.w, o));
         flag = comb(flag, __shfl_xor_sync(0xffffffffu, flag, o));
     }
-    if (lane == 0) { wbox[warp] = b; wflag[warp] = flag; }
+    if (lane == 0) {
+        wbox[warp] = b; wflag[warp] = flag;
+        cbox[blockIdx.x * MC_CPB + warp] = b;
+        cflag[blockIdx.x * MC_CPB + warp] = flag;
+    }
     __syncthreads();
-    if (threadIdx.x < MC_SPB + 1) {
-        // thread s < MC_SPB: stage s (its MS_CT / 32 warps); thread MC_SPB: the whole block
-        const int w0 = threadIdx.x < MC_SPB ? threadIdx.x * (MS_CT / 32) : 0;
-        const int w1 = threadIdx.x < MC_SPB ? w0 + MS_CT / 32 : MS_BLOCK / 32;
+    if (threadIdx.x < MC_RPB + 1) {
+        // thread r < MC_RPB: row tile r (its MC_RT / 32 warps); thread MC_RPB: the whole block
+        const int w0 = threadIdx.x < MC_RPB ? threadIdx.x * (MC_RT / 32) : 0;
+        const int w1 = threadIdx.x < MC_RPB ? w0 + MC_RT / 32 : MS_BLOCK / 32;
         float4 u = wbox[w0];
         unsigned f = wflag[w0];
         for (int w = w0 + 1; w < w1; ++w) {
@@ -855,9 +873,9 @@ __global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
             u.x = fminf(u.x, t.x); u.y = fminf(u.y, t.y); u.z = fmaxf(u.z, t.z); u.w = fmaxf(u.w, t.w);
             f = comb(f, wflag[w]);
         }
-        if (threadIdx.x < MC_SPB) {
-            sbox[blockIdx.x * MC_SPB + threadIdx.x] = u;
-            sflag[blockIdx.x * MC_SPB + threadIdx.x] = f;
+        if (threadIdx.x < MC_RPB) {
+            rbox[blockIdx.x * MC_RPB + threadIdx.x] = u;
+            rflag[blockIdx.x * MC_RPB + threadIdx.x] = f;
         } else {
             bbox[blockIdx.x] = u;
             bflag[blockIdx.x] = f;
@@ -865,119 +883,176 @@ __global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
     }
 }
 
-// Keep-predicate of the work list over candidate c = ((I * (D + 1) + d) * MC_SPB + stage): rows = block I, columns =
-// stage `stage` of block J = I + d mod T (circulant schedule of mlapm_sym_kernel).  The box gap is rounded down, so a
-// kept-or-not decision never depends on fp32 rounding in the skipping direction.
+// Whether two boxes (with their flags) may hold a pair within rc.  The box gap is rounded down, so a kept-or-not
+// decision never depends on fp32 rounding in the skipping direction.
+__device__ __forceinline__ bool cull_near(float4 a, unsigned fa, float4 b, unsigned fb, float rc) {
+    if ((fa | fb) & MC_EMPTY) return false;
+    if ((fa | fb) & MC_NEAR_ALL) return true;
+    const float gx = fmaxf(fmaxf(__fsub_rd(b.x, a.z), __fsub_rd(a.x, b.z)), 0.f);
+    const float gy = fmaxf(fmaxf(__fsub_rd(b.y, a.w), __fsub_rd(a.y, b.w)), 0.f);
+    return __fadd_rd(__fmul_rd(gx, gx), __fmul_rd(gy, gy)) <= rc * rc;
+}
+
+// Item c = R * (D + 1) + d of the schedule: row tile R of block I = R / MC_RPB against column block J = I + d mod T.
+// The items of one row tile are consecutive, so a CTA keeps its rows over a run of them.
+struct CullItem {
+    int R, d, J;
+    __device__ __forceinline__ CullItem(int c, int T, int D) {
+        R = c / (D + 1);
+        d = c - R * (D + 1);
+        const int I = R / MC_RPB;
+        J = I + d >= T ? I + d - T : I + d;
+    }
+    // first column tile of block J that the item covers: d = 0 skips the row tiles r' < r of the own block
+    __device__ __forceinline__ int first_tile() const { return d == 0 ? (R % MC_RPB) * (MC_CPB / MC_RPB) : 0; }
+};
+
+// Keep-predicate of the work list: the row tile's box within r_cut of block J's box (circulant schedule of
+// mlapm_sym_kernel; for even T the pairs at d = T/2 belong to I < T/2).
 struct CullKeep {
-    const float4 *sbox, *bbox;
-    const unsigned *sflag, *bflag;
+    const float4 *rbox, *bbox;
+    const unsigned *rflag, *bflag;
     int T, D;
     float rc;
     __device__ __forceinline__ bool operator()(int c) const {
-        const int st = c % MC_SPB, pd = c / MC_SPB;
-        const int I = pd / (D + 1), d = pd - I * (D + 1);
-        if (!(T & 1) && d == D && 2 * I >= T) return false;     // even T: the pairs at d = T/2 belong to I < T/2
-        int J = I + d;
-        J = J >= T ? J - T : J;
-        const int s = J * MC_SPB + st;
-        const unsigned fr = bflag[I], fc = sflag[s];
-        if ((fr | fc) & MC_EMPTY) return false;
-        if ((fr | fc) & MC_NEAR_ALL) return true;
-        const float4 a = bbox[I], b = sbox[s];
-        const float gx = fmaxf(fmaxf(__fsub_rd(b.x, a.z), __fsub_rd(a.x, b.z)), 0.f);
-        const float gy = fmaxf(fmaxf(__fsub_rd(b.y, a.w), __fsub_rd(a.y, b.w)), 0.f);
-        return __fadd_rd(__fmul_rd(gx, gx), __fmul_rd(gy, gy)) <= rc * rc;
+        const CullItem it(c, T, D);
+        if (!(T & 1) && it.d == D && 2 * (it.R / MC_RPB) >= T) return false;
+        return cull_near(rbox[it.R], rflag[it.R], bbox[it.J], bflag[it.J], rc);
     }
 };
 
-// The symmetric pair kernel over the work list.  Persistent: CTA b takes the contiguous items [b n / G, (b+1) n / G)
-// of the n = *nitems on the list (read on the device: no host sync).  Rows stay in registers while consecutive items
-// share the row block; when it changes, and at the end, the row sums go into the fixed-point accumulators with the
-// opposite sign of the column shares (acc = column share - row share; the finalize kernel subtracts acc).  The stages
-// are evaluated as in mlapm_sym_kernel (ms_diag_tile, ms_pair_tile, ms_add_columns).
-template <int VERSION>
-__global__ void __launch_bounds__(MC_THREADS, 8) mlapm_sym_list_kernel(const float4 *__restrict__ rec,
-                                                                      const int *__restrict__ items,
-                                                                      const int *__restrict__ nitems, int T, int D,
-                                                                      M2Const k, unsigned long long *__restrict__ acc,
-                                                                      unsigned *__restrict__ bad, float colscale) {
-    constexpr int THREADS = MC_THREADS, RPS = MS_BLOCK / (2 * THREADS);
-    extern __shared__ __align__(128) unsigned char ms_smem_raw[];
-    MsSmem<THREADS> &sm = *reinterpret_cast<MsSmem<THREADS> *>(ms_smem_raw);
-    // the item of the stage in tile[buf] (I, d, first column j0 = J * MS_BLOCK + stage * MS_CT), written by the thread
-    // that issues its copy; the loop state lives here too, which keeps the pair loop at 128 registers without spills
-    __shared__ int meta[2][3];
-    __shared__ int s_lo, s_cnt;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    __builtin_assume(bad != nullptr);                          // never null here: one copy of ms_add_columns' loop
+// masks[i] = the column tiles of block J that list item i evaluates: within r_cut of the row tile's box and allowed by
+// the d = 0 rule.  Grid-stride over the n = *nitems items (read on the device).
+__global__ void mlapm_cull_masks_kernel(const int *__restrict__ items, const int *__restrict__ nitems,
+                                        const float4 *__restrict__ rbox, const unsigned *__restrict__ rflag,
+                                        const float4 *__restrict__ cbox, const unsigned *__restrict__ cflag, int T,
+                                        int D, float rc, uint16_t *__restrict__ masks) {
     const int n = *nitems;
-    const int lo = static_cast<int>(static_cast<int64_t>(n) * blockIdx.x / gridDim.x);
-    const int cnt = static_cast<int>(static_cast<int64_t>(n) * (blockIdx.x + 1) / gridDim.x) - lo;
-    if (cnt <= 0) return;
-    constexpr uint32_t STAGE_BYTES = MS_CT * MS_RECF * sizeof(float);
-    auto stage_load = [&](int s, int buf) {                    // thread 0
-        const int c = items[s];
-        const int st = c % MC_SPB, pd = c / MC_SPB;
-        const int I = pd / (D + 1), d = pd - I * (D + 1);
-        const int J = I + d >= T ? I + d - T : I + d;
-        const int j0 = J * MS_BLOCK + st * MS_CT;
-        meta[buf][0] = I; meta[buf][1] = d; meta[buf][2] = j0;
-        mbar_expect_tx(&sm.bars[buf], STAGE_BYTES);
-        tma_bulk_g2s(sm.tile[buf], rec + static_cast<int64_t>(j0) * 2, STAGE_BYTES, &sm.bars[buf]);
-    };
-    if (tid == 0) {
-        mbar_init(&sm.bars[0], 1);
-        mbar_init(&sm.bars[1], 1);
-        mbar_fence_init();
-        s_lo = lo;
-        s_cnt = cnt;
-        stage_load(lo, 0);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const CullItem it(items[i], T, D);
+        const float4 a = rbox[it.R];
+        const unsigned fa = rflag[it.R];
+        unsigned m = 0;
+        for (int ct = it.first_tile(); ct < MC_CPB; ++ct) {
+            const int s = it.J * MC_CPB + ct;
+            if (cull_near(a, fa, cbox[s], cflag[s], rc)) m |= 1u << ct;
+        }
+        masks[i] = static_cast<uint16_t>(m);
     }
-    __syncthreads();
+}
+
+// Live units of item i for the scan: popcount of its mask; 0 past the end of the list.
+struct MaskCount {
+    const uint16_t *masks;
+    const int *nitems;
+    __device__ __forceinline__ long long operator()(int i) const { return i < *nitems ? __popc(masks[i]) : 0; }
+};
+
+// The symmetric pair kernel over the live units.  Persistent, one warp per CTA: CTA b takes the units
+// [b W / G, (b+1) W / G) of the W = uoff[n] on the list (read on the device: no host sync), finds the item of its first
+// unit by binary search in the scan and walks the masks from there.  A unit is one 1 KB column tile, staged by a TMA
+// bulk copy (double buffered) and evaluated against the warp's 128 rows by the dense kernel's bodies (ms_pair_tile,
+// ms_diag_tile); each column's warp sum goes straight into the fixed-point accumulators.  Rows stay in registers while
+// consecutive units share the row tile; when it changes, and at the end, the row sums go into the same accumulators
+// with the opposite sign of the column shares (acc = column share - row share; the finalize kernel subtracts acc).
+template <int VERSION>
+__global__ void __launch_bounds__(MC_THREADS, 16) mlapm_sym_tiles_kernel(
+    const float4 *__restrict__ rec, const int *__restrict__ items, const int *__restrict__ nitems,
+    const uint16_t *__restrict__ masks, const long long *__restrict__ uoff, int T, int D, M2Const k,
+    unsigned long long *__restrict__ acc, unsigned *__restrict__ bad, float colscale) {
+    constexpr int RPS = MC_RT / (2 * MC_THREADS);
+    constexpr uint32_t TILE_BYTES = MC_CT * MS_RECF * sizeof(float);
+    __shared__ __align__(128) float4 tile[2][MC_CT * 2];
+    __shared__ __align__(16) float4 red[MS_BATCH * MS_RED_STRIDE];
+    __shared__ __align__(8) uint64_t bars[2];
+    const int lane = threadIdx.x;
+    const int n = *nitems;
+    const long long W = uoff[n];
+    const long long u0 = W * blockIdx.x / gridDim.x, u1 = W * (blockIdx.x + 1) / gridDim.x;
+    if (u1 <= u0) return;
+    int lo = 0, hi = n;                                        // uoff[lo] <= u0 < uoff[hi]
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (uoff[mid] <= u0) lo = mid;
+        else hi = mid;
+    }
+    int item = lo;
+    unsigned mask = masks[item];
+    for (long long s = u0 - uoff[item]; s > 0; --s) mask &= mask - 1;
+    // the next unit in list order: row tile R, first column slot j0, whether it is one of the row tile's own tiles
+    auto next_unit = [&](int &R, int &j0, bool &diag) {
+        while (mask == 0) mask = masks[++item];
+        const int ct = __ffs(mask) - 1;
+        mask &= mask - 1;
+        const CullItem it(items[item], T, D);
+        R = it.R;
+        j0 = it.J * MS_BLOCK + ct * MC_CT;
+        diag = it.d == 0 && ct / (MC_CPB / MC_RPB) == it.R % MC_RPB;
+    };
+    auto stage = [&](int j0, int buf) {
+        if (lane == 0) {
+            mbar_expect_tx(&bars[buf], TILE_BYTES);
+            tma_bulk_g2s(tile[buf], rec + static_cast<int64_t>(j0) * 2, TILE_BYTES, &bars[buf]);
+        }
+    };
+    if (lane == 0) {
+        mbar_init(&bars[0], 1);
+        mbar_init(&bars[1], 1);
+        mbar_fence_init();
+    }
+    __syncwarp();
+    int R, j0;
+    bool diag;
+    next_unit(R, j0, diag);
+    stage(j0, 0);
 
     MsRows<RPS> rw;
     const float2 Bl = splat(k.Bl), Cl = splat(k.Cl), Dl = splat(k.Dl);
-    auto flush_rows = [&](int I) {
+    auto add = [&](int64_t j, float a0, float a1, float a2, float a3, float scale) {
+        if (!isfinite(a0 + a1 + a2 + a3)) bad[j] = 1u;
+        unsigned long long *dst = acc + j * 4;
+        atomicAdd(dst + 0, static_cast<unsigned long long>(__float2ll_rn(a0 * scale)));
+        atomicAdd(dst + 1, static_cast<unsigned long long>(__float2ll_rn(a1 * scale)));
+        atomicAdd(dst + 2, static_cast<unsigned long long>(__float2ll_rn(a2 * scale)));
+        atomicAdd(dst + 3, static_cast<unsigned long long>(__float2ll_rn(a3 * scale)));
+    };
+    auto flush_rows = [&](int Rf) {
 #pragma unroll
         for (int i = 0; i < RPS; ++i) {
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-                const int64_t j = static_cast<int64_t>(I) * MS_BLOCK + (2 * i + h) * THREADS + tid;
-                const float a0 = h ? rw.Sx[i].y : rw.Sx[i].x, a1 = h ? rw.Sy[i].y : rw.Sy[i].x;
-                const float a2 = h ? rw.Tx[i].y : rw.Tx[i].x, a3 = h ? rw.Ty[i].y : rw.Ty[i].x;
-                if (!isfinite(a0 + a1 + a2 + a3)) bad[j] = 1u;
-                unsigned long long *dst = acc + j * 4;
-                atomicAdd(dst + 0, static_cast<unsigned long long>(__float2ll_rn(-a0 * colscale)));
-                atomicAdd(dst + 1, static_cast<unsigned long long>(__float2ll_rn(-a1 * colscale)));
-                atomicAdd(dst + 2, static_cast<unsigned long long>(__float2ll_rn(-a2 * colscale)));
-                atomicAdd(dst + 3, static_cast<unsigned long long>(__float2ll_rn(-a3 * colscale)));
-            }
+            const int64_t j = static_cast<int64_t>(Rf) * MC_RT + (2 * i) * MC_THREADS + lane;
+            add(j, rw.Sx[i].x, rw.Sy[i].x, rw.Tx[i].x, rw.Ty[i].x, -colscale);
+            add(j + MC_THREADS, rw.Sx[i].y, rw.Sy[i].y, rw.Tx[i].y, rw.Ty[i].y, -colscale);
         }
     };
-
-    // runs of consecutive items with the same row block: rows loaded once per run, row sums flushed at its end.
-    // meta[t & 1] was written before the barrier that ended item t - 1 and is rewritten only after item t's.
-    int t = 0;
-    while (t < s_cnt) {
-        const int I = meta[t & 1][0];
-        ms_load_rows(rw, rec, I, tid);
-        do {
+    const int cnt = static_cast<int>(u1 - u0);
+    int Rrun = -1;
+    for (int t = 0; t < cnt; ++t) {
         const int buf = t & 1;
-        if (tid == 0 && t + 1 < s_cnt) stage_load(s_lo + t + 1, buf ^ 1);   // tile[buf^1] was released by the
-        mbar_wait(&sm.bars[buf], (t >> 1) & 1);                   // the (t/2)-th use of this buffer
-        // the off-diagonal branch first: in the other order ptxas emits the diagonal loop twice
-        if (meta[buf][1] != 0) {
-            ms_pair_tile<VERSION>(rw, sm.tile[buf], sm.red[warp], sm.colacc[warp], lane, Bl, Cl, Dl);
-            __syncthreads();
-            ms_add_columns<THREADS>(sm.colacc, acc, bad, meta[buf][2], colscale, tid);
-        } else {
-            ms_diag_tile<VERSION>(rw, sm.tile[buf], Bl, Cl, Dl);
+        int Rn = 0, jn = 0;
+        bool dn = false;
+        if (t + 1 < cnt) {                                     // tile[buf^1] was released by the __syncwarp below
+            next_unit(Rn, jn, dn);
+            stage(jn, buf ^ 1);
         }
-        __syncthreads();
-        ++t;
-        } while (t < s_cnt && meta[t & 1][0] == I);
-        flush_rows(I);
+        if (R != Rrun) {
+            if (Rrun >= 0) flush_rows(Rrun);
+            ms_load_rows<RPS, MC_THREADS>(rw, rec, static_cast<int64_t>(R) * MC_RT, lane);
+            Rrun = R;
+        }
+        mbar_wait(&bars[buf], (t >> 1) & 1);                   // the (t/2)-th use of this buffer
+        // the off-diagonal branch first: in the other order ptxas emits the diagonal loop twice
+        if (!diag) {
+            const int64_t jc = j0;
+            ms_pair_tile<VERSION, RPS, MC_CT>(rw, tile[buf], red, lane, Bl, Cl, Dl, [&](int c, float4 a) {
+                add(jc + c, a.x, a.y, a.z, a.w, colscale);
+            });
+        } else {
+            ms_diag_tile<VERSION, RPS, MC_CT>(rw, tile[buf], Bl, Cl, Dl);
+        }
+        __syncwarp();
+        R = Rn; j0 = jn; diag = dn;
     }
+    flush_rows(Rrun);
 }
 
 // Exchange step of an agent-sharded crowd fused into the finalize kernel: rank g's NEXT-state arrays, mapped into this
@@ -1352,26 +1427,28 @@ static SymLayout sym_layout(int64_t N, int world, void *base) {
     return l;
 }
 
-// Culled symmetric evaluation (mlapm_sym_list_kernel).  Candidates of the work list: T * (floor(T/2) + 1) * MC_SPB,
+// Culled symmetric evaluation (mlapm_sym_tiles_kernel).  Candidates of the work list: T * (floor(T/2) + 1) * MC_RPB,
 // the dense worst case (every item within r_cut); the list index is an int.
 static int64_t cull_candidates(int64_t N) {
     const int64_t T = sym_blocks(N);
-    return T * (T / 2 + 1) * MC_SPB;
+    return T * (T / 2 + 1) * MC_RPB;
 }
 // Reserved CUB scratch, computable without a device (CUB's own size query needs one).  Radix sort on DoubleBuffers
 // (onesweep): 4 passes x 256 bins of 8 B, and 256 look-back counters of 4 B per tile of >= 256 keys -- at most 4 B
-// per key.  Select: one 16 B tile descriptor per tile of >= 128 candidates -- at most 1 B per candidate.  64 KB for
-// the counters, padding and alignment of both.  The real size is checked against this at every call.
+// per key.  Select, and the scan of the candidates + 1 unit counts: one 16 B tile descriptor per tile of >= 128
+// items -- at most 1 B per candidate.  64 KB for the counters, padding and alignment of all three.  The real size is checked against this at every call.
 static int64_t cull_cub_bound(int64_t N) {
     const int64_t a = 4 * N, b = cull_candidates(N);
     return (int64_t{1} << 16) + (a > b ? a : b);
 }
 struct CullLayout {
     float4 *rec; long long *acc; unsigned *bad; uint32_t *key[2]; int *val[2]; int *slot;
-    float4 *sbox, *bbox; unsigned *sflag, *bflag; int *items, *nitems; void *temp; int64_t temp_bytes, total;
+    float4 *cbox, *rbox, *bbox; unsigned *cflag, *rflag, *bflag; int *items, *nitems; uint16_t *masks;
+    long long *uoff; void *temp; int64_t temp_bytes, total;
 };
 // records, accumulators (4 x int64) and flags per padded agent; keys, values (both double-buffered) and slots per
-// agent; boxes and flags per stage and block; the work list; CUB's scratch.  0.1 GB at N = 10^6.
+// agent; boxes and flags per column tile, row tile and block; the work list, its masks and the scan of their
+// popcounts (14 B per candidate); CUB's scratch.  0.2 GB at N = 10^6.
 static CullLayout cull_layout(int64_t N, void *base) {
     const int64_t T = sym_blocks(N), npad = T * MS_BLOCK;
     CullLayout l{};
@@ -1384,12 +1461,16 @@ static CullLayout cull_layout(int64_t N, void *base) {
         l.val[b] = static_cast<int *>(c.take(N * sizeof(int)));
     }
     l.slot = static_cast<int *>(c.take(N * sizeof(int)));
-    l.sbox = static_cast<float4 *>(c.take(T * MC_SPB * sizeof(float4)));
+    l.cbox = static_cast<float4 *>(c.take(T * MC_CPB * sizeof(float4)));
+    l.rbox = static_cast<float4 *>(c.take(T * MC_RPB * sizeof(float4)));
     l.bbox = static_cast<float4 *>(c.take(T * sizeof(float4)));
-    l.sflag = static_cast<unsigned *>(c.take(T * MC_SPB * sizeof(unsigned)));
+    l.cflag = static_cast<unsigned *>(c.take(T * MC_CPB * sizeof(unsigned)));
+    l.rflag = static_cast<unsigned *>(c.take(T * MC_RPB * sizeof(unsigned)));
     l.bflag = static_cast<unsigned *>(c.take(T * sizeof(unsigned)));
     l.items = static_cast<int *>(c.take(cull_candidates(N) * sizeof(int)));
     l.nitems = static_cast<int *>(c.take(sizeof(int)));
+    l.masks = static_cast<uint16_t *>(c.take(cull_candidates(N) * sizeof(uint16_t)));
+    l.uoff = static_cast<long long *>(c.take((cull_candidates(N) + 1) * sizeof(long long)));
     l.temp_bytes = cull_cub_bound(N);
     l.temp = c.take(l.temp_bytes);
     l.total = c.off + 256;                                          // + 256: room to align the caller's base
@@ -1424,7 +1505,9 @@ extern "C" int piml_mlapm_cull_items(const void *workspace, int64_t N, int64_t *
     const CullLayout l = cull_layout(N, ws_align(workspace));
     int n = 0;
     PIML_CUDA(cudaMemcpy(&n, l.nitems, sizeof(int), cudaMemcpyDeviceToHost));
-    *items = n;
+    long long w = 0;
+    PIML_CUDA(cudaMemcpy(&w, l.uoff + n, sizeof(long long), cudaMemcpyDeviceToHost));
+    *items = w;
     return PIML_OK;
 }
 
@@ -1445,7 +1528,7 @@ static bool sym_params_ok(const piml_mlapm_params *prm, const MlConst &k, int64_
            sym_colscale_log2(N, prm) >= 30;                        // 2^-30 resolution at the very least (|C| < ~15)
 }
 
-// Distance beyond which every pair's production weight is exactly +0 (see mlapm_sym_list_kernel): arg <= (Bl + |Dl|) r
+// Distance beyond which every pair's production weight is exactly +0 (see the culled symmetric evaluation): arg <= (Bl + |Dl|) r
 // + |Cl| < -127 (raw: Bl r < -127), from the same fp32 constants the kernels use.  The margin (1 % + 0.01 m) covers
 // the rsqrt.approx error in r and q and fp32 rounding of coordinates; ex2.approx.ftz already returns 0 below -126.
 // +inf (no culling) where the symmetric kernels do not run.
@@ -1519,12 +1602,13 @@ static int launch_sym_culled(int version, const float2 *p2, const float2 *v2, co
     PIML_CUDA(cub::DeviceRadixSort::SortPairs(l.temp, temp_bytes, keys, vals, N, 0, 32, st));
     count_launch(cub_sort_launches(N, 32));
     mlapm_prep_cull_kernel<<<static_cast<unsigned>(T), MS_BLOCK, 0, st>>>(
-        p2, v2, d2, vals.Current(), N, l.rec, l.slot, reinterpret_cast<ulonglong2 *>(l.acc), l.bad, l.sbox, l.sflag,
-        l.bbox, l.bflag);
+        p2, v2, d2, vals.Current(), N, l.rec, l.slot, reinterpret_cast<ulonglong2 *>(l.acc), l.bad, l.cbox, l.cflag,
+        l.rbox, l.rflag, l.bbox, l.bflag);
     count_launch();
     rc_ = check_launch("mlapm_prep_cull_kernel");
     if (rc_) return rc_;
-    const CullKeep keep{l.sbox, l.bbox, l.sflag, l.bflag, static_cast<int>(T), static_cast<int>(D), rc};
+    const int iT = static_cast<int>(T), iD = static_cast<int>(D);
+    const CullKeep keep{l.rbox, l.bbox, l.rflag, l.bflag, iT, iD, rc};
     const int ncand = static_cast<int>(cull_candidates(N));
     cub::CountingInputIterator<int> cand(0);
     need = 0;
@@ -1535,31 +1619,45 @@ static int launch_sym_culled(int version, const float2 *p2, const float2 *v2, co
     temp_bytes = static_cast<size_t>(l.temp_bytes);
     PIML_CUDA(cub::DeviceSelect::If(l.temp, temp_bytes, cand, l.items, l.nitems, ncand, keep, st));
     count_launch(2);                                              // tile-state init + select
-    using Smem = MsSmem<MC_THREADS>;
-    static_assert(sizeof(Smem) <= 48 * 1024, "mlapm_sym_list_kernel: shared memory above the default limit");
-    const void *kfn = version == 0 ? reinterpret_cast<const void *>(&mlapm_sym_list_kernel<0>)
-                                   : reinterpret_cast<const void *>(&mlapm_sym_list_kernel<1>);
+    // the list's length stays on the device: a fixed grid strides over it, and the scan runs over every candidate
+    // (MaskCount is 0 past the list's end), so uoff[n] = W, the live units
+    mlapm_cull_masks_kernel<<<static_cast<unsigned>(4 * sm_count()), threads, 0, st>>>(
+        l.items, l.nitems, l.rbox, l.rflag, l.cbox, l.cflag, iT, iD, rc, l.masks);
+    count_launch();
+    rc_ = check_launch("mlapm_cull_masks_kernel");
+    if (rc_) return rc_;
+    const auto counts = thrust::make_transform_iterator(thrust::counting_iterator<int>(0), MaskCount{l.masks, l.nitems});
+    need = 0;
+    PIML_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, need, counts, l.uoff, ncand + 1, st));
+    PIML_REQUIRE(static_cast<int64_t>(need) <= l.temp_bytes,
+                 "piml_mlapm: CUB scan needs %lld bytes of scratch, %lld reserved", static_cast<long long>(need),
+                 static_cast<long long>(l.temp_bytes));
+    temp_bytes = static_cast<size_t>(l.temp_bytes);
+    PIML_CUDA(cub::DeviceScan::ExclusiveSum(l.temp, temp_bytes, counts, l.uoff, ncand + 1, st));
+    count_launch(2);                                              // tile-state init + scan
+    const void *kfn = version == 0 ? reinterpret_cast<const void *>(&mlapm_sym_tiles_kernel<0>)
+                                   : reinterpret_cast<const void *>(&mlapm_sym_tiles_kernel<1>);
     static const void *cached_fn = nullptr;
     static int cached_occ = 0;
     if (kfn != cached_fn) {
         int occ = 0;
-        PIML_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kfn, MC_THREADS, sizeof(Smem)));
+        PIML_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kfn, MC_THREADS, 0));
         cached_occ = occ < 1 ? 1 : occ;
         cached_fn = kfn;
     }
-    // persistent grid: one CTA per resident slot, capped by the largest list (it can never have more items)
+    // persistent grid: one CTA per resident slot, capped by the most units a list can hold
     int64_t grid = static_cast<int64_t>(cached_occ) * sm_count();
-    if (grid > ncand) grid = ncand;
+    if (grid > static_cast<int64_t>(ncand) * MC_CPB) grid = static_cast<int64_t>(ncand) * MC_CPB;
     M2Const k2{k.Bl, k.Cl, k.Dl};
     unsigned long long *acc = reinterpret_cast<unsigned long long *>(l.acc);
     if (version == 0)
-        mlapm_sym_list_kernel<0><<<static_cast<unsigned>(grid), MC_THREADS, sizeof(Smem), st>>>(
-            l.rec, l.items, l.nitems, static_cast<int>(T), static_cast<int>(D), k2, acc, l.bad, colscale);
+        mlapm_sym_tiles_kernel<0><<<static_cast<unsigned>(grid), MC_THREADS, 0, st>>>(
+            l.rec, l.items, l.nitems, l.masks, l.uoff, iT, iD, k2, acc, l.bad, colscale);
     else
-        mlapm_sym_list_kernel<1><<<static_cast<unsigned>(grid), MC_THREADS, sizeof(Smem), st>>>(
-            l.rec, l.items, l.nitems, static_cast<int>(T), static_cast<int>(D), k2, acc, l.bad, colscale);
+        mlapm_sym_tiles_kernel<1><<<static_cast<unsigned>(grid), MC_THREADS, 0, st>>>(
+            l.rec, l.items, l.nitems, l.masks, l.uoff, iT, iD, k2, acc, l.bad, colscale);
     count_launch();
-    return check_launch("mlapm_sym_list_kernel");
+    return check_launch("mlapm_sym_tiles_kernel");
 }
 
 static int mlapm_advance_impl(const float *pos, const float *vel, const float *desired_speed, int ds_dim,

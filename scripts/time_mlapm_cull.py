@@ -4,7 +4,7 @@
 
 Per size: culled (algorithm 2) and dense (algorithm 3) steps alternate in one process, `rounds` x `steps` each, with
 a 160 MB L2 flush before every step outside its CUDA-event pair; min / median / max ms per step.  The dense arm at
-N >= 10^6 runs one step per round (about 0.7 s each).  Then the work-list length, the evaluated pairs and their rate
+N >= 10^6 runs one step per round (about 0.7 s each).  Then the live units, the evaluated pairs and their rate
 against the dense kernel's, a torch.profiler run for the per-kernel split (written under --out), and 50 consecutive
 culled steps on the moving crowd.
 """
@@ -24,7 +24,7 @@ import bench  # noqa: E402
 import piml_b200 as P  # noqa: E402
 from piml_b200 import _lib as L  # noqa: E402
 
-STAGE_PAIRS = 512 * 128          # (row block, column stage) item
+UNIT_PAIRS = 128 * 32            # (row tile, column tile) unit
 
 
 def algo(a):
@@ -36,9 +36,10 @@ def groups(name):
         return "keys + sort"
     if "prep_cull" in name:
         return "prep + boxes"
-    if "Select" in name or "Compact" in name or "ScanTileState" in name or "InitKernel" in name:
+    if ("Select" in name or "Compact" in name or "Scan" in name or "InitKernel" in name
+            or "cull_masks" in name):
         return "list build"
-    if "sym_list" in name:
+    if "sym_tiles" in name:
         return "pair kernel (culled)"
     if "mlapm_sym_kernel" in name:
         return "pair kernel (dense)"
@@ -93,15 +94,17 @@ def main():
             ms["dense"] += run(3, dense_steps)
         res = {k: {"min": min(t), "median": statistics.median(t), "max": max(t), "n": len(t)} for k, t in ms.items()}
         res["speedup_median"] = res["dense"]["median"] / res["culled"]["median"]
-        # work list of the culled step on the bench crowd
+        # live units of the culled step on the bench crowd
         run(2, 1)
-        items = C.c_int64()
-        L.check(L.load().piml_mlapm_cull_items(L.ptr(model._ws), N, C.byref(items)), "piml_mlapm_cull_items")
+        units = C.c_int64()
+        L.check(L.load().piml_mlapm_cull_items(L.ptr(model._ws), N, C.byref(units)), "piml_mlapm_cull_items")
         T = (N + 511) // 512
-        cand = T * (T // 2 + 1) * 4
-        ordered = items.value * 2 * STAGE_PAIRS - 4 * T * STAGE_PAIRS   # diagonal items: one direction
-        res.update({"items": items.value, "candidates": cand, "item_share": items.value / cand,
-                    "unordered_pairs_evaluated": items.value * STAGE_PAIRS,
+        cand = T * (T // 2 + 1) * 4 * 16                             # (row tile, d) candidates x 16 column tiles
+        diag = (N + 31) // 32                                        # each column tile's own unit: one direction
+        off = units.value - diag
+        ordered = off * 2 * UNIT_PAIRS + diag * UNIT_PAIRS
+        res.update({"units": units.value, "unit_candidates": cand, "unit_share": units.value / cand,
+                    "unordered_pairs_evaluated": off * UNIT_PAIRS + diag * UNIT_PAIRS // 2,
                     "ordered_pair_equivalents": ordered})
         # per-kernel split (a separate, traced run)
         prof_steps = 5
