@@ -313,22 +313,20 @@ PIML_API int piml_pinnsf_forward_f32(const piml_net_desc *desc, const float *par
                             int norm_group, const float *drop_ped, const float *drop_obs, float *acc,
                             float *ped_msgs, float *obs_msgs, float *coll, void *stream);
 
-/* Self test of the tensor-core path (tcgen05 kind::tf32, A in TMEM, accumulator in TMEM): y (128,N) = x (128,K) w^T
- * with w (N,K) row-major; terms = 1: plain TF32, 3: 3xTF32 split (fp32-grade).  K % 8 == 0, N % 16 == 0, both <= 128. */
-PIML_API int piml_tc_selftest_f32(const float *x, const float *w, int K, int N, int terms, float *y, void *stream);
-
-/* The same product on the 16-bit path (tcgen05 kind::f16): x and w split into fp16 hi + lo, terms = 3:
- * x_lo w_hi + x_hi w_lo + x_hi w_hi with fp32 accumulation in TMEM (fp32-grade, like 3xTF32, at twice the K per
- * instruction and half the TMEM / shared-memory footprint).  K % 16 == 0, N % 16 == 0, both <= 128.  swap = 0. */
-PIML_API int piml_tc16_selftest_f32(const float *x, const float *w, int K, int N, int terms, int swap, float *y,
-                                    void *stream);
-
-/* Tensor-core forward (tcgen05 kind::tf32 with the 3xTF32 split, accumulators and activations in TMEM): the inference
- * path of the rollouts.  Same contract as piml_pinnsf_forward_f32 in eval mode without the collision head:
- * acc (R,2) and, for kind 0 models, optional 2-d messages ped_msgs (R,kp,2) / obs_msgs (R,ko,2) (NULL to skip).
+/* Tensor-core forward (tcgen05, accumulators and activations in TMEM): the inference path of the rollouts.  Same
+ * contract as piml_pinnsf_forward_f32 in eval mode without the collision head: acc (R,2) and, for kind 0 models,
+ * optional 2-d messages ped_msgs (R,kp,2) / obs_msgs (R,ko,2) (NULL to skip).
  * Needs processor_hidden_layers > 1 and hidden widths that are multiples of 32 (<= 128);
  * piml_pinnsf_packed_tc_floats returns -1 for networks it cannot run (callers then use piml_pinnsf_forward_f32).
- * packed_tc: written by piml_pinnsf_pack_tc_f32 from the torch-layout vector (see piml_pinnsf_pack_f32). */
+ * packed_tc: written by piml_pinnsf_pack_tc_f32 from the torch-layout vector (see piml_pinnsf_pack_f32).
+ * The kernel and its mode follow from the network and the batch alone:
+ *   - compact mode when no messages are requested and the dense tiles (128 / k agents per tile and branch) exceed one
+ *     wave: only the non-zero slot rows (kind 0) or the agents with a non-zero slot (kind 1, "agent-compact") go
+ *     through the network, the all-zero ones share one evaluation; the result is bit-identical to the dense mode;
+ *   - the 16-bit kernel (fp16 hi + lo operand split, weights resident in shared memory) when its plan accepts the
+ *     network -- kind 0, widths 32, 64 or 128, one branch's weights within the shared memory -- and the batch is not
+ *     in agent-compact mode;
+ *   - otherwise the tf32 kernel (3xTF32 split, weights streamed through a shared-memory ring). */
 PIML_API int64_t piml_pinnsf_packed_tc_floats(const piml_net_desc *desc);
 PIML_API int piml_pinnsf_pack_tc_f32(const piml_net_desc *desc, const float *params_torch, float *packed_tc, void *stream);
 PIML_API int piml_pinnsf_forward_tc_f32(const piml_net_desc *desc, const float *packed_tc, int has_obs, float tau,

@@ -129,8 +129,6 @@ SIGNATURES = {
     "piml_pinnsf_pack_f32": (i32, [C.POINTER(NetDesc), vp, vp, vp]),
     "piml_pinnsf_forward_f32": (i32, [C.POINTER(NetDesc), vp, i32, f32, vp, vp, vp, i64, i32, i32, i32, vp, vp, vp,
                                       vp, vp, vp, vp]),
-    "piml_tc_selftest_f32": (i32, [vp, vp, i32, i32, i32, vp, vp]),
-    "piml_tc16_selftest_f32": (i32, [vp, vp, i32, i32, i32, i32, vp, vp]),
     "piml_pinnsf_packed_tc_floats": (i64, [C.POINTER(NetDesc)]),
     "piml_pinnsf_pack_tc_f32": (i32, [C.POINTER(NetDesc), vp, vp, vp]),
     "piml_pinnsf_forward_tc_f32": (i32, [C.POINTER(NetDesc), vp, i32, f32, vp, vp, vp, i64, i32, i32, i32, vp, vp, vp,

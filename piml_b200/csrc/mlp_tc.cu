@@ -1,285 +1,9 @@
-// mlp_tc.cu -- interaction-network forward on the 5th-generation tensor cores (tcgen05, TMEM) with 3xTF32 operand
-// splitting, for sm_100a.   (work in progress: the single-layer self test)
-#include <stdlib.h>
-
+// mlp_tc.cu -- interaction-network forward on the 5th-generation tensor cores (tcgen05, TMEM), for sm_100a: the
+// 3xTF32 kernel, the packing of both tensor-core weight images and the C entry points, which choose between this
+// kernel and the 16-bit one (mlp_tc16.cu).
 #include "common.cuh"
 #include "tc.cuh"
 #include "mlp_tc16.cuh"
-
-namespace piml {
-
-// Self test of the tensor-core path: Y (128,N) = X (128,K) W^T, W (N,K) row-major like torch's Linear.weight, evaluated
-// as 3 tf32 MMAs per K step (x_lo w_hi + x_hi w_lo + x_hi w_hi), A in TMEM, B in shared memory, D in TMEM.
-__global__ void __launch_bounds__(128, 1) tc_probe_kernel(const float *__restrict__ x, const float *__restrict__ w, int K,
-                                                          int N, int terms, int lbo_o, int sbo_o, int cold, int colah, int colal, float *__restrict__ y,
-                                                          float *__restrict__ dbg) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    uint32_t *w_hi = reinterpret_cast<uint32_t *>(smem_raw);                  // [K/4][N][4]
-    uint32_t *w_lo = w_hi + K * N;
-    __shared__ __align__(8) uint64_t bar;
-    __shared__ uint32_t tmem_slot;
-    const int tid = threadIdx.x, warp = tid >> 5;
-    if (warp == 0) tc::tmem_alloc(&tmem_slot, 512);
-    if (tid == 0) { mbar_init(&bar, 1); mbar_fence_init(); }
-    for (int e = tid; e < N * K; e += 128) {
-        const int n = e / K, k = e % K;
-        uint32_t hi, lo;
-        tc::split_tf32(w[e], hi, lo);
-        const int cell = ((k >> 2) * N + n) * 4 + (k & 3);
-        w_hi[cell] = hi; w_lo[cell] = lo;
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");              // generic-proxy writes -> tensor core reads
-    tc::fence_before_sync();
-    __syncthreads();
-    tc::fence_after_sync();
-    const uint32_t tbase = tmem_slot;
-    const uint32_t lane_base = tbase + (static_cast<uint32_t>(warp * 32) << 16);
-    const uint32_t COL_D = cold, COL_AH = colah, COL_AL = colal;
-    // A: thread = row
-    for (int k0 = 0; k0 < K; k0 += 8) {
-        uint32_t hi[8], lo[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) tc::split_tf32(x[tid * K + k0 + q], hi[q], lo[q]);
-        tc::st8(lane_base + COL_AH + k0, hi);
-        tc::st8(lane_base + COL_AL + k0, lo);
-    }
-    tc::wait_st();
-    tc::fence_before_sync();
-    __syncthreads();
-    if (tid == 0) {
-        tc::fence_after_sync();
-        const uint32_t idesc = tc::idesc_tf32(N);
-        const uint32_t lbo = lbo_o > 0 ? lbo_o : N * 16, sbo = (lbo_o >= 0 && sbo_o) ? sbo_o : 128;
-        const uint32_t kstep = 2 * N * 16;
-        bool acc = false;
-        for (int j = 0; j < K / 8; ++j) {
-            const uint64_t bh = tc::smem_desc(tc::smem_addr(w_hi) + j * kstep, lbo, sbo);
-            const uint64_t bl = tc::smem_desc(tc::smem_addr(w_lo) + j * kstep, lbo, sbo);
-            if (terms >= 3) { tc::mma_tf32_ts(tbase + COL_D, tbase + COL_AL + j * 8, bh, idesc, acc); acc = true; }
-            if (terms >= 2) { tc::mma_tf32_ts(tbase + COL_D, tbase + COL_AH + j * 8, bl, idesc, acc); acc = true; }
-            tc::mma_tf32_ts(tbase + COL_D, tbase + COL_AH + j * 8, bh, idesc, acc);
-            acc = true;
-        }
-        tc::commit(&bar);
-    }
-    if (lbo_o < 0) {
-        // micro-benchmark (bring-up only): -lbo_o repetitions of the whole MMA chain; variant = sbo_o
-        //   0: as is (one accumulator)   1: alternate two accumulators   2: only x_hi w_hi   3: 2 with two accumulators
-        const bool ok = mbar_wait_bounded(&bar, 0, 1u << 22);
-        long long cyc = 0;
-        if (tid == 0 && ok) {
-            tc::fence_after_sync();
-            const uint32_t idesc = tc::idesc_tf32(N);
-            const uint32_t lbo = N * 16, sbo = 128, kstep = 2 * N * 16;
-            const long long t0 = clock64();
-            int cnt = 0;
-            for (int rep = 0; rep < -lbo_o; ++rep)
-                for (int j = 0; j < K / 8; ++j) {
-                    const uint64_t bh = tc::smem_desc(tc::smem_addr(w_hi) + j * kstep, lbo, sbo);
-                    const uint64_t bl = tc::smem_desc(tc::smem_addr(w_lo) + j * kstep, lbo, sbo);
-                    const uint32_t d0 = tbase + COL_D, d1 = tbase + ((sbo_o & 1) ? 384u : COL_D);
-                    if (!(sbo_o & 2)) {
-                        tc::mma_tf32_ts(d0, tbase + COL_AL + j * 8, bh, idesc, true);
-                        tc::mma_tf32_ts(d1, tbase + COL_AH + j * 8, bl, idesc, true);
-                        cnt += 2;
-                    }
-                    tc::mma_tf32_ts((j & 1) ? d1 : d0, tbase + COL_AH + j * 8, bh, idesc, true);
-                    ++cnt;
-                }
-            tc::commit(&bar);
-            const long long t1 = clock64();
-            mbar_wait_bounded(&bar, 1, 1u << 24);
-            const long long t2 = clock64();
-            y[0] = static_cast<float>(t1 - t0) / cnt;       // issue cycles per MMA
-            y[1] = static_cast<float>(t2 - t0) / cnt;       // issue + drain cycles per MMA
-            y[2] = static_cast<float>(cnt);
-            cyc = t2 - t0;
-        }
-        (void)cyc;
-        tc::fence_before_sync();
-        __syncthreads();
-        if (warp == 0) tc::tmem_dealloc(tbase, 512);
-        return;
-    }
-    const bool done = mbar_wait_bounded(&bar, 0, 1u << 22);
-    tc::fence_after_sync();
-    if (!done) {                                                              // never hang the box on a bad descriptor
-        for (int n = 0; n < N; ++n) y[tid * N + n] = __int_as_float(0x7fc00000);
-        __syncthreads();
-        if (warp == 0) tc::tmem_dealloc(tbase, 512);
-        return;
-    }
-    for (int n0 = 0; n0 < N; n0 += 32) {
-        uint32_t r[32];
-        tc::ld32(lane_base + COL_D + n0, r);
-        tc::wait_ld();
-#pragma unroll
-        for (int q = 0; q < 32; ++q)
-            if (n0 + q < N) y[tid * N + n0 + q] = __uint_as_float(r[q]);
-    }
-    if (dbg)
-        for (int k0 = 0; k0 < K; k0 += 32) {                                  // what does the A region hold afterwards?
-            uint32_t r[32];
-            tc::ld32(lane_base + COL_AH + k0, r);
-            tc::wait_ld();
-#pragma unroll
-            for (int q = 0; q < 32; ++q)
-                if (k0 + q < K) dbg[tid * K + k0 + q] = __uint_as_float(r[q]);
-        }
-    tc::fence_before_sync();
-    __syncthreads();
-    if (warp == 0) tc::tmem_dealloc(tbase, 512);
-}
-
-// Self test of the 16-bit path: the same product with x and W split into fp16 hi + lo (3 MMAs per K = 16 step,
-// kind::f16, two A elements per 32-bit TMEM column, eight W elements per 16-byte shared-memory cell).
-// swap != 0 puts the EVEN K index into the high half of a column / cell pair instead (bring-up knob).
-__global__ void __launch_bounds__(128, 1) tc16_probe_kernel(const float *__restrict__ x, const float *__restrict__ w,
-                                                            int K, int N, int terms, int swap, float *__restrict__ y) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    uint16_t *w_hi = reinterpret_cast<uint16_t *>(smem_raw);                  // [K/8][N][8]
-    uint16_t *w_lo = w_hi + K * N;
-    __shared__ __align__(8) uint64_t bar;
-    __shared__ uint32_t tmem_slot;
-    const int tid = threadIdx.x, warp = tid >> 5;
-    if (warp == 0) tc::tmem_alloc(&tmem_slot, 512);
-    if (tid == 0) { mbar_init(&bar, 1); mbar_fence_init(); }
-    for (int e = tid; e < N * K; e += 128) {
-        const int n = e / K, k = e % K;
-        uint16_t hi, lo;
-        tc::split_f16(w[e], hi, lo);
-        const int cell = ((k >> 3) * N + n) * 8 + (k & 7);
-        w_hi[cell] = hi; w_lo[cell] = lo;
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    tc::fence_before_sync();
-    __syncthreads();
-    tc::fence_after_sync();
-    const uint32_t tbase = tmem_slot;
-    const uint32_t lane_base = tbase + (static_cast<uint32_t>(warp * 32) << 16);
-    const uint32_t COL_D = 0, COL_AH = 128, COL_AL = 192;
-    for (int k0 = 0; k0 < K; k0 += 16) {                                      // A: thread = row, 8 columns per K = 16
-        uint32_t hi[8], lo[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) {
-            const float a0 = x[tid * K + k0 + 2 * q], a1 = x[tid * K + k0 + 2 * q + 1];
-            if (swap > 0) tc::split_f16x2(a1, a0, hi[q], lo[q]); else tc::split_f16x2(a0, a1, hi[q], lo[q]);
-        }
-        tc::st8(lane_base + COL_AH + k0 / 2, hi);
-        tc::st8(lane_base + COL_AL + k0 / 2, lo);
-    }
-    tc::wait_st();
-    tc::fence_before_sync();
-    __syncthreads();
-    if (tid == 0) {
-        tc::fence_after_sync();
-        const uint32_t idesc = tc::idesc_f16(N);
-        const uint32_t lbo = N * 16, sbo = 128, kstep = 2 * N * 16;
-        bool acc = false;
-        for (int j = 0; j < K / 16; ++j) {
-            const uint64_t bh = tc::smem_desc(tc::smem_addr(w_hi) + j * kstep, lbo, sbo);
-            const uint64_t bl = tc::smem_desc(tc::smem_addr(w_lo) + j * kstep, lbo, sbo);
-            if (terms >= 3) { tc::mma_f16_ts(tbase + COL_D, tbase + COL_AL + j * 8, bh, idesc, acc); acc = true; }
-            if (terms >= 2) { tc::mma_f16_ts(tbase + COL_D, tbase + COL_AH + j * 8, bl, idesc, acc); acc = true; }
-            tc::mma_f16_ts(tbase + COL_D, tbase + COL_AH + j * 8, bh, idesc, acc);
-            acc = true;
-        }
-        tc::commit(&bar);
-    }
-    const bool done = mbar_wait_bounded(&bar, 0, 1u << 22);
-    tc::fence_after_sync();
-    if (swap < 0) {
-        // micro-benchmark (bring-up only): -swap repetitions of the whole chain; y[0] = issue cycles per MMA,
-        // y[1] = issue + drain cycles per MMA, y[2] = MMAs.  terms: 3 = the 3-term chain, 1 = hi*hi only
-        if (tid == 0 && done) {
-            const uint32_t idesc = tc::idesc_f16(N);
-            const uint32_t lbo = N * 16, sbo = 128, kstep = 2 * N * 16;
-            const long long t0 = clock64();
-            int cnt = 0;
-            // variant (-swap / 1000): 0 one accumulator; 1 alternate D0 / D1 per chain; 2 = 1 + a commit per chain (on a
-            // dummy barrier); 3 alternate D0 / D1 per K step; 4 = 1 with acc = false on each chain's first MMA
-            const int variant = (-swap) / 1000, reps = (-swap) % 1000;
-            __shared__ __align__(8) uint64_t dummy;
-            if (variant == 2) { mbar_init(&dummy, 1); mbar_fence_init(); }
-            for (int rep = 0; rep < reps; ++rep)
-                for (int j = 0; j < K / 16; ++j) {
-                    const uint64_t bh = tc::smem_desc(tc::smem_addr(w_hi) + j * kstep, lbo, sbo);
-                    const uint64_t bl = tc::smem_desc(tc::smem_addr(w_lo) + j * kstep, lbo, sbo);
-                    const int which = variant == 3 ? (j & 1) : ((variant == 1 || variant == 2 || variant == 4) ? (rep & 1) : 0);
-                    const uint32_t d = tbase + COL_D + which * 256, aoff = which * 256;
-                    const bool first = variant == 4 && j == 0;
-                    if (terms >= 3) { tc::mma_f16_ts(d, tbase + aoff + COL_AL + j * 8, bh, idesc, !first); ++cnt; }
-                    if (terms >= 2) { tc::mma_f16_ts(d, tbase + aoff + COL_AH + j * 8, bl, idesc, true); ++cnt; }
-                    tc::mma_f16_ts(d, tbase + aoff + COL_AH + j * 8, bh, idesc, true); ++cnt;
-                    if (variant == 2 && j == K / 16 - 1) tc::commit(&dummy);
-                }
-            tc::commit(&bar);
-            const long long t1 = clock64();
-            mbar_wait_bounded(&bar, 1, 1u << 26);
-            const long long t2 = clock64();
-            y[0] = static_cast<float>(t1 - t0) / cnt;
-            y[1] = static_cast<float>(t2 - t0) / cnt;
-            y[2] = static_cast<float>(cnt);
-        }
-        tc::fence_before_sync();
-        __syncthreads();
-        if (warp == 0) tc::tmem_dealloc(tbase, 512);
-        return;
-    }
-    if (!done) {
-        for (int n = 0; n < N; ++n) y[tid * N + n] = __int_as_float(0x7fc00000);
-    } else {
-        for (int n0 = 0; n0 < N; n0 += 32) {
-            uint32_t r[32];
-            tc::ld32(lane_base + COL_D + n0, r);
-            tc::wait_ld();
-#pragma unroll
-            for (int q = 0; q < 32; ++q)
-                if (n0 + q < N) y[tid * N + n0 + q] = __uint_as_float(r[q]);
-        }
-    }
-    tc::fence_before_sync();
-    __syncthreads();
-    if (warp == 0) tc::tmem_dealloc(tbase, 512);
-}
-
-}  // namespace piml
-
-using namespace piml;
-
-extern "C" int piml_tc16_selftest_f32(const float *x, const float *w, int K, int N, int terms, int swap, float *y,
-                                      void *stream) {
-    PIML_REQUIRE(x && w && y, "piml_tc16_selftest_f32: null pointer");
-    PIML_REQUIRE(K >= 16 && K <= 128 && K % 16 == 0 && N >= 16 && N <= 128 && N % 16 == 0,
-                 "piml_tc16_selftest_f32: need K in [16,128] multiple of 16 and N in [16,128] multiple of 16");
-    PIML_REQUIRE(terms >= 1 && terms <= 3, "piml_tc16_selftest_f32: terms must be 1, 2 or 3");
-    const size_t smem = sizeof(uint16_t) * 2 * K * N;
-    PIML_CUDA(cudaFuncSetAttribute(tc16_probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    tc16_probe_kernel<<<1, 128, smem, static_cast<cudaStream_t>(stream)>>>(x, w, K, N, terms, swap, y);
-    count_launch();
-    return check_launch("tc16_probe_kernel");
-}
-
-extern "C" int piml_tc_selftest_f32(const float *x, const float *w, int K, int N, int terms, float *y, void *stream) {
-    int lbo_o = 0, sbo_o = 0;
-    if (const char *e = getenv("PIML_TC_LBO")) lbo_o = atoi(e);
-    if (const char *e = getenv("PIML_TC_SBO")) sbo_o = atoi(e);
-    int cold = 0, colah = 128, colal = 256;
-    if (const char *e = getenv("PIML_TC_COLD")) cold = atoi(e);
-    if (const char *e = getenv("PIML_TC_COLAH")) colah = atoi(e);
-    if (const char *e = getenv("PIML_TC_COLAL")) colal = atoi(e);
-    float *dbg = nullptr;
-    if (getenv("PIML_TC_DBG")) dbg = y + 128 * N;                             // caller allocated 128*(N+K) floats
-    PIML_REQUIRE(x && w && y, "piml_tc_selftest_f32: null pointer");
-    PIML_REQUIRE(K >= 8 && K <= 128 && K % 8 == 0 && N >= 16 && N <= 128 && N % 16 == 0,
-                 "piml_tc_selftest_f32: need K in [8,128] multiple of 8 and N in [16,128] multiple of 16");
-    PIML_REQUIRE(terms >= 1 && terms <= 3, "piml_tc_selftest_f32: terms must be 1 (plain tf32), 2 or 3 (3xTF32)");
-    const size_t smem = sizeof(uint32_t) * 2 * K * N;
-    PIML_CUDA(cudaFuncSetAttribute(tc_probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    tc_probe_kernel<<<1, 128, smem, static_cast<cudaStream_t>(stream)>>>(x, w, K, N, terms, lbo_o, sbo_o, cold, colah, colal, y, dbg);
-    count_launch();
-    return check_launch("tc_probe_kernel");
-}
 
 // =====================================================================================================================
 // Fused interaction-network forward on the tensor cores (inference: eval mode, acceleration output [+ 2-d messages]).
@@ -325,8 +49,6 @@ struct TcArgs {
     const float *params; const float *ped; const float *obs;
     int64_t R; int kp, ko, ag_ped, ag_obs; int64_t n_ped_tiles, n_obs_tiles;
     float *sums; float *ped_msgs; float *obs_msgs;
-    long long *prof;                               // optional cycle counters of CTA 0 (bring-up only)
-    int dbg;                                       // timing experiments only (PIML_TC_DEBUG): 1 = skip epilogue math, 2 = one MMA term
     // Compact mode (kind 0): zero-padded slot rows all produce the same message f(0), so only the non-zero rows (+ one
     // zero row per branch that yields f(0)) go through the network; the slot sums are formed by the finish kernel.
     int compact; int has_obs;
@@ -398,16 +120,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) pinnsf_tc_kernel(const __grid_c
                 const float *wbase = a.params + P.w_off[br];
                 for (int c = 0; c < P.nch; ++c, ++pc) {
                     const uint32_t s = pc % TC_STAGES, ph = (pc / TC_STAGES) & 1u;
-                    const long long t0 = clock64();
                     tc_wait(&empty[s], ph ^ 1u);
-                    if (a.prof && blockIdx.x == 0) a.prof[0] += clock64() - t0;
-                    const uint32_t bytes = static_cast<uint32_t>(P.C[c].bytes);
+                    const uint32_t bytes = static_cast<uint32_t>(P.C[c].bytes);   // <= TC_STAGE_BYTES
                     mbar_expect_tx(&full[s], bytes);
-                    // several smaller bulk copies per chunk: one cp.async.bulk keeps only a few lines in flight
-                    const uint32_t piece = TC_STAGE_BYTES >> ((a.dbg >> 4) & 7);
-                    for (uint32_t o = 0; o < bytes; o += piece)
-                        tma_bulk_g2s(ring + s * TC_STAGE_BYTES + o, reinterpret_cast<const unsigned char *>(wbase + P.C[c].off) + o,
-                                     min(piece, bytes - o), &full[s]);
+                    tma_bulk_g2s(ring + s * TC_STAGE_BYTES, reinterpret_cast<const unsigned char *>(wbase + P.C[c].off),
+                                 bytes, &full[s]);
                 }
             }
         }
@@ -428,14 +145,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) pinnsf_tc_kernel(const __grid_c
                 const uint32_t lbo = Ly.N * 16, sbo = 128, kstep = 2 * lbo;
                 bool acc = false;
                 for (int c = 0; c < Ly.nchunks; ++c, ++pc) {
-                    const long long t0 = clock64();
                     tc_wait(&a_ready[c], (aph >> c) & 1u);         // A columns of this K chunk are in TMEM
                     aph ^= (1u << c);
-                    const long long t1 = clock64();
                     const uint32_t s = pc % TC_STAGES, ph = (pc / TC_STAGES) & 1u;
                     tc_wait(&full[s], ph);
                     tc::fence_after_sync();
-                    const long long t2 = clock64();
                     const TcChunk &Ch = P.C[Ly.chunk0 + c];
                     const uint32_t hi_addr = ring_addr + s * TC_STAGE_BYTES;
                     uint64_t bh = tc::smem_desc(hi_addr, lbo, sbo);
@@ -444,28 +158,18 @@ __global__ void __launch_bounds__(TC_THREADS, 1) pinnsf_tc_kernel(const __grid_c
                     uint32_t ah = tb + TC_COL_AH + c * 32, al = tb + TC_COL_AL + c * 32;
                     const int nks = Ch.cells / 2;
                     if (tc::elect_one()) {
-                        if (a.dbg & 2) {
-                            for (int ks = 0; ks < nks; ++ks, bh += dstep, ah += 8) {
-                                tc::mma_tf32_ts(dcol, ah, bh, idesc, acc);
-                                acc = true;
-                            }
-                        } else {
 #pragma unroll 4
-                            for (int ks = 0; ks < nks; ++ks, bh += dstep, bl += dstep, ah += 8, al += 8) {
-                                tc::mma_tf32_ts(dcol, al, bh, idesc, acc);      // x_lo w_hi
-                                tc::mma_tf32_ts(dcol, ah, bl, idesc, true);     // x_hi w_lo
-                                tc::mma_tf32_ts(dcol, ah, bh, idesc, true);     // x_hi w_hi
-                                acc = true;
-                            }
+                        for (int ks = 0; ks < nks; ++ks, bh += dstep, bl += dstep, ah += 8, al += 8) {
+                            tc::mma_tf32_ts(dcol, al, bh, idesc, acc);      // x_lo w_hi
+                            tc::mma_tf32_ts(dcol, ah, bl, idesc, true);     // x_hi w_lo
+                            tc::mma_tf32_ts(dcol, ah, bh, idesc, true);     // x_hi w_hi
+                            acc = true;
                         }
                         tc::commit(&empty[s]);                     // ring stage free once these MMAs have read it
                         if (c == Ly.nchunks - 1) tc::commit(&d_ready[li & 1]);   // accumulator of this layer complete
                     }
                     acc = true;
                     __syncwarp();
-                    if (a.prof && blockIdx.x == 0 && lane == 0) {
-                        a.prof[1] += t1 - t0; a.prof[2] += t2 - t1; a.prof[3] += clock64() - t2;
-                    }
                 }
             }
         }
@@ -552,20 +256,14 @@ __global__ void __launch_bounds__(TC_THREADS, 1) pinnsf_tc_kernel(const __grid_c
                 const bool last = li == P.nl - 1;
                 const bool to_sum = P.kind == 1 && li == P.n_enc - 1;        // kind 1: sum the slot embeddings per agent
                 const uint32_t dcol = tl + ((li & 1) ? TC_COL_D1 : TC_COL_D0);
-                const long long e0 = clock64();
                 tc_wait(&d_ready[li & 1], (dph >> (li & 1)) & 1u);
                 dph ^= (1u << (li & 1));
                 tc::fence_after_sync();
-                if (a.prof && blockIdx.x == 0 && tid == 64) a.prof[4 + li] += clock64() - e0;
                 const float *bias = bb + Ly.bias_off;
                 // every 32-column group is converted by BOTH warps of the lane quarter (16 columns each), so that
                 // the first K chunk of the next layer is released after half the latency
                 for (int g = 0; g < Ly.N / 32; ++g) {
                     const int n0 = g * 32 + half * 16;
-                    if (a.dbg & 1) {                               // timing experiment: no epilogue work at all
-                        if (!last) { tc::fence_before_sync(); tc::mbar_arrive(&a_ready[g]); }
-                        continue;
-                    }
                     uint32_t r[16];
                     tc::ld16(dcol + n0, r);
                     tc::wait_ld();
@@ -605,7 +303,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) pinnsf_tc_kernel(const __grid_c
                     tc::mbar_arrive(&a_ready[g]);                  // K chunk g of the next layer may start
                 }
             }
-            if (a.prof && blockIdx.x == 0 && tid == 64) a.prof[15] += 1;
             // combine the two column halves of the predictor, then sum over an agent's slots
             small[(half * 128 + m) * 2] = m0;
             small[(half * 128 + m) * 2 + 1] = m1;
@@ -961,6 +658,8 @@ static int tc_scratch_get(cudaStream_t st, int64_t floats, float **out) {
 
 }  // namespace piml
 
+using namespace piml;
+
 extern "C" int64_t piml_pinnsf_packed_tc_floats(const piml_net_desc *desc) {
     if (!desc) return -1;
     TcPlan P;
@@ -1033,12 +732,10 @@ extern "C" int piml_pinnsf_forward_tc_f32(const piml_net_desc *desc, const float
     if (R == 0) return PIML_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     float *scratch = nullptr;
-    // compact mode: network kind 0, messages not requested (PIML_TC_COMPACT=0 disables it)
-    const char *cenv = getenv("PIML_TC_COMPACT");                  // read per call: tests compare both modes
-    const bool compact_env = !(cenv && atoi(cenv) == 0);
-    // (a scene whose dense tiles fit one wave gains nothing from it and would pay two more launches)
+    // compact mode: messages not requested and the dense tiles exceed one wave (a scene whose dense tiles fit one wave
+    // gains nothing from it and would pay two more launches)
     const int64_t dense_tiles = (R + 128 / kp - 1) / (128 / kp) + ((has_obs && ko) ? (R + 128 / ko - 1) / (128 / ko) : 0);
-    const bool compact_ok = compact_env && !ped_msgs && !obs_msgs && dense_tiles > sm_count() &&
+    const bool compact_ok = !ped_msgs && !obs_msgs && dense_tiles > sm_count() &&
                             R * static_cast<int64_t>(kp > ko ? kp : ko) < (1LL << 31);
     const bool compact = compact_ok && P.kind == 0;               // row level (per-slot decoders)
     const bool compact2 = compact_ok && P.kind == 1;              // agent level (summed embeddings)
@@ -1065,8 +762,6 @@ extern "C" int piml_pinnsf_forward_tc_f32(const piml_net_desc *desc, const float
     a.n_ped_tiles = (R + a.ag_ped - 1) / a.ag_ped;
     a.n_obs_tiles = has_obs ? (R + a.ag_obs - 1) / a.ag_obs : 0;
     a.sums = scratch; a.ped_msgs = ped_msgs; a.obs_msgs = has_obs ? obs_msgs : nullptr;
-    a.dbg = 0;
-    a.prof = nullptr;
     a.compact = compact ? 1 : (compact2 ? 2 : 0);
     a.has_obs = has_obs ? 1 : 0;
     a.list_ped = a.list_obs = nullptr; a.counts = nullptr; a.cmsg_ped = a.cmsg_obs = a.f0 = nullptr;
@@ -1086,13 +781,6 @@ extern "C" int piml_pinnsf_forward_tc_f32(const piml_net_desc *desc, const float
         count_launch();
         rc = check_launch("tc_compact_kernel");
         if (rc) return rc;
-    }
-    if (const char *e = getenv("PIML_TC_DEBUG")) a.dbg = atoi(e);
-    if (getenv("PIML_TC_PROF")) {
-        static long long *prof_buf = nullptr;
-        if (!prof_buf) { PIML_CUDA(cudaMalloc(&prof_buf, 512 * sizeof(long long))); }
-        PIML_CUDA(cudaMemsetAsync(prof_buf, 0, 512 * sizeof(long long), st));
-        a.prof = prof_buf;
     }
     const size_t smem = static_cast<size_t>(TC_STAGES) * TC_STAGE_BYTES +
                         sizeof(float) * (2 * P.bias_floats + 512 + 2 * 128 * TC_STAGE_LD) + 8 * (2 * TC_STAGES + 6) + 64;
@@ -1121,12 +809,10 @@ extern "C" int piml_pinnsf_forward_tc_f32(const piml_net_desc *desc, const float
     }
     const int64_t tiles = compact ? (rows_ped + 128) / 128 + (has_obs ? (rows_obs + 128) / 128 : 0)
                                   : a.n_ped_tiles + a.n_obs_tiles + (compact2 ? 2 : 0);
-    // 16-bit path (two tiles in flight, resident weights): per-slot-decoder networks; PIML_TC_F16=0 keeps the tf32 kernel
+    // 16-bit path (two tiles in flight, resident weights) for every network its plan accepts; the agent-compact mode
+    // (summed-embedding networks) only exists in the tf32 kernel
     Tc16Plan P16;
-    const char *e16 = getenv("PIML_TC_F16");
-    const bool use16 = !(e16 && atoi(e16) == 0) && !compact2 && tc16_build_plan(desc, P.total, &P16) == 0 &&
-                       (!has_obs || tiles >= 2);
-    if (use16) {
+    if (!compact2 && tc16_build_plan(desc, P.total, &P16) == 0) {
         Tc16Args b;
         b.params = packed_tc; b.ped = ped; b.obs = obs; b.R = R; b.kp = kp; b.ko = ko;
         b.ag_ped = a.ag_ped; b.ag_obs = a.ag_obs; b.n_ped_tiles = a.n_ped_tiles; b.n_obs_tiles = a.n_obs_tiles;
@@ -1134,50 +820,14 @@ extern "C" int piml_pinnsf_forward_tc_f32(const piml_net_desc *desc, const float
         b.compact = compact ? 1 : 0; b.has_obs = a.has_obs;
         b.list_ped = a.list_ped; b.list_obs = a.list_obs; b.counts = a.counts;
         b.cmsg_ped = a.cmsg_ped; b.cmsg_obs = a.cmsg_obs; b.f0 = a.f0;
-        b.prof = a.prof; b.dbg = a.dbg;
         rc = tc16_launch(P16, b, tiles, st);
-        if (rc) return rc;
-        if (a.prof) {
-            long long h[512];
-            PIML_CUDA(cudaMemcpyAsync(h, a.prof, sizeof(h), cudaMemcpyDeviceToHost, st));
-            PIML_CUDA(cudaStreamSynchronize(st));
-            {
-                long long kmin = 1LL << 62, kmax = 0, lmax = 0; int imax = 0;
-                for (int c = 0; c < 148; ++c) {
-                    const long long k = h[16 + 3 * c];
-                    if (k == 0) continue;
-                    if (k < kmin) kmin = k;
-                    if (k > kmax) { kmax = k; imax = c; }
-                    if (h[17 + 3 * c] > lmax) lmax = h[17 + 3 * c];
-                }
-                fprintf(stderr, "[tc16 prof] kernel cycles per CTA: min %lld max %lld (CTA %d, %lld tiles); CTA 0: %lld, slot-0 loop %lld, "
-                        "%lld tiles; CTA 147: %lld, %lld tiles; longest slot-0 loop %lld\n", kmin, kmax, imax, h[18 + 3 * imax],
-                        h[16], h[17], h[18], h[16 + 3 * 147], h[18 + 3 * 147], lmax);
-            }
-            const long long t = h[15] > 0 ? h[15] : 1;
-            fprintf(stderr, "[tc16 prof, CTA 0, %lld tiles] cycles/tile: mma wait A %lld, wait W %lld, issue %lld | epilogue (slot 0, "
-                    "warp 2): wait D %lld, ld %lld, pass1 %lld, max exchange %lld, pass2 %lld, st+signal %lld, tile start %lld, "
-                    "predictor + tile end %lld, whole tile %lld\n", t, h[0] / t,
-                    h[1] / t, h[2] / t, h[3] * 2 / t, h[4] * 2 / t, h[5] * 2 / t, h[6] * 2 / t, h[7] * 2 / t, h[8] * 2 / t,
-                    h[10] * 2 / t, h[9] * 2 / t, h[11] * 2 / t);
-            a.prof = nullptr;
-        }
     } else {
-    const int grid = static_cast<int>(tiles < sm_count() ? tiles : sm_count());
-    pinnsf_tc_kernel<<<grid, TC_THREADS, smem, st>>>(P, a);
-    count_launch();
-    rc = check_launch("pinnsf_tc_kernel");
+        const int grid = static_cast<int>(tiles < sm_count() ? tiles : sm_count());
+        pinnsf_tc_kernel<<<grid, TC_THREADS, smem, st>>>(P, a);
+        count_launch();
+        rc = check_launch("pinnsf_tc_kernel");
+    }
     if (rc) return rc;
-    }
-    if (a.prof) {
-        long long h[16];
-        PIML_CUDA(cudaMemcpyAsync(h, a.prof, sizeof(h), cudaMemcpyDeviceToHost, st));
-        PIML_CUDA(cudaStreamSynchronize(st));
-        fprintf(stderr, "[tc prof, CTA 0, %lld tiles] cycles/tile: producer wait empty %lld | mma wait A %lld, wait W %lld, issue %lld | "
-                "epilogue wait D per layer:", h[15], h[0] / h[15], h[1] / h[15], h[2] / h[15], h[3] / h[15]);
-        for (int i = 0; i < 8; ++i) fprintf(stderr, " %lld", h[4 + i] / h[15]);
-        fprintf(stderr, "\n");
-    }
     const int threads = 256;
     if (compact2) {
         pinnsf_tc_finish_compact2_kernel<<<static_cast<unsigned>((2 * R + threads - 1) / threads), threads, 0, st>>>(

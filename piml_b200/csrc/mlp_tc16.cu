@@ -15,7 +15,7 @@
 // weights or activations:  * per layer (pack time): W * 2^e_l with max|W| in [2^13, 2^14);
 //                          * per tile row and layer (epilogue): y * 2^s with max|y_row| in [2^14, 2^15);
 // both are undone in the next epilogue (y = D * 2^-s * 2^-e_l + b).  The split drops lo*lo = O(2^-22): measured
-// 6.8e-7 of fp64 for a 128 x 128 x 128 layer (3xTF32: 1.0e-6; scripts/probe_tc16.py).
+// 6.8e-7 of fp64 for a 128 x 128 x 128 layer (3xTF32: 1.0e-6).
 //
 // Per CTA (persistent, one per SM, ONE branch per CTA, 576 threads):
 //   warp 0   : loads the branch's weight images (hi + lo per layer, UMMA K-major core matrices written by
@@ -27,8 +27,6 @@
 //              the two halves through shared memory) -> scale, split into fp16 hi / lo pairs, tcgen05.st as the NEXT
 //              layer's A operand; the 2-wide predictor and the slot sums run on the CUDA cores in fp32.
 // TMEM columns of slot s: D [256 s, +128), A_hi [256 s + 128, +64), A_lo [256 s + 192, +64).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tc.cuh"
 #include "mlp_tc16.cuh"
@@ -51,10 +49,7 @@ __device__ __forceinline__ void row_scale(float mx, float &s, float &inv_s) {
     inv_s = __uint_as_float(static_cast<uint32_t>(E - 14) << 23);
 }
 
-// PROF: in-kernel cycle counters (PIML_TC_PROF); compiled out of the production instantiation (the clock reads and
-// their branches were 4 % of the epilogue's instructions).
-#define T16_CLOCK() (PROF ? clock64() : 0LL)
-template <bool PROF, bool COMPACT>
+template <bool COMPACT>
 __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __grid_constant__ Tc16Plan P,
                                                                      const __grid_constant__ Tc16Args a) {
     extern __shared__ __align__(128) unsigned char t16_smem[];
@@ -64,10 +59,7 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
     uint64_t *bars = reinterpret_cast<uint64_t *>(small + 2048);
     uint64_t *w_ready = bars, *a_ready = bars + T16_MAXL, *d_ready = a_ready + 2;
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(d_ready + 2);
-    long long *sprof = reinterpret_cast<long long *>(d_ready + 4);     // [16] cycle counters (PIML_TC_PROF), flushed at the end
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid < 16) sprof[tid] = 0;
-    const long long k_start = T16_CLOCK();
 
     if (warp == 0) tc::tmem_alloc(tmem_slot, 512);
     if (tid == 32) {
@@ -139,13 +131,10 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                 any = true;
                 const int li = layer[s];
                 const Tc16Layer &Ly = P.L[li];
-                const long long p0 = T16_CLOCK();
                 t16_wait(&a_ready[s], (aph >> s) & 1u);            // A of (this slot's tile, layer li) is in TMEM
                 aph ^= (1u << s);
-                const long long p1 = T16_CLOCK();
                 if (!((wseen >> li) & 1u)) { t16_wait(&w_ready[li], 0); wseen |= (1u << li); }
                 tc::fence_after_sync();
-                const long long p2 = T16_CLOCK();
                 const uint32_t dcol = tb + s * T16_SLOT_COLS + T16_COL_D;
                 uint32_t ah = tb + s * T16_SLOT_COLS + T16_COL_AH, al = tb + s * T16_SLOT_COLS + T16_COL_AL;
                 const uint32_t idesc = tc::idesc_f16(Ly.N);
@@ -167,10 +156,6 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                     tc::commit(&d_ready[s]);                       // accumulator of this (slot, layer) complete
                 }
                 __syncwarp();
-                if (PROF && a.prof && lane == 0) {
-                    sprof[0] += p1 - p0; sprof[1] += p2 - p1; sprof[2] += T16_CLOCK() - p2;
-                    if (li == 0) sprof[15] += 1;
-                }
                 if (++layer[s] == P.nl) { layer[s] = 0; ++done[s]; }
             }
             if (!any) break;
@@ -257,30 +242,15 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
             const int64_t row0 = agent0 * k;
             float inv_s_next = 1.f;
             int crow_next = -1;
-            const long long t0 = T16_CLOCK();
-            long long tl2 = t0;
             float m0 = 0.f, m1 = 0.f;
             for (int li = 0; li < P.nl; ++li) {
                 const Tc16Layer &Ly = P.L[li];
                 const bool last = li == P.nl - 1;
                 const int hc = Ly.N >> 1;                          // columns of this thread: [half * hc, +hc), 16 at a time
                 const int nchunk = hc >> 4;
-                const long long q0 = T16_CLOCK();
                 t16_wait(&d_ready[slot], dph);
                 dph ^= 1u;
                 tc::fence_after_sync();
-                const long long q1 = T16_CLOCK();
-                const bool prof = PROF && a.prof && tid == 64;
-                if (prof) sprof[3] += q1 - q0;
-                if (a.dbg & 1) {                                   // timing experiment: no epilogue work at all
-                    if (!last) { tc::fence_before_sync(); tc::mbar_arrive(&a_ready[slot]); }
-                    else {
-                        const RowFeat nxt = load_row(j + 2);
-                        crow_next = nxt.crow;
-                        if (j + 2 < my_tiles) write_features(nxt, inv_s_next);
-                    }
-                    continue;
-                }
                 const float *bias = biasb + Ly.bias_off + half * hc;
                 const float sc = inv_s * biasb[P.winv_off + li];   // undo the input's row scale and the layer's weight scale
                 // all of this thread's columns in one go: the loads overlap, one wait
@@ -299,8 +269,6 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                     crow_next = nxt.crow;
                     if (j + 2 < my_tiles) write_features(nxt, inv_s_next);
                 }
-                const long long q2 = T16_CLOCK();
-                if (prof) sprof[4] += q2 - q1;
                 float *v = reinterpret_cast<float *>(r);
                 float mx = 0.f, mxb4[4] = {0.f, 0.f, 0.f, 0.f};   // four independent maximum chains (ILP), merged below
                 const float2 sc2 = make_float2(sc, sc);
@@ -324,7 +292,6 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                 }
                 mx = fmaxf(fmaxf(mxb4[0], mxb4[1]), fmaxf(mxb4[2], mxb4[3]));
                 if (last) {                                        // predictor Linear(dw, 2) on the CUDA cores
-                    tl2 = q2;
                     const float *w0 = biasb + P.predw_off + half * hc, *w1 = w0 + P.dw;
 #pragma unroll
                     for (int c = 0; c < 4; ++c)
@@ -337,14 +304,10 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                         }
                     break;
                 }
-                const long long q3 = T16_CLOCK();
-                if (prof) sprof[5] += q3 - q2;
                 float *mxb = smax + (li & 1) * 256;                // double buffered: one barrier per layer is enough
                 mxb[half * 128 + m] = mx;                          // row maximum over both column halves
                 slot_barrier(slot);
                 mx = fmaxf(mx, mxb[(half ^ 1) * 128 + m]);
-                const long long q4c = T16_CLOCK();
-                if (prof) sprof[6] += q4c - q3;
                 float s;
                 row_scale(mx, s, inv_s);
                 // Split relative to the ROW: after scaling, |x| < 2^15; hi = x rounded to a multiple of 16 (the fp16
@@ -367,11 +330,9 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                         tc::st8(tl + T16_COL_AL + ((half * hc + c * 16) >> 1), lo);
                     }
                 }
-                const long long q5 = T16_CLOCK();
                 tc::wait_st();
                 tc::fence_before_sync();
                 tc::mbar_arrive(&a_ready[slot]);                   // the next layer of this slot may start
-                if (prof) { sprof[7] += q5 - q4c; sprof[8] += T16_CLOCK() - q5; }
             }
             // combine the two column halves of the predictor: half 1 hands its partial sums over and moves on
             // (bar.arrive), only half 0 waits (the next write of sm2 is several slot barriers away)
@@ -404,21 +365,19 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                 slot_barrier(slot);                                // sm2 is free for this slot's next tile
             }
             inv_s = inv_s_next; crow = crow_next;
-            if (PROF && a.prof && tid == 64) { const long long te = T16_CLOCK(); sprof[9] += te - tl2; sprof[11] += te - t0; }
         }
     }
     tc::fence_before_sync();
     __syncthreads();
     if (warp == 0) tc::tmem_dealloc(tbase, 512);
-    if (PROF && a.prof && blockIdx.x == 0 && tid < 16) a.prof[tid] = sprof[tid];
-    if (PROF && a.prof && tid == 64 && blockIdx.x < 160) {                 // per CTA: whole kernel, slot-0 tile loop, tiles
-        a.prof[16 + 3 * blockIdx.x] = T16_CLOCK() - k_start;
-        a.prof[17 + 3 * blockIdx.x] = sprof[11];
-        a.prof[18 + 3 * blockIdx.x] = my_tiles;
-    }
 }
 
 // ---- plan ------------------------------------------------------------------------------------------------------------
+// weight images | bias block | row maxima and predictor scratch (2 slots x 1024 floats) | mbarriers | TMEM address
+size_t tc16_smem_bytes(const Tc16Plan &P) {
+    return static_cast<size_t>(P.w_bytes) + sizeof(float) * (P.bias_floats + 2048) + 8 * (T16_MAXL + 4) + 16;
+}
+
 // Layers as the tf32 plan lists them (K, N, relu, ResDNN 2x fold): enc..., dec...; K padded to 16.
 int tc16_build_plan(const piml_net_desc *d, int64_t base_floats, Tc16Plan *P) {
     if (d->kind != 0 || d->proc_mode != 0 || d->enc_dims[0] != 6) return 1;       // per-slot-decoder networks only
@@ -446,13 +405,10 @@ int tc16_build_plan(const piml_net_desc *d, int64_t base_floats, Tc16Plan *P) {
     P->bias_floats = (boff + 3) & ~3;
     P->branch_floats = P->w_bytes / 4 + P->bias_floats;
     P->base = (base_floats + 31) & ~static_cast<int64_t>(31);      // 128-byte aligned behind the tf32 image
-    const size_t smem = static_cast<size_t>(P->w_bytes) + sizeof(float) * (P->bias_floats + 2048) + 8 * (T16_MAXL + 4) + 16 + 128;
-    if (smem > 220 * 1024) return 1;                               // the branch must stay resident in shared memory
+    // the branch must stay resident in shared memory.  220 KB - 128 B: the kernel's shared memory used to include 128 B
+    // of cycle counters; the limit moved down with them, so that every network keeps the kernel it ran on
+    if (tc16_smem_bytes(*P) > 220 * 1024 - 128) return 1;
     return 0;
-}
-
-size_t tc16_smem_bytes(const Tc16Plan &P) {
-    return static_cast<size_t>(P.w_bytes) + sizeof(float) * (P.bias_floats + 2048) + 8 * (T16_MAXL + 4) + 16 + 128;
 }
 
 // ---- packing -----------------------------------------------------------------------------------------------------------
@@ -539,17 +495,10 @@ int tc16_pack(const Tc16Plan &P, const Tc16Src &S, const float *params_torch, fl
 int tc16_launch(const Tc16Plan &P, const Tc16Args &a, int64_t tiles_bound, cudaStream_t st) {
     const size_t smem = tc16_smem_bytes(P);
     const int grid = static_cast<int>(tiles_bound < sm_count() ? tiles_bound : sm_count());
-    // (the compact / dense and the profiling variants are separate instantiations: at the epilogue's 96-register ceiling
-    // every dead path costs spills)
-#define T16_LAUNCH(PROF_, COMPACT_)                                                                                        \
-    do {                                                                                                                   \
-        PIML_CUDA(cudaFuncSetAttribute(pinnsf_tc16_kernel<PROF_, COMPACT_>, cudaFuncAttributeMaxDynamicSharedMemorySize,   \
-                                       static_cast<int>(smem)));                                                           \
-        pinnsf_tc16_kernel<PROF_, COMPACT_><<<grid, T16_THREADS, smem, st>>>(P, a);                                        \
-    } while (0)
-    if (a.prof) { if (a.compact) T16_LAUNCH(true, true); else T16_LAUNCH(true, false); }
-    else { if (a.compact) T16_LAUNCH(false, true); else T16_LAUNCH(false, false); }
-#undef T16_LAUNCH
+    // (compact and dense are separate instantiations: at the epilogue's 96-register ceiling every dead path costs spills)
+    const auto kernel = a.compact ? pinnsf_tc16_kernel<true> : pinnsf_tc16_kernel<false>;
+    PIML_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    kernel<<<grid, T16_THREADS, smem, st>>>(P, a);
     count_launch();
     return check_launch("pinnsf_tc16_kernel");
 }

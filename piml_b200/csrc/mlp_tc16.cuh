@@ -32,8 +32,6 @@ struct Tc16Args {
     int compact, has_obs;
     const int *list_ped, *list_obs; const int *counts;   // lists NULL: ped / obs hold the compact rows themselves (nn_step.cu)
     float *cmsg_ped, *cmsg_obs; float *f0;
-    long long *prof;                           // optional cycle counters of CTA 0 (PIML_TC_PROF, bring-up only)
-    int dbg;                                   // timing experiments only (PIML_TC_DEBUG): 1 = no epilogue work, 4 = no TMEM ld/st
 };
 
 int tc16_build_plan(const piml_net_desc *d, int64_t base_floats, Tc16Plan *P);   // 0 = the network fits this path

@@ -215,7 +215,6 @@ int nn_step_launch(const piml_nn_step_args *r, const int *t_dev, cudaStream_t st
     b.compact = 1; b.has_obs = has_obs;
     b.list_ped = nullptr; b.list_obs = nullptr; b.counts = counts;
     b.cmsg_ped = msg_p; b.cmsg_obs = msg_o; b.f0 = f0;
-    b.prof = nullptr; b.dbg = 0;
     const int64_t tiles = (rows_ped + 128) / 128 + (has_obs ? (rows_obs + 128) / 128 : 0);
     rc = tc16_launch(P16, b, tiles < 2 ? 2 : tiles, st);
     if (rc) return rc;

@@ -9,7 +9,6 @@ the same `torch.manual_seed` gives the same initial weights), but `forward` runs
 `forward_from_module(module, ped, obs, self)` runs the same kernel on the weights of an UNMODIFIED reference
 module; piml_b200.patch uses it to drop the CUDA path in behind `model(*state_features)`.
 """
-import os
 
 import torch
 import torch.nn as nn
@@ -135,11 +134,6 @@ def pack_device(sd, spec, device=None):
     return out
 
 
-def tc_enabled():
-    """The tensor-core forward is on unless PIML_MLP_TC=0 (A/B switch for measurements)."""
-    return os.environ.get("PIML_MLP_TC", "1") != "0"
-
-
 def pack_device_tc(sd, spec, device=None):
     """Parameter layout of the tensor-core forward (piml_pinnsf_pack_tc_f32): per Linear the tf32 hi / lo images of the
     weight as UMMA K-major core matrices, fp32 biases and predictor.  Returns None when the network cannot run on the
@@ -182,7 +176,7 @@ def pinnsf_forward(spec, packed, ped_features, obs_features, self_features, drop
         ko = obs.shape[-2]
     acc = torch.empty(*lead, 2, dtype=torch.float32, device=dev)
     mw = spec.msg_width
-    use_tc = (packed_tc is not None and drop_ped is None and drop_obs is None and tc_enabled()
+    use_tc = (packed_tc is not None and drop_ped is None and drop_obs is None
               and (not need_msgs or (spec.kind == 0 and not spec.coll_dims)))
     if use_tc:
         pm = torch.empty(*lead, kp, 2, dtype=torch.float32, device=dev) if need_msgs else None

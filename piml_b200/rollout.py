@@ -182,7 +182,7 @@ def rollout_scenes(spec, packed, args, scene, t_start=0, num_frames=None, packed
         desc = spec.desc()
         r.desc = L.C.pointer(desc)
         r.packed = L.ptr(packed)
-        r.packed_tc = L.ptr(packed_tc) if (packed_tc is not None and M.tc_enabled()) else None
+        r.packed_tc = L.ptr(packed_tc) if packed_tc is not None else None
     r.has_obs, r.tau = (1 if (spec.has_obs and Mo) else 0), spec.tau
     r.S, r.N, r.M, r.D, r.T, r.t_start, r.dt = S, N, Mo, wp.shape[-3], T, t_start, dt
     r.kp, r.cos_p, r.thr_p = args.topk_ped, cos_threshold(args.sight_angle_ped), float(args.dist_threshold_ped)

@@ -210,7 +210,7 @@ class ShardedNNCrowd(object):
         self.obstacles = L.f32c(obstacles.to(self.device))
         self.Mo = self.obstacles.shape[-2] if self.obstacles.numel() else 0
         can_fuse = False
-        if not self.sfm and self.packed_tc is not None and M.tc_enabled():
+        if not self.sfm and self.packed_tc is not None:
             self._desc = self.spec.desc()
             can_fuse = bool(L.load().piml_nn_step_supported(C.byref(self._desc))) and self.world <= 8
         self.fused = can_fuse if fused is None else (bool(fused) and can_fuse)

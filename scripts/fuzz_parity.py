@@ -1,7 +1,8 @@
 """Randomised self-consistency sweep on the GPU (bounded by --seconds): pairs of independent evaluations that must agree
    1. MLAPM symmetric kernel vs ordered-pair kernel, random N in [2, 40000], versions raw / GC, stationary / NaN agents
    2. cell-list vs all-pairs neighbour features, random N, M, k, angles, thresholds: bit-identical
-   3. tensor-core forward compact vs dense (pinnsf_bm row level, pinnsf_m agent level): bit-identical
+   3. tensor-core forward compact vs dense (pinnsf_bm row level, pinnsf_m agent level), the dense reference evaluated
+      in chunks whose dense tiles fit one wave: bit-identical
    4. persistent social-force rollout kernel vs the per-step route: bit-identical
    5. fused NN step (piml_nn_step_f32) vs state_features -> pinnsf_forward -> integrate_step, and the rollout loop with the
       fused step forced vs the per-stage loop: random scenes / sizes / k / angles / thresholds, absent agents: bit-identical
@@ -76,7 +77,9 @@ def fuzz_features():
 
 
 def fuzz_tc():
+    from tests.util import tc_forward_in_dense_chunks
     t0, n = time.time(), 0
+    sms = torch.cuda.get_device_properties(dev).multi_processor_count
     nets = {}
     for kind in ("pinnsf_bm", "pinnsf_m"):
         torch.manual_seed(1)
@@ -92,12 +95,9 @@ def fuzz_tc():
         ped[torch.rand(R, generator=g) < pz] = 0; obs[torch.rand(R, generator=g) < 0.9] = 0
         slf = torch.randn(R, 7, generator=g)
         ped, obs, slf = ped.to(dev), obs.to(dev), slf.to(dev)
-        outs = {}
-        for mode in ("1", "0"):
-            os.environ["PIML_TC_COMPACT"] = mode
-            outs[mode] = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=False, packed_tc=ptc)[0].clone()
-        os.environ.pop("PIML_TC_COMPACT", None)
-        assert torch.equal(outs["1"], outs["0"]), ("tc compact", kind, R, pz)
+        compact = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=False, packed_tc=ptc)[0]
+        dense = tc_forward_in_dense_chunks(net.spec, packed, ptc, ped, obs, slf, sms)[0]
+        assert torch.equal(compact, dense), ("tc compact", kind, R, pz)
         n += 1
     print(f"tensor-core forward compact vs dense: {n} batches, bit-identical")
 
@@ -211,33 +211,34 @@ def fuzz_nn_step():
 
 
 def fuzz_tc_vs_fp32():
-    """6. both tensor-core forwards (fp16 split / 3xTF32, dense and compact as the size decides) vs the FP32-pipe kernel:
-    random row counts, topk, zero-slot patterns, with and without the per-slot messages; 1e-5 of the summed operands."""
+    """6. both tensor-core forwards (dense and compact as the size decides) vs the FP32-pipe kernel: pinnsf_bm on the
+    fp16-split kernel and, at width 96, on the 3xTF32 kernel; pinnsf_m on the 3xTF32 kernel.  Random row counts, topk,
+    zero-slot patterns, with and without the per-slot messages; 1e-5 of the summed operands."""
     from tests.util import accel_err
     t0, n, worst = time.time(), 0, 0.0
     nets = {}
-    for kind in ("pinnsf_bm", "pinnsf_m"):
+    for key, kind, width in (("pinnsf_bm", "pinnsf_bm", 128), ("pinnsf_bm_w96", "pinnsf_bm", 96),
+                             ("pinnsf_m", "pinnsf_m", 128)):
         torch.manual_seed(2)
-        net = M.CLASSES[kind](base_args(model=kind, dataset_name="gc1560")).to(dev).eval()
-        nets[kind] = (net, M.pack_device(net.state_dict(), net.spec, dev), M.pack_device_tc(net.state_dict(), net.spec, dev))
+        args = base_args(model=kind, dataset_name="gc1560", encoder_hidden_size=width, processor_hidden_size=width)
+        net = M.CLASSES[kind](args).to(dev).eval()
+        nets[key] = (net, M.pack_device(net.state_dict(), net.spec, dev), M.pack_device_tc(net.state_dict(), net.spec, dev))
     while time.time() - t0 < budget:
         kind = "pinnsf_bm" if rng.random() < 0.6 else "pinnsf_m"
-        net, packed, ptc = nets[kind]
         R = int(rng.integers(1, 9000)); kp = int(rng.integers(1, 9)); ko = int(rng.integers(1, 13)); pz = float(rng.random())
         g = torch.Generator().manual_seed(int(rng.integers(1 << 30)))
         ped = torch.randn(R, kp, 6, generator=g); obs = torch.randn(R, ko, 6, generator=g)
         ped[torch.rand(R, kp, generator=g) < pz] = 0; obs[torch.rand(R, ko, generator=g) < pz] = 0
         slf = torch.randn(R, 7, generator=g)
         ped, obs, slf = ped.to(dev), obs.to(dev), slf.to(dev)
-        ref = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=True)[0]
-        for f16 in ("1", "0"):
-            os.environ["PIML_TC_F16"] = f16
+        for key in (("pinnsf_bm", "pinnsf_bm_w96") if kind == "pinnsf_bm" else ("pinnsf_m",)):
+            net, packed, ptc = nets[key]
+            ref = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=True)[0]
             for need in ((False, True) if kind == "pinnsf_bm" else (False,)):
                 got = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=need, packed_tc=ptc)[0]
                 err = accel_err(got.cpu().numpy(), ref.cpu().numpy(), slf.cpu().numpy(), net.spec.tau)
                 worst = max(worst, err)
-                assert err < 1e-5, ("tc vs fp32", kind, R, kp, ko, pz, f16, need, err)
-        os.environ.pop("PIML_TC_F16", None)
+                assert err < 1e-5, ("tc vs fp32", key, R, kp, ko, pz, need, err)
         n += 1
     print(f"tensor-core forwards vs FP32-pipe forward: {n} batches, worst operand-scaled error {worst:.2e}")
 

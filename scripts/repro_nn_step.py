@@ -41,22 +41,17 @@ for it in range(400):
         pf, of, sf = state_features(A[0], A[1], A[2], A[3], obd, A[5], dsd, *fa)
         an = M.pinnsf_forward(net.spec, packed, pf.view(S * N, -1, 6), of.view(S * N, -1, 6), sf.view(S * N, 7),
                               need_msgs=False, packed_tc=ptc)[0].view(S, N, 2)
-        os.environ["PIML_TC_COMPACT"] = "0"
-        an_d = M.pinnsf_forward(net.spec, packed, pf.view(S * N, -1, 6), of.view(S * N, -1, 6), sf.view(S * N, 7),
-                                need_msgs=False, packed_tc=ptc)[0].view(S, N, 2)
-        os.environ.pop("PIML_TC_COMPACT")
         integrate_step(A[0], A[1], A[2], an, A[3], A[4], dn, wp, 0.08, True, hist_v=A[5])
         step.step()
         torch.cuda.synchronize()
         eq = lambda x, y: bool(torch.equal(torch.nan_to_num(x, nan=-7.0), torch.nan_to_num(y, nan=-7.0)))
-        names = ["ped_f", "obs_f", "self_f", "a_next(default)", "a_next(dense forced)"]
-        pairs = [(dense[0], pf), (dense[1], of), (dense[2], sf), (a_out, an), (a_out, an_d)]
+        names = ["ped_f", "obs_f", "self_f", "a_next"]
+        pairs = [(dense[0], pf), (dense[1], of), (dense[2], sf), (a_out, an)]
         msgs = [nm for nm, (x, y) in zip(names, pairs) if not eq(x, y)]
         if msgs:
             d = (torch.nan_to_num(a_out) - torch.nan_to_num(an)).abs()
             print(f"it {it} step {s_}: S={S} N={N} Mo={Mo} kp={kp} ko={ko} ang={ang} thr={thr}: differ: {msgs}; "
-                  f"a_next max diff {float(d.max()):.3e} on {int((d > 0).any(-1).sum())} agents; "
-                  f"an vs dense-forced equal: {eq(an, an_d)}", flush=True)
+                  f"a_next max diff {float(d.max()):.3e} on {int((d > 0).any(-1).sum())} agents", flush=True)
             bad += 1
             break
     if bad >= 6:

@@ -446,15 +446,17 @@ def test_pinnsf_forward_tensor_cores_vs_fp32_kernel(kind, R, kp, ko, chan, has_o
             assert float((got[2] - ref[2]).abs().max()) < TOL * float(ref[2].abs().max())
 
 
-@pytest.mark.parametrize("f16", ["1", "0"])
+@pytest.mark.parametrize("width,kernel", [(128, "pinnsf_tc16_kernel"), (96, "pinnsf_tc_kernel")])
 @pytest.mark.parametrize("R,kp,ko", [(700, 1, 1), (401, 1, 7), (333, 2, 1), (130, 3, 1)])
-def test_tensor_core_forward_with_one_slot_per_agent(R, kp, ko, f16, monkeypatch):
+def test_tensor_core_forward_with_one_slot_per_agent(R, kp, ko, width, kernel):
     """topk = 1 packs 128 agents into a dense tile: 256 slot sums for 128 threads (the dense mode of both tensor-core
-    kernels wrote only the first 64 agents' sums until round 2; found by scripts/fuzz_parity.py's fused-step family)."""
+    kernels wrote only the first 64 agents' sums until round 2; found by scripts/fuzz_parity.py's fused-step family).
+    Width 128 runs on the 16-bit kernel; width 96, a multiple of 32 that the 16-bit kernel does not take, on the
+    tf32 kernel.  The profiler shows which one ran."""
     from piml_b200 import models as M
     from .golden_args import base_args
-    monkeypatch.setenv("PIML_TC_F16", f16)
-    net = M.CLASSES["pinnsf_bm"](base_args(model="pinnsf_bm", dataset_name="gc1560")).cuda().eval()
+    args = base_args(model="pinnsf_bm", dataset_name="gc1560", encoder_hidden_size=width, processor_hidden_size=width)
+    net = M.CLASSES["pinnsf_bm"](args).cuda().eval()
     g = torch.Generator().manual_seed(R)
     ped = torch.randn(R, kp, 6, generator=g).cuda()
     obs = torch.randn(R, ko, 6, generator=g).cuda()
@@ -463,6 +465,11 @@ def test_tensor_core_forward_with_one_slot_per_agent(R, kp, ko, f16, monkeypatch
     packed = M.pack_device(net.state_dict(), net.spec)
     ptc = M.pack_device_tc(net.state_dict(), net.spec)
     ref = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=True)
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=False, packed_tc=ptc)
+        torch.cuda.synchronize()
+    names = [e.name for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA]
+    assert any(kernel + "(" in n or kernel + "<" in n for n in names), names
     for need in (False, True):
         got = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=need, packed_tc=ptc)
         err = accel_err(npy(got[0]), npy(ref[0]), npy(slf), net.spec.tau)
@@ -505,14 +512,18 @@ def test_tensor_core_compact_mode_is_bit_identical(R, kp, ko, pz, chan):
     assert err < TOL, err
 
 
-@pytest.mark.parametrize("R,kp,ko,pz,chan", [(6000, 6, 10, 0.75, 0), (3100, 6, 0, 0.5, 0), (5000, 4, 7, 0.9, 5)])
+@pytest.mark.parametrize("R,kp,ko,pz,chan", [(6000, 6, 10, 0.75, 0), (3100, 6, 0, 0.5, 0), (3300, 6, 0, 0.5, 0),
+                                             (5000, 4, 7, 0.9, 5)])
 def test_tensor_core_agent_compact_mode_is_bit_identical(R, kp, ko, pz, chan):
     """Summed-embedding networks (pinnsf_m, model.py:1274-1279): an agent whose slots are all zero (an absent agent, or
     one with no obstacle in range) yields the same per-branch output, so only the agents with a non-zero slot (+ one
-    all-zero agent per branch) go through the network.  Bit-identical to the dense evaluation (PIML_TC_COMPACT=0)."""
-    import os
-    from piml_b200 import models as M
+    all-zero agent per branch) go through the network.  Bit-identical to the dense evaluation, which the library runs
+    for the chunks of a batch whose dense tiles fit one wave.  Launch counts show each call's route: the agent-compact
+    mode adds tc_compact_agents_kernel, and runs when the whole batch's dense tiles exceed one wave (3100 agents with
+    6 slots and no obstacle branch are 148 tiles: dense on a 148-SM B200, compact with 3300)."""
+    from piml_b200 import _lib as L, models as M
     from .golden_args import base_args
+    from .util import dense_tile_count, tc_forward_in_dense_chunks
     has_obs = ko > 0
     args = base_args(model="pinnsf_m", dataset_name="gc1560", obs_feature_dim=6 if has_obs else 0)
     torch.manual_seed(R)
@@ -530,16 +541,16 @@ def test_tensor_core_agent_compact_mode_is_bit_identical(R, kp, ko, pz, chan):
     packed = M.pack_device(net.state_dict(), net.spec)
     ptc = M.pack_device_tc(net.state_dict(), net.spec)
     assert ptc is not None
-    outs = {}
-    for mode in ("1", "0"):
-        os.environ["PIML_TC_COMPACT"] = mode
-        try:
-            outs[mode] = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=False, packed_tc=ptc)[0].clone()
-        finally:
-            os.environ.pop("PIML_TC_COMPACT", None)
-    assert torch.equal(outs["1"], outs["0"])
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    l0 = L.launch_count()
+    full = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=False, packed_tc=ptc)[0]
+    launches = L.launch_count() - l0
+    dense, chunk_launches = tc_forward_in_dense_chunks(net.spec, packed, ptc, ped, obs, slf, sms)
+    compact = dense_tile_count(R, kp, ko) > sms
+    assert set(chunk_launches) == {launches - compact}, (launches, chunk_launches, compact)
+    assert torch.equal(full, dense)
     ref = M.pinnsf_forward(net.spec, packed, ped, obs, slf, need_msgs=True)
-    err = accel_err(npy(outs["1"]).reshape(-1, 2), npy(ref[0]).reshape(-1, 2), npy(slf).reshape(-1, 7), net.spec.tau)
+    err = accel_err(npy(full).reshape(-1, 2), npy(ref[0]).reshape(-1, 2), npy(slf).reshape(-1, 7), net.spec.tau)
     assert err < TOL, err
 
 

@@ -73,3 +73,30 @@ def accel_err(got, ref, self_f, tau):
     dterm = (self_f[:, 6:7] * self_f[:, :2] / n - self_f[:, 2:4]) / tau
     scale = np.maximum(np.maximum(np.linalg.norm(ref, axis=-1), np.linalg.norm(dterm, axis=-1)), 1e-3)
     return float((np.linalg.norm(got - ref, axis=-1) / scale).max())
+
+
+def dense_tile_count(n, kp, ko):
+    """128-row tiles of the tensor-core forward's dense mode for n agents with kp / ko slots (128 // k agents a tile
+    and branch; ko = 0: no obstacle branch).  The library runs the compact mode only when this exceeds the SM count."""
+    return -(-n // (128 // kp)) + (-(-n // (128 // ko)) if ko else 0)
+
+
+def tc_forward_in_dense_chunks(spec, packed, packed_tc, ped, obs, slf, sms):
+    """The tensor-core forward's acceleration without messages, evaluated in chunks of agents whose dense tiles fit
+    one wave of `sms` CTAs, so that every chunk runs in the dense mode.  Channelled (C,N,.) inputs are split by whole
+    channels, which keeps each channel's destination norm.  Returns the acceleration and each chunk's launch count."""
+    import torch
+    from piml_b200 import _lib as L, models as M
+    kp, ko = ped.shape[-2], (obs.shape[-2] if spec.has_obs else 0)
+    if slf.dim() == 3:
+        step = max(c for c in range(1, slf.shape[0] + 1) if dense_tile_count(c * slf.shape[1], kp, ko) <= sms)
+    else:
+        per_tile = [128 // kp] + ([128 // ko] if ko else [])
+        step = sms // len(per_tile) * min(per_tile)
+    accs, launches = [], []
+    for i in range(0, slf.shape[0], step):
+        l0 = L.launch_count()
+        accs.append(M.pinnsf_forward(spec, packed, ped[i:i + step], obs[i:i + step], slf[i:i + step], need_msgs=False,
+                                     packed_tc=packed_tc)[0])
+        launches.append(L.launch_count() - l0)
+    return torch.cat(accs), launches
