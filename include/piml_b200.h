@@ -333,6 +333,17 @@ PIML_API int piml_pinnsf_forward_tc_f32(const piml_net_desc *desc, const float *
                                const float *ped, const float *obs, const float *self, int64_t R, int kp, int ko,
                                int norm_group, float *acc, float *ped_msgs, float *obs_msgs, void *stream);
 
+/* The tensor-core forward under S networks of ONE description at once: set s evaluates rows [s N, (s+1) N) of ped
+ * (S N,kp,6), obs (S N,ko,6) and self (S N,7) with the piml_pinnsf_pack_tc_f32 vector at packed_tc + s set_stride
+ * and writes acc (S N,2).  set_stride: floats, a multiple of 4 and >= piml_pinnsf_packed_tc_floats(desc); packed_tc
+ * 16-byte aligned.  Each set's result equals piml_pinnsf_forward_tc_f32 on its rows and vector alone (norm_group 0,
+ * no messages), bit for bit.  The 16-bit kernel in dense mode, one (set, branch) per CTA with its weights resident;
+ * networks its plan does not accept (piml_nn_step_supported() == 0, e.g. kind 1) -> PIML_ERR_UNSUPPORTED.
+ * Uses the library's stream-keyed scratch (S N 4 floats). */
+PIML_API int piml_pinnsf_forward_tc_sets_f32(const piml_net_desc *desc, const float *packed_tc, int64_t set_stride,
+                                             int S, int has_obs, float tau, const float *ped, const float *obs,
+                                             const float *self, int64_t N, int kp, int ko, float *acc, void *stream);
+
 /* ---- training: forward with activation stash + backward (loss.backward(), simulators.py:359, through the models) -- */
 
 /* Floats of the activation stash of the training-mode forward for R agents (every Linear's post-activation output,
@@ -486,6 +497,43 @@ typedef struct {
 /* Workspace bytes piml_sfm_sweep_f32 needs for these sizes and the route it will take: O(S N), never O(S T N). */
 PIML_API int64_t piml_sfm_sweep_workspace_bytes(const piml_sfm_sweep_args *args);
 PIML_API int piml_sfm_sweep_f32(const piml_sfm_sweep_args *args, void *stream);
+
+/* ---- interaction-network sweep: one clip rolled out under S trained networks ------------------------------------- */
+
+/* piml_sfm_sweep_f32 with the social-force constants replaced by S networks of ONE description (the same class,
+ * widths and tau): checkpoint selection, seed ensembles and grid-search evaluation on one clip.  For each set s the
+ * trajectory equals piml_rollout_f32 on the clip alone with desc and the vector at packed_tc + s set_stride, bit for
+ * bit; the score is piml_sfm_sweep_f32's (the same definition, order and independence of S and position), so networks
+ * and social-force constant sets rank on one scale.  One route: per step the tensor-core forward with one network per
+ * set (piml_pinnsf_forward_tc_sets_f32), the state update and the feature rebuild on the (S,N) state.  Networks the
+ * 16-bit tensor-core forward does not take (piml_nn_step_supported() == 0) -> PIML_ERR_UNSUPPORTED.  The clip fields
+ * are piml_sfm_sweep_args'; all pointers are device pointers. */
+typedef struct {
+    int S, N, M, D, T, t_start; float dt;
+    int kp; float cos_p, thr_p; int ko; float cos_o, thr_o;            /* topk / cos(sight angle) / distance threshold */
+    const float *obstacles;                                             /* (M,2), NULL when M == 0 */
+    const float *pos_tm, *vel_tm, *acc_tm, *dest_tm;                    /* (T,N,2) */
+    const int64_t *dest_idx_tm;                                         /* (T,N) */
+    const int64_t *entry_tm;                                            /* (T,N) mask_p - mask_p_pred (simulators.py:593) */
+    const float *mask_p;                                                /* (T,N): the slots the score compares */
+    const int64_t *dest_num;                                            /* (N) */
+    const float *waypoints;                                             /* (D,N,2) */
+    const float *desired_speed;                                         /* (N) */
+    const float *p, *v, *a, *dest; const int64_t *dest_idx;             /* (N,..) state at t_start (read only) */
+    const float *ped_f, *obs_f, *self_f;                                /* (N,kp',6), (N,ko',6), (N,7) its features */
+    const piml_net_desc *desc;                                          /* the networks' common description */
+    const float *packed_tc;                                             /* S piml_pinnsf_pack_tc_f32 vectors, 16-byte aligned */
+    int64_t set_stride;                                                 /* floats between them: multiple of 4, >= packed_tc_floats */
+    int has_obs; float tau;                                             /* obstacle branch used; tau of every network */
+    double *err_sum; int64_t *err_count;                                /* (S) out */
+    float *rec_p, *rec_v, *rec_a, *rec_mask;  /* (T,S,N,2) x3, (T,S,N): rows t >= t_start written as piml_rollout_f32
+                                                 writes them; all four NULL for a score-only sweep */
+    void *workspace; int64_t workspace_bytes;                           /* >= piml_nn_sweep_workspace_bytes(args) */
+} piml_nn_sweep_args;
+
+/* Workspace bytes piml_nn_sweep_f32 needs for these sizes: O(S N), never O(S T N). */
+PIML_API int64_t piml_nn_sweep_workspace_bytes(const piml_nn_sweep_args *args);
+PIML_API int piml_nn_sweep_f32(const piml_nn_sweep_args *args, void *stream);
 
 /* ---- one NN-augmented rollout step, fused: src/models/simulators.py:595-652 ----------------------------------------- */
 

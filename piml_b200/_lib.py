@@ -56,6 +56,19 @@ class SfmSweepArgs(C.Structure):
                 ("workspace_bytes", i64)]
 
 
+class NnSweepArgs(C.Structure):
+    """piml_nn_sweep_args"""
+    _fields_ = [("S", i32), ("N", i32), ("M", i32), ("D", i32), ("T", i32), ("t_start", i32), ("dt", f32),
+                ("kp", i32), ("cos_p", f32), ("thr_p", f32), ("ko", i32), ("cos_o", f32), ("thr_o", f32),
+                ("obstacles", vp), ("pos_tm", vp), ("vel_tm", vp), ("acc_tm", vp), ("dest_tm", vp),
+                ("dest_idx_tm", vp), ("entry_tm", vp), ("mask_p", vp), ("dest_num", vp), ("waypoints", vp),
+                ("desired_speed", vp), ("p", vp), ("v", vp), ("a", vp), ("dest", vp), ("dest_idx", vp),
+                ("ped_f", vp), ("obs_f", vp), ("self_f", vp), ("desc", C.POINTER(NetDesc)), ("packed_tc", vp),
+                ("set_stride", i64), ("has_obs", i32), ("tau", f32), ("err_sum", vp), ("err_count", vp),
+                ("rec_p", vp), ("rec_v", vp), ("rec_a", vp), ("rec_mask", vp), ("workspace", vp),
+                ("workspace_bytes", i64)]
+
+
 class NnStepArgs(C.Structure):
     """piml_nn_step_args"""
     _fields_ = [("desc", C.POINTER(NetDesc)), ("packed_tc", vp), ("has_obs", i32), ("tau", f32),
@@ -133,6 +146,8 @@ SIGNATURES = {
     "piml_pinnsf_pack_tc_f32": (i32, [C.POINTER(NetDesc), vp, vp, vp]),
     "piml_pinnsf_forward_tc_f32": (i32, [C.POINTER(NetDesc), vp, i32, f32, vp, vp, vp, i64, i32, i32, i32, vp, vp, vp,
                                          vp]),
+    "piml_pinnsf_forward_tc_sets_f32": (i32, [C.POINTER(NetDesc), vp, i64, i32, i32, f32, vp, vp, vp, i64, i32, i32,
+                                              vp, vp]),
     "piml_pinnsf_stash_floats": (i64, [C.POINTER(NetDesc), i32, i64, i32, i32]),
     "piml_pinnsf_backward_workspace_floats": (i64, [C.POINTER(NetDesc), i32, i64, i32, i32]),
     "piml_pinnsf_forward_train_f32": (i32, [C.POINTER(NetDesc), vp, i32, f32, vp, vp, vp, i64, i32, i32, i32, vp, vp,
@@ -146,6 +161,8 @@ SIGNATURES = {
     "piml_rollout_f32": (i32, [C.POINTER(RolloutArgs), vp]),
     "piml_sfm_sweep_workspace_bytes": (i64, [C.POINTER(SfmSweepArgs)]),
     "piml_sfm_sweep_f32": (i32, [C.POINTER(SfmSweepArgs), vp]),
+    "piml_nn_sweep_workspace_bytes": (i64, [C.POINTER(NnSweepArgs)]),
+    "piml_nn_sweep_f32": (i32, [C.POINTER(NnSweepArgs), vp]),
     "piml_nn_step_supported": (i32, [C.POINTER(NetDesc)]),
     "piml_nn_step_f32": (i32, [C.POINTER(NnStepArgs), vp]),
     "piml_nn_step_shard_f32": (i32, [C.POINTER(NnStepArgs), i64, i64, i32, vp, vp, vp, vp]),

@@ -846,3 +846,56 @@ extern "C" int piml_pinnsf_forward_tc_f32(const piml_net_desc *desc, const float
     count_launch();
     return check_launch("pinnsf_tc_finish_kernel");
 }
+
+namespace piml {
+// S networks of one description, set s on rows [s N, (s+1) N): the 16-bit kernel in dense mode with one (set, branch)
+// per CTA, then the finish kernel on all S N rows.  sums: S N 4 floats of scratch.
+int tc16_forward_sets(const piml_net_desc *desc, const float *packed_tc, int64_t set_stride, int S, int has_obs,
+                      float tau, const float *ped, const float *obs, const float *self, int64_t N, int kp, int ko,
+                      float *sums, float *acc, cudaStream_t st) {
+    Tc16Plan P16;
+    if (tc16_plan_for(desc, &P16))
+        return fail(PIML_ERR_UNSUPPORTED, "piml_pinnsf_forward_tc_sets_f32: the 16-bit tensor-core path does not take "
+                    "this network (per-slot decoders with hidden widths 32 / 64 / 128 only)");
+    PIML_REQUIRE(set_stride >= piml_pinnsf_packed_tc_floats(desc) && set_stride % 4 == 0,
+                 "piml_pinnsf_forward_tc_sets_f32: set_stride %lld must be a multiple of 4 and >= %lld "
+                 "(piml_pinnsf_packed_tc_floats)", static_cast<long long>(set_stride),
+                 static_cast<long long>(piml_pinnsf_packed_tc_floats(desc)));
+    PIML_REQUIRE(aligned16(packed_tc), "piml_pinnsf_forward_tc_sets_f32: packed_tc must be 16-byte aligned");
+    if (!has_obs || ko == 0) { has_obs = 0; ko = 0; }
+    PIML_REQUIRE(!has_obs || obs, "piml_pinnsf_forward_tc_sets_f32: has_obs set but obs is null");
+    const int64_t R = static_cast<int64_t>(S) * N;
+    if (R == 0) return PIML_OK;
+    Tc16Args b = {};
+    b.params = packed_tc; b.ped = ped; b.obs = obs; b.R = N; b.kp = kp; b.ko = ko;
+    b.ag_ped = 128 / kp; b.ag_obs = ko ? 128 / ko : 1;
+    b.n_ped_tiles = (N + b.ag_ped - 1) / b.ag_ped;
+    b.n_obs_tiles = has_obs ? (N + b.ag_obs - 1) / b.ag_obs : 0;
+    b.sums = sums; b.has_obs = has_obs; b.set_stride = set_stride;
+    int rc = tc16_launch_sets(P16, b, S, st);
+    if (rc) return rc;
+    const int threads = 256;
+    pinnsf_tc_finish_kernel<<<static_cast<unsigned>((2 * R + threads - 1) / threads), threads, 0, st>>>(
+        sums, self, nullptr, R, has_obs, tau, acc);
+    count_launch();
+    return check_launch("pinnsf_tc_finish_kernel");
+}
+}  // namespace piml
+
+extern "C" int piml_pinnsf_forward_tc_sets_f32(const piml_net_desc *desc, const float *packed_tc, int64_t set_stride,
+                                               int S, int has_obs, float tau, const float *ped, const float *obs,
+                                               const float *self, int64_t N, int kp, int ko, float *acc,
+                                               void *stream) {
+    PIML_REQUIRE(desc && packed_tc && ped && self && acc, "piml_pinnsf_forward_tc_sets_f32: null pointer");
+    PIML_REQUIRE(S >= 0 && N >= 0 && kp >= 1 && ko >= 0 && kp <= 128 && ko <= 128 &&
+                     N * (kp > ko ? kp : ko) < (1LL << 31),
+                 "piml_pinnsf_forward_tc_sets_f32: bad dimensions S=%d N=%lld kp=%d ko=%d", S,
+                 static_cast<long long>(N), kp, ko);
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    float *sums = nullptr;
+    if (static_cast<int64_t>(S) * N > 0) {
+        const int rc = tc_scratch_get(st, static_cast<int64_t>(S) * N * 4, &sums);
+        if (rc) return rc;
+    }
+    return tc16_forward_sets(desc, packed_tc, set_stride, S, has_obs, tau, ped, obs, self, N, kp, ko, sums, acc, st);
+}

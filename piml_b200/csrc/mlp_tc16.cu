@@ -17,6 +17,12 @@
 // both are undone in the next epilogue (y = D * 2^-s * 2^-e_l + b).  The split drops lo*lo = O(2^-22): measured
 // 6.8e-7 of fp64 for a 128 x 128 x 128 layer (3xTF32: 1.0e-6).
 //
+// Per set (SETS, piml_pinnsf_forward_tc_sets_f32): S networks of one description, each with its own rows; CTA
+// blockIdx.x serves set blockIdx.x / ctas_per_set and splits its ctas_per_set CTAs between the set's two branches as
+// the single-network kernel splits the grid, so every CTA still keeps ONE branch's weights resident.  More sets than
+// SMs run as several waves.  A row's result depends only on the row and its set's weights (per-row scaling, in-tile
+// slot sums), so set s equals piml_pinnsf_forward_tc_f32 on set s alone, bit for bit.
+//
 // Per CTA (persistent, one per SM, ONE branch per CTA, 576 threads):
 //   warp 0   : loads the branch's weight images (hi + lo per layer, UMMA K-major core matrices written by
 //              piml_pinnsf_pack_tc_f32) with cp.async.bulk, one mbarrier per layer, once;
@@ -49,7 +55,7 @@ __device__ __forceinline__ void row_scale(float mx, float &s, float &inv_s) {
     inv_s = __uint_as_float(static_cast<uint32_t>(E - 14) << 23);
 }
 
-template <bool COMPACT>
+template <bool COMPACT, bool SETS>
 __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __grid_constant__ Tc16Plan P,
                                                                      const __grid_constant__ Tc16Args a) {
     extern __shared__ __align__(128) unsigned char t16_smem[];
@@ -72,7 +78,10 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
     const int cnt_ped = COMPACT ? a.counts[0] + 1 : 0, cnt_obs = (COMPACT && a.has_obs) ? a.counts[1] + 1 : 0;
     const int nP = COMPACT ? (cnt_ped + 127) / 128 : static_cast<int>(a.n_ped_tiles);
     const int nO = COMPACT ? (cnt_obs + 127) / 128 : static_cast<int>(a.n_obs_tiles);
-    const int G = gridDim.x;
+    // SETS: this CTA's set and its place among the set's CTAs (a.R, tile counts and the split are per set)
+    const int G = SETS ? a.ctas_per_set : static_cast<int>(gridDim.x);
+    const int set = SETS ? static_cast<int>(blockIdx.x) / a.ctas_per_set : 0;
+    const int cta = SETS ? static_cast<int>(blockIdx.x) - set * a.ctas_per_set : static_cast<int>(blockIdx.x);
     // CTAs per branch (one branch per CTA: its weights stay resident).  The kernel ends with its slowest CTA, so the
     // split minimises the larger per-CTA tile count: start from the proportional share and give the obstacle branch
     // CTAs until it is no longer the straggler (rounding to nearest left 43 obstacle tiles on ONE CTA next to 32 per
@@ -87,13 +96,13 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
         }
     }
     const int gP = G - gO;
-    const int br = static_cast<int>(blockIdx.x) < gP ? 0 : 1;
-    const int first = br == 0 ? static_cast<int>(blockIdx.x) : static_cast<int>(blockIdx.x) - gP;
+    const int br = cta < gP ? 0 : 1;
+    const int first = br == 0 ? cta : cta - gP;
     const int stride = br == 0 ? gP : gO;
     const int ntiles_br = br == 0 ? nP : nO;
     const int my_tiles = first < ntiles_br ? (ntiles_br - first + stride - 1) / stride : 0;
 
-    const float *branch = a.params + P.base + static_cast<int64_t>(br) * P.branch_floats;
+    const float *branch = a.params + (SETS ? set * a.set_stride : 0) + P.base + static_cast<int64_t>(br) * P.branch_floats;
     for (int e = tid; e < P.bias_floats; e += T16_THREADS) biasb[e] = branch[P.w_bytes / 4 + e];
     tc::fence_before_sync();
     __syncthreads();
@@ -171,7 +180,7 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
         const int AG = br == 0 ? a.ag_ped : a.ag_obs;
         const int cnt = br == 0 ? cnt_ped : cnt_obs;
         const int *list = br == 0 ? a.list_ped : a.list_obs;
-        const float *feat = br == 0 ? a.ped : a.obs;
+        const float *feat = (br == 0 ? a.ped : a.obs) + (SETS ? static_cast<int64_t>(set) * a.R * k * 6 : 0);
         float *smax = small + slot * 1024;                         // [2 parities][2 halves][128] row maxima
         float *sm2 = smax + 512;                                   // [2 halves][128][2] predictor partials / slot sums
         uint32_t dph = 0;
@@ -350,7 +359,7 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                     dst[0] = m0; dst[1] = m1;
                 }
             } else {
-                float *msgs_out = br == 0 ? a.ped_msgs : a.obs_msgs;
+                float *msgs_out = SETS ? nullptr : (br == 0 ? a.ped_msgs : a.obs_msgs);   // SETS: no messages
                 if (half == 0 && msgs_out && m < nrows) { msgs_out[(row0 + m) * 2] = m0; msgs_out[(row0 + m) * 2 + 1] = m1; }
                 slot_barrier(slot);                                // every partial read before the totals overwrite
                 if (half == 0) { sm2[m * 2] = m0; sm2[m * 2 + 1] = m1; }
@@ -360,7 +369,7 @@ __global__ void __launch_bounds__(T16_THREADS, 1) pinnsf_tc16_kernel(const __gri
                         const int ag = e >> 1, c = e & 1;          // k = 1: 128 agents per tile, two sums per thread
                         float sum = 0.f;
                         for (int jj = 0; jj < k; ++jj) sum += sm2[(ag * k + jj) * 2 + c];
-                        a.sums[(agent0 + ag) * 4 + br * 2 + c] = sum;
+                        a.sums[((SETS ? static_cast<int64_t>(set) * a.R : 0) + agent0 + ag) * 4 + br * 2 + c] = sum;
                     }
                 slot_barrier(slot);                                // sm2 is free for this slot's next tile
             }
@@ -496,9 +505,24 @@ int tc16_launch(const Tc16Plan &P, const Tc16Args &a, int64_t tiles_bound, cudaS
     const size_t smem = tc16_smem_bytes(P);
     const int grid = static_cast<int>(tiles_bound < sm_count() ? tiles_bound : sm_count());
     // (compact and dense are separate instantiations: at the epilogue's 96-register ceiling every dead path costs spills)
-    const auto kernel = a.compact ? pinnsf_tc16_kernel<true> : pinnsf_tc16_kernel<false>;
+    const auto kernel = a.compact ? pinnsf_tc16_kernel<true, false> : pinnsf_tc16_kernel<false, false>;
     PIML_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
     kernel<<<grid, T16_THREADS, smem, st>>>(P, a);
+    count_launch();
+    return check_launch("pinnsf_tc16_kernel");
+}
+
+// S sets of a.R rows each, dense mode: a.ctas_per_set CTAs per set (at least one per branch with tiles, at most one
+// per tile), as many as fill the SMs; more sets than SMs make several waves of a.ctas_per_set CTAs per set.
+int tc16_launch_sets(const Tc16Plan &P, Tc16Args a, int S, cudaStream_t st) {
+    const int64_t tiles = a.n_ped_tiles + a.n_obs_tiles;
+    const int64_t fill = sm_count() / S, least = a.n_obs_tiles > 0 ? 2 : 1;
+    a.ctas_per_set = static_cast<int>(fill < least ? least : (fill > tiles ? tiles : fill));
+    const size_t smem = tc16_smem_bytes(P);
+    PIML_CUDA(cudaFuncSetAttribute(pinnsf_tc16_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   static_cast<int>(smem)));
+    pinnsf_tc16_kernel<false, true><<<static_cast<unsigned>(static_cast<int64_t>(S) * a.ctas_per_set), T16_THREADS,
+                                      smem, st>>>(P, a);
     count_launch();
     return check_launch("pinnsf_tc16_kernel");
 }

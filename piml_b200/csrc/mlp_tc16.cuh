@@ -32,12 +32,15 @@ struct Tc16Args {
     int compact, has_obs;
     const int *list_ped, *list_obs; const int *counts;   // lists NULL: ped / obs hold the compact rows themselves (nn_step.cu)
     float *cmsg_ped, *cmsg_obs; float *f0;
+    int64_t set_stride; int ctas_per_set;                 // per-set launch only: floats between the sets' vectors
 };
 
 int tc16_build_plan(const piml_net_desc *d, int64_t base_floats, Tc16Plan *P);   // 0 = the network fits this path
 size_t tc16_smem_bytes(const Tc16Plan &P);
 int tc16_pack(const Tc16Plan &P, const Tc16Src &S, const float *params_torch, float *packed, cudaStream_t st);
 int tc16_launch(const Tc16Plan &P, const Tc16Args &a, int64_t tiles_bound, cudaStream_t st);
+// one network per set: rows [s a.R, (s+1) a.R) use the vector at a.params + s a.set_stride; dense mode, no messages
+int tc16_launch_sets(const Tc16Plan &P, Tc16Args a, int S, cudaStream_t st);
 int tc16_plan_for(const piml_net_desc *d, Tc16Plan *P);    // mlp_tc.cu: plan inside a piml_pinnsf_pack_tc_f32 vector; 0 = ok
 
 }  // namespace piml

@@ -134,17 +134,22 @@ def pack_device(sd, spec, device=None):
     return out
 
 
-def pack_device_tc(sd, spec, device=None):
+def pack_device_tc(sd, spec, device=None, out=None):
     """Parameter layout of the tensor-core forward (piml_pinnsf_pack_tc_f32): per Linear the tf32 hi / lo images of the
     weight as UMMA K-major core matrices, fp32 biases and predictor.  Returns None when the network cannot run on the
-    tensor-core path (widths not multiples of 32, single-block processor); callers then use the FP32-pipe kernel."""
+    tensor-core path (widths not multiples of 32, single-block processor); callers then use the FP32-pipe kernel.
+    out: a contiguous, 16-byte aligned float32 CUDA tensor of at least piml_pinnsf_packed_tc_floats floats to write
+    the vector into (e.g. one row of a sweep's stacked networks); default: a new tensor."""
     dev = device if device is not None else L.cuda_device()
     desc = spec.desc()
     n = int(L.load().piml_pinnsf_packed_tc_floats(L.C.byref(desc)))
     if n < 0:
         return None
     src = pack_state_dict(sd, spec).to(dev)
-    out = torch.empty(n, dtype=torch.float32, device=dev)
+    if out is None:
+        out = torch.empty(n, dtype=torch.float32, device=dev)
+    elif out.dtype != torch.float32 or not out.is_contiguous() or out.numel() < n or out.device != torch.device(dev):
+        raise ValueError(f"pack_device_tc: out must be a contiguous float32 tensor of >= {n} floats on {dev}")
     L.check(L.load().piml_pinnsf_pack_tc_f32(L.C.byref(desc), L.ptr(src), L.ptr(out), L.stream_ptr(dev)),
             "piml_pinnsf_pack_tc_f32")
     return out

@@ -281,6 +281,63 @@ def _write_back_side_effects(data, t_start, v_res, final):
     sf[t_start, :, 2:4] = hist
 
 
+def _sweep_spec(models):
+    """The one NetSpec every model of a sweep shares (None for an empty list).  Touches neither library nor device."""
+    if isinstance(models, torch.nn.Module) or not isinstance(models, (list, tuple)):
+        raise ValueError("sweep_networks: models must be a list or tuple of PINNSF modules")
+    mods = [m.module if isinstance(m, torch.nn.DataParallel) else m for m in models]
+    specs = [M.spec_from_module(m) for m in mods]
+    if not specs:
+        return None, mods
+    s0, c0 = specs[0], M._REF_CLASS_TO_MODEL[type(mods[0]).__name__]
+    for i, (m, s) in enumerate(zip(mods, specs)):
+        if M._REF_CLASS_TO_MODEL[type(m).__name__] != c0 or (s.enc_dims, s.proc_mode, s.dec_dims, s.coll_dims,
+                                                              s.kind, s.has_obs) != \
+                (s0.enc_dims, s0.proc_mode, s0.dec_dims, s0.coll_dims, s0.kind, s0.has_obs):
+            raise ValueError(f"sweep_networks: model {i} differs from model 0 in class or widths; one sweep takes "
+                             "one architecture")
+        if s.tau != s0.tau:
+            raise ValueError(f"sweep_networks: model {i} has tau {s.tau}, model 0 has {s0.tau}; one sweep takes one tau")
+    return s0, mods
+
+
+def sweep_networks(data_or_scene, models, args, t_start=0, num_frames=None, record=False):
+    """Roll ONE clip out from t_start under S trained interaction networks in one library call (piml_nn_sweep_f32),
+    and score each network: checkpoint selection, seed ensembles, grid-search evaluation.
+
+    data_or_scene: a reference `TimeIndexedPedData` or the single-scene dict, exactly as `sfm.sweep` takes it.
+    models: a list of S reference PINNSF modules (or piml_b200.models mirrors) of one class, the same widths and the
+        same tau; networks the 16-bit tensor-core forward does not take (pinnsf_m / pinnsf, widths other than 32 / 64 /
+        128) raise NotImplementedError before any device work.
+    Network s rolls out exactly as `rollout_scenes(spec, None, args, scene, t_start, T, packed_tc=its vector)` on the
+    clip alone.  Returns (err_sum (S,) float64, err_count (S,) int64) with sfm.sweep's definition, so networks and
+    social-force constant sets rank on one scale; with record=True also (p_res, v_res, a_res (S,T,N,2),
+    mask_p_new (S,T,N)).  Device memory: O(S N) plus the S packed networks (and 28 bytes per set, frame and slot with
+    record=True)."""
+    from .sfm import _clip_scene, _clip_shapes, _run_sweep, _stage_clip
+    spec, mods = _sweep_spec(models)
+    if spec is not None and not L.load().piml_nn_step_supported(L.C.byref(spec.desc())):
+        raise NotImplementedError("sweep_networks runs the 16-bit tensor-core forward: per-slot-decoder networks "
+                                  "(pinnsf_bm, pinnsf_bottleneck) with hidden widths 32 / 64 / 128")
+    scene, dt, num_frames = _clip_scene(data_or_scene, args, t_start, num_frames, "sweep_networks")
+    T, N, Mo = _clip_shapes(scene, args, dt, t_start, num_frames, "sweep_networks")
+    if spec is not None and spec.has_obs and not Mo:
+        raise ValueError("the network has an obstacle branch but the scene has no obstacles")
+    S = len(mods)
+    dev, sc = _stage_clip(scene)
+    r = L.NnSweepArgs()
+    if S:
+        desc = spec.desc()
+        n = int(L.load().piml_pinnsf_packed_tc_floats(L.C.byref(desc)))
+        stride = -(-n // 32) * 32                  # 128-byte rows: each vector as aligned as a lone allocation
+        packed = torch.empty(S, stride, dtype=torch.float32, device=dev)
+        for s, m in enumerate(mods):
+            M.pack_device_tc(m.state_dict(), spec, dev, out=packed[s])
+        r.desc, r.packed_tc, r.set_stride = L.C.pointer(desc), L.ptr(packed), stride
+        r.has_obs, r.tau = (1 if (spec.has_obs and Mo) else 0), spec.tau
+    return _run_sweep(r, dev, sc, S, T, N, Mo, t_start, dt, args, record, "piml_nn_sweep")
+
+
 class _with_dt(object):
     """args view whose time_unit is the clip's (simulators.py uses data.time_unit, not args.time_unit)."""
 
