@@ -22,7 +22,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 
-#include <cub/device/device_radix_sort.cuh>
+#include <cooperative_groups.h>
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 #include <cub/iterator/counting_input_iterator.cuh>
@@ -32,6 +32,8 @@
 #include "common.cuh"
 
 namespace piml {
+
+namespace cg = cooperative_groups;
 
 constexpr int ML_THREADS = 128;
 constexpr int ML_TILE = 512;          // columns per shared-memory stage: 4 KB positions + 4 KB velocities
@@ -767,9 +769,10 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
 // pair has arg < -127: ex2 flushes to +0, every fma(w, r, S) returns S unchanged and every fixed-point column share is
 // 0.  Skipping those pairs changes nothing but the fp32 summation order.
 //
-// Per call: (1) a 32-bit Hilbert key of each agent's 4 m cell, sorted stably (cub::DeviceRadixSort, key + agent
-// index), so that the agents of a 512-block live close together; (2) records in sorted order plus an axis-aligned box
-// per 512-agent block, per 128-agent row tile and per 32-agent column tile; (3) the work list: every (row tile R of
+// Per call: (1+2) one cooperative kernel (mlapm_cull_order_kernel): an 18-bit Hilbert key of each agent's cell on a
+// 512 x 512 grid fitted to the crowd's box, sorted stably (two 9-bit LSD passes, key + agent index), so that the agents
+// of a 512-block live close together, then records in sorted order plus an axis-aligned box per 512-agent block, per
+// 128-agent row tile and per 32-agent column tile; (3) the work list: every (row tile R of
 // block I, column block J = I + d mod T) item of the circulant schedule whose boxes are within r_cut, compacted in
 // order (cub::DeviceSelect), the mask of its column tiles within r_cut, and the exclusive scan of the masks' popcounts
 // (cub::DeviceScan): the live (row tile, column tile) units; (4) a persistent pair kernel over the units; (5) the
@@ -779,59 +782,52 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
 // tiles of the row tiles r' > r of the own block in both directions and the row tile's own 4 column tiles in the row
 // direction only (every ordered pair of the row tile appears there); r' < r belongs to row tile r'.
 // =====================================================================================================================
-constexpr float MC_CELL = 4.0f;                   // metres per cell of the sort key
 constexpr int MC_RT = 128;                        // rows per row tile
-constexpr int MC_CT = 32;                         // columns per column tile: one warp of the prep kernel, 1 KB
+constexpr int MC_CT = 32;                         // columns per column tile: one warp of the order kernel, 1 KB
 constexpr int MC_RPB = MS_BLOCK / MC_RT;          // row tiles per block
 constexpr int MC_CPB = MS_BLOCK / MC_CT;          // column tiles per block: one bit each in a uint16_t mask
 constexpr int MC_THREADS = 32;                    // pair kernel: one warp per row tile, 4 rows per thread
 constexpr unsigned MC_NEAR_ALL = 1u, MC_EMPTY = 2u;   // box flags: holds a NaN / inf, holds no agent
 static_assert(MC_CPB <= 16 && MC_RT % (2 * MC_THREADS) == 0, "bad tile shape");
+constexpr int MC_KEY_BITS = 9;                    // the sort key's grid: 2^9 x 2^9 cells, one 9-bit digit per pass
+constexpr int MC_BINS = (1 << MC_KEY_BITS) + 1;   // bins of a digit pass: the 512 digits, then the non-finite agents
+constexpr uint32_t MC_NONFINITE = 0xFFFFFFFFu;    // key of an agent with a NaN / inf coordinate: sorts last
+constexpr int MO_WARPS = MS_BLOCK / 32;           // order kernel: MS_BLOCK threads, one agent each per tile
 
-// Hilbert index of cell (x, y) on the 2^16 x 2^16 grid.
-__device__ __forceinline__ uint32_t hilbert16(uint32_t x, uint32_t y) {
+// Hilbert index of cell (x, y) on the 2^9 x 2^9 grid: 18 bits.
+__device__ __forceinline__ uint32_t hilbert9(uint32_t x, uint32_t y) {
     uint32_t d = 0;
-    for (uint32_t s = 1u << 15; s > 0; s >>= 1) {
+    for (uint32_t s = 1u << (MC_KEY_BITS - 1); s > 0; s >>= 1) {
         const uint32_t rx = (x & s) ? 1u : 0u, ry = (y & s) ? 1u : 0u;
         d += s * s * ((3u * rx) ^ ry);
         if (ry == 0) {
-            if (rx == 1) { x = 0xFFFFu - x; y = 0xFFFFu - y; }
+            if (rx == 1) { x = (1u << MC_KEY_BITS) - 1u - x; y = (1u << MC_KEY_BITS) - 1u - y; }
             const uint32_t t = x; x = y; y = t;
         }
     }
     return d;
 }
 
-// key[n] = Hilbert index of floor(p_n / MC_CELL) (cell coordinates wrap modulo 2^16: only locality is lost), agent
-// index as the value; a non-finite position sorts last.
-__global__ void mlapm_cull_keys_kernel(const float2 *__restrict__ pos, int N, uint32_t *__restrict__ key,
-                                       int *__restrict__ val) {
-    const int n = blockIdx.x * blockDim.x + threadIdx.x;
-    if (n >= N) return;
-    const float2 p = pos[n];
-    uint32_t k = 0xFFFFFFFFu;
-    if (isfinite(p.x) && isfinite(p.y)) {
-        const uint32_t cx = static_cast<uint32_t>(__float2int_rd(p.x * (1.0f / MC_CELL))) & 0xFFFFu;
-        const uint32_t cy = static_cast<uint32_t>(__float2int_rd(p.y * (1.0f / MC_CELL))) & 0xFFFFu;
-        k = hilbert16(cx, cy);
-    }
-    key[n] = k;
-    val[n] = n;
+// Bin of a key in digit pass `pass` (0: low 9 bits, 1: high 9 bits).
+__device__ __forceinline__ int mo_digit(uint32_t key, int pass) {
+    return key == MC_NONFINITE ? MC_BINS - 1
+                               : static_cast<int>((key >> (MC_KEY_BITS * pass)) & ((1u << MC_KEY_BITS) - 1u));
 }
 
-// One CTA of MS_BLOCK threads per block of the sorted crowd: slot j holds the agent perm[j] (ms_prep_slot; j >= N:
-// padding), slot[agent] = j, and the boxes {min x, min y, max x, max y} of its MC_CPB column tiles (one warp each), its
-// MC_RPB row tiles and the block.  Agents with a non-finite position or velocity do not enter the min / max (no
-// fminf / fmaxf on NaN); they flag their tiles and block MC_NEAR_ALL instead, which keeps every unit that touches them.
-__global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
-    const float2 *__restrict__ pos, const float2 *__restrict__ vel, const float2 *__restrict__ dest,
-    const int *__restrict__ perm, int N, float4 *__restrict__ rec, int *__restrict__ slot,
+// Slots [blk MS_BLOCK, (blk + 1) MS_BLOCK) of the sorted crowd, called by all MS_BLOCK threads of a CTA: slot j holds
+// the agent perm[j] (ms_prep_slot; j >= N: padding), slot[agent] = j, and the boxes {min x, min y, max x, max y} of the
+// block's MC_CPB column tiles (one warp each), its MC_RPB row tiles and the block.  Agents with a non-finite position
+// or velocity do not enter the min / max (no fminf / fmaxf on NaN); they flag their tiles and block MC_NEAR_ALL
+// instead, which keeps every unit that touches them.
+__device__ __forceinline__ void mc_prep_block(
+    int blk, const float2 *__restrict__ pos, const float2 *__restrict__ vel, const float2 *__restrict__ dest,
+    const int *perm, int N, float4 *__restrict__ rec, int *__restrict__ slot,
     ulonglong2 *__restrict__ acc, unsigned *__restrict__ bad, float4 *__restrict__ cbox, unsigned *__restrict__ cflag,
     float4 *__restrict__ rbox, unsigned *__restrict__ rflag, float4 *__restrict__ bbox, unsigned *__restrict__ bflag) {
     static_assert(MC_CT == 32, "a column tile is one warp");
     __shared__ float4 wbox[MS_BLOCK / 32];
     __shared__ unsigned wflag[MS_BLOCK / 32];
-    const int j = blockIdx.x * MS_BLOCK + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int j = blk * MS_BLOCK + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const bool agent = j < N;
     const int n = agent ? perm[j] : 0;
     if (agent) slot[n] = j;
@@ -858,8 +854,8 @@ __global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
     }
     if (lane == 0) {
         wbox[warp] = b; wflag[warp] = flag;
-        cbox[blockIdx.x * MC_CPB + warp] = b;
-        cflag[blockIdx.x * MC_CPB + warp] = flag;
+        cbox[blk * MC_CPB + warp] = b;
+        cflag[blk * MC_CPB + warp] = flag;
     }
     __syncthreads();
     if (threadIdx.x < MC_RPB + 1) {
@@ -874,13 +870,231 @@ __global__ void __launch_bounds__(MS_BLOCK) mlapm_prep_cull_kernel(
             f = comb(f, wflag[w]);
         }
         if (threadIdx.x < MC_RPB) {
-            rbox[blockIdx.x * MC_RPB + threadIdx.x] = u;
-            rflag[blockIdx.x * MC_RPB + threadIdx.x] = f;
+            rbox[blk * MC_RPB + threadIdx.x] = u;
+            rflag[blk * MC_RPB + threadIdx.x] = f;
         } else {
-            bbox[blockIdx.x] = u;
-            bflag[blockIdx.x] = f;
+            bbox[blk] = u;
+            bflag[blk] = f;
         }
     }
+    __syncthreads();                                               // wbox / wflag are reused by the next block
+}
+
+// Buffers of mlapm_cull_order_kernel (cull_layout) and the inputs it orders.  A tile is MS_BLOCK consecutive entries
+// of the array a phase reads; tiles and 512-agent blocks coincide, T of each.  What one phase writes and a later one
+// reads is never accessed through a const __restrict__ pointer: such loads may take the non-coherent path.
+struct CullOrderArgs {
+    const float2 *pos, *vel, *dest;
+    int N, T;
+    float4 *cta_box;                 // [gridDim]: box of the finite positions of each CTA's tiles
+    uint32_t *key0;                  // [N] keys in agent order
+    uint32_t *key1; int *val1;       // [N] keys and agents after the low-digit pass
+    int *perm;                       // [N] agents after the high-digit pass: slot j holds agent perm[j]
+    int *rank;                       // [N] rank of an entry among the equal digits before it in its CTA's tiles
+    int *cnt;                        // [MC_BINS][gridDim] bin counts per CTA, then their exclusive sum over the CTAs
+    int *dtotal;                     // [MC_BINS] entries per bin
+    float4 *rec; int *slot; ulonglong2 *acc; unsigned *bad;
+    float4 *cbox, *rbox, *bbox; unsigned *cflag, *rflag, *bflag;
+};
+
+struct MoSmem {
+    int wcnt[MO_WARPS][MC_BINS];     // per warp: digit counts, then the exclusive sum over the CTA's entries before it
+    int run[MC_BINS];                // count: the CTA's entries per bin so far; scatter: each bin's first destination
+    int wsum[MO_WARPS];
+    float4 box[MO_WARPS];
+};
+static_assert(MC_BINS == MS_BLOCK + 1, "mo_bases: one bin per thread and the non-finite bin");
+
+// The CTA's tiles [t0, t1): a contiguous run, so that the order of its entries is the order of the array.  gridDim <= T,
+// so every CTA has at least one.
+__device__ __forceinline__ void mo_tiles(int T, int &t0, int &t1) {
+    t0 = static_cast<int>(static_cast<int64_t>(T) * blockIdx.x / gridDim.x);
+    t1 = static_cast<int>(static_cast<int64_t>(T) * (blockIdx.x + 1) / gridDim.x);
+}
+
+// Rank of this thread's entry of bin dig (-1: no entry) among the entries of the same bin before it in the CTA's tiles
+// (sm.run: those of the earlier tiles, advanced by this tile's counts).  All threads call it.
+__device__ __forceinline__ int mo_rank(MoSmem &sm, int dig) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int i = tid; i < MO_WARPS * MC_BINS; i += MS_BLOCK) (&sm.wcnt[0][0])[i] = 0;
+    __syncthreads();
+    const unsigned peers = __match_any_sync(0xffffffffu, dig);
+    const int below = __popc(peers & ((1u << lane) - 1u));
+    if (dig >= 0 && below == 0) sm.wcnt[warp][dig] = __popc(peers);
+    __syncthreads();
+    for (int d = tid; d < MC_BINS; d += MS_BLOCK) {
+        int s = sm.run[d];
+#pragma unroll
+        for (int w = 0; w < MO_WARPS; ++w) {
+            const int c = sm.wcnt[w][d];
+            sm.wcnt[w][d] = s;
+            s += c;
+        }
+        sm.run[d] = s;
+    }
+    __syncthreads();
+    const int r = dig >= 0 ? sm.wcnt[warp][dig] + below : 0;
+    __syncthreads();                                               // wcnt is cleared by the next tile
+    return r;
+}
+
+// Count pass over the CTA's tiles: rank[i] of every entry (digit(i): its bin), and the CTA's bin counts into cnt.
+template <class Dig>
+__device__ __forceinline__ void mo_count(MoSmem &sm, const CullOrderArgs &a, int t0, int t1, Dig digit) {
+    for (int d = threadIdx.x; d < MC_BINS; d += MS_BLOCK) sm.run[d] = 0;   // read after mo_rank's first barrier
+    for (int tile = t0; tile < t1; ++tile) {
+        const int i = tile * MS_BLOCK + threadIdx.x;
+        const int r = mo_rank(sm, i < a.N ? digit(i) : -1);
+        if (i < a.N) a.rank[i] = r;
+    }
+    for (int d = threadIdx.x; d < MC_BINS; d += MS_BLOCK) a.cnt[static_cast<int64_t>(d) * gridDim.x + blockIdx.x] = sm.run[d];
+}
+
+// cnt[d][.] -> its exclusive sum over the CTAs, dtotal[d] = the sum; one warp per bin, each lane a run of CTAs (a
+// contiguous row: the second walk over it hits L1).
+__device__ __forceinline__ void mo_scan_ctas(const CullOrderArgs &a) {
+    const int lane = threadIdx.x & 31, G = gridDim.x;
+    const int gw = blockIdx.x * MO_WARPS + (threadIdx.x >> 5), nw = G * MO_WARPS;
+    const int per = (G + 31) / 32, c0 = min(lane * per, G), c1 = min(c0 + per, G);
+    for (int d = gw; d < MC_BINS; d += nw) {
+        int *row = a.cnt + static_cast<int64_t>(d) * G;
+        int s = 0;
+#pragma unroll 4
+        for (int c = c0; c < c1; ++c) s += row[c];
+        int incl = s;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int u = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += u;
+        }
+        int off = incl - s;
+        for (int c = c0; c < c1; ++c) {
+            const int v = row[c];
+            row[c] = off;
+            off += v;
+        }
+        if (lane == 31) a.dtotal[d] = incl;
+    }
+}
+
+// sm.run[d] = first destination of this CTA's entries of bin d: every entry of the bins before d, and those of bin d
+// in the CTAs before this one.  One block-wide scan of the bin totals.
+__device__ __forceinline__ void mo_bases(MoSmem &sm, const CullOrderArgs &a) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int v = a.dtotal[tid];
+    int incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int u = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += u;
+    }
+    if (lane == 31) sm.wsum[warp] = incl;
+    __syncthreads();
+    int excl = incl - v;
+    for (int w = 0; w < warp; ++w) excl += sm.wsum[w];
+    const int *own = a.cnt + blockIdx.x;
+    sm.run[tid] = excl + own[static_cast<int64_t>(tid) * gridDim.x];
+    if (tid == MS_BLOCK - 1) sm.run[MC_BINS - 1] = excl + v + own[static_cast<int64_t>(MC_BINS - 1) * gridDim.x];
+    __syncthreads();
+}
+
+// The spatial order of the culled evaluation and everything laid out in it, in one cooperative launch (a co-resident
+// grid; each CTA owns a contiguous run of tiles; grid-wide barriers between the phases):
+//   (a) the box of the finite positions (per CTA, then every CTA reduces the CTAs' boxes: no atomics, no state);
+//   (b) key of each agent = Hilbert index of its cell on the 2^9 x 2^9 grid of square cells fitted to the box's larger
+//       side, bin counts per CTA and ranks of the low digit;
+//   (c) two stable LSD scatter passes (low digit, then high digit, the first followed by the counts of the second):
+//       the CTAs' counts scanned per bin, then each entry to its bin's first destination in its CTA + its rank, so
+//       perm is a pure function of the positions;
+//   (d) mc_prep_block over the sorted order.
+// The box is computed in halves (x/2 - min/2 <= max/2 - min/2), so coordinates near +-3e38 give finite keys.
+__global__ void __launch_bounds__(MS_BLOCK) mlapm_cull_order_kernel(const __grid_constant__ CullOrderArgs a) {
+    __shared__ MoSmem sm;
+    cg::grid_group grid = cg::this_grid();
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    int t0, t1;
+    mo_tiles(a.T, t0, t1);
+    auto finite2 = [](float2 p) { return isfinite(p.x) && isfinite(p.y); };
+    auto box_reduce = [&](float4 b) {                              // over the CTA; result in sm.box[0]
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            b.x = fminf(b.x, __shfl_xor_sync(0xffffffffu, b.x, o));
+            b.y = fminf(b.y, __shfl_xor_sync(0xffffffffu, b.y, o));
+            b.z = fmaxf(b.z, __shfl_xor_sync(0xffffffffu, b.z, o));
+            b.w = fmaxf(b.w, __shfl_xor_sync(0xffffffffu, b.w, o));
+        }
+        if (lane == 0) sm.box[warp] = b;
+        __syncthreads();
+        if (tid == 0) {
+            float4 u = sm.box[0];
+            for (int w = 1; w < MO_WARPS; ++w) {
+                const float4 t = sm.box[w];
+                u.x = fminf(u.x, t.x); u.y = fminf(u.y, t.y); u.z = fmaxf(u.z, t.z); u.w = fmaxf(u.w, t.w);
+            }
+            sm.box[0] = u;
+        }
+        __syncthreads();
+        return sm.box[0];
+    };
+    const float4 none = make_float4(CUDART_INF_F, CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F);
+
+    // (a)
+    float4 b = none;
+    for (int n = t0 * MS_BLOCK + tid; n < min(t1 * MS_BLOCK, a.N); n += MS_BLOCK) {
+        const float2 p = a.pos[n];
+        if (finite2(p)) { b.x = fminf(b.x, p.x); b.y = fminf(b.y, p.y); b.z = fmaxf(b.z, p.x); b.w = fmaxf(b.w, p.y); }
+    }
+    b = box_reduce(b);
+    if (tid == 0) a.cta_box[blockIdx.x] = b;
+    grid.sync();
+    b = none;
+    for (int c = tid; c < static_cast<int>(gridDim.x); c += MS_BLOCK) {
+        const float4 t = a.cta_box[c];
+        b.x = fminf(b.x, t.x); b.y = fminf(b.y, t.y); b.z = fmaxf(b.z, t.z); b.w = fmaxf(b.w, t.w);
+    }
+    b = box_reduce(b);
+
+    // (b) half the box's larger side; cell = floor(offset / side * 2^9), clamped (offset <= side)
+    const float lx = 0.5f * b.x, ly = 0.5f * b.y;
+    const float half = fmaxf(0.5f * b.z - lx, 0.5f * b.w - ly);
+    constexpr float CELLS = static_cast<float>(1 << MC_KEY_BITS);
+    auto cell = [half](float v, float lo) {
+        const float t = half > 0.f ? __fdiv_rn(0.5f * v - lo, half) * CELLS : 0.f;
+        return static_cast<uint32_t>(fminf(t, CELLS - 1.f));
+    };
+    mo_count(sm, a, t0, t1, [&a, cell, finite2, lx, ly](int n) {
+        const float2 p = a.pos[n];
+        const uint32_t key = finite2(p) ? hilbert9(cell(p.x, lx), cell(p.y, ly)) : MC_NONFINITE;
+        a.key0[n] = key;
+        return mo_digit(key, 0);
+    });
+    grid.sync();
+
+    // (c) low digit: key0, agent order -> key1, val1
+    mo_scan_ctas(a);
+    grid.sync();
+    mo_bases(sm, a);
+    for (int i = t0 * MS_BLOCK + tid; i < min(t1 * MS_BLOCK, a.N); i += MS_BLOCK) {
+        const uint32_t key = a.key0[i];
+        const int dst = sm.run[mo_digit(key, 0)] + a.rank[i];
+        a.key1[dst] = key;
+        a.val1[dst] = i;
+    }
+    grid.sync();
+    mo_count(sm, a, t0, t1, [&a](int i) { return mo_digit(a.key1[i], 1); });
+    grid.sync();
+    // high digit: key1, val1 -> perm
+    mo_scan_ctas(a);
+    grid.sync();
+    mo_bases(sm, a);
+    for (int i = t0 * MS_BLOCK + tid; i < min(t1 * MS_BLOCK, a.N); i += MS_BLOCK)
+        a.perm[sm.run[mo_digit(a.key1[i], 1)] + a.rank[i]] = a.val1[i];
+    grid.sync();
+
+    // (d)
+    for (int blk = blockIdx.x; blk < a.T; blk += gridDim.x)
+        mc_prep_block(blk, a.pos, a.vel, a.dest, a.perm, a.N, a.rec, a.slot, a.acc, a.bad, a.cbox, a.cflag, a.rbox,
+                      a.rflag, a.bbox, a.bflag);
 }
 
 // Whether two boxes (with their flags) may hold a pair within rc.  The box gap is rounded down, so a kept-or-not
@@ -1095,9 +1309,11 @@ __global__ void mlapm_sym_colpush_kernel(const long long *__restrict__ colsum, f
     if (threadIdx.x == 0) __threadfence_system();                         // visible to the owner before the barrier
 }
 
-constexpr int FZ_LPR = 8;                        // lanes per row in the finalize kernel
+constexpr int FZ_LPR = 8;                        // lanes per row in the finalize kernel when there are split partials
 
 // force = (v0*ed - v)/tau - A*R(sum partial) ; action = v + force*dt ; optional p' = p + action*dt and arrival.
+// LPR = FZ_LPR with split partials, 1 without (the culled evaluation: nothing to spread over lanes).
+template <int LPR>
 __global__ void mlapm_finalize2_kernel(const float2 *__restrict__ pos, const float2 *__restrict__ vel,
                                        const float *__restrict__ ds, int ds_dim, const float2 *__restrict__ dest,
                                        int row0, int row1, int nsplit, const float4 *__restrict__ partial, float A,
@@ -1105,22 +1321,22 @@ __global__ void mlapm_finalize2_kernel(const float2 *__restrict__ pos, const flo
                                        float2 *__restrict__ action, float2 *__restrict__ pos_new,
                                        uint8_t *__restrict__ arrived, const __grid_constant__ PeerPush push,
                                        const __grid_constant__ SymPartials sym) {
-    // FZ_LPR lanes share a row: lane j adds the split partials j, j + FZ_LPR, ... and the lanes' sums are combined in
-    // lane order -- a fixed order (deterministic), but FZ_LPR loads in flight per row instead of one dependent chain of
+    // LPR lanes share a row: lane j adds the split partials j, j + LPR, ... and the lanes' sums are combined in
+    // lane order -- a fixed order (deterministic), but LPR loads in flight per row instead of one dependent chain of
     // up to 396 (an 8-way shard of 100k agents): the kernel was latency bound at 70 us of a 1.05 ms step.
     const int gt = blockIdx.x * blockDim.x + threadIdx.x;
-    const int rl_raw = gt / FZ_LPR, sub = gt % FZ_LPR;
+    const int rl_raw = gt / LPR, sub = gt % LPR;
     const int nrows = row1 - row0;
     const bool live = rl_raw < nrows;
     const int rl = live ? rl_raw : nrows - 1;                     // idle lanes shadow the last row (shuffles stay converged)
     const int64_t pstride = (sym.colsum || sym.inbox) ? sym.nrows_pad : nrows;
     float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int q = sub; q < nsplit; q += FZ_LPR) {
+    for (int q = sub; q < nsplit; q += LPR) {
         const float4 t = partial[static_cast<int64_t>(q) * pstride + rl];
         s.x += t.x; s.y += t.y; s.z += t.z; s.w += t.w;
     }
 #pragma unroll
-    for (int o = 1; o < FZ_LPR; o <<= 1) {                        // tree in a fixed shape: deterministic
+    for (int o = 1; o < LPR; o <<= 1) {                           // tree in a fixed shape: deterministic
         s.x += __shfl_xor_sync(0xffffffffu, s.x, o);
         s.y += __shfl_xor_sync(0xffffffffu, s.y, o);
         s.z += __shfl_xor_sync(0xffffffffu, s.z, o);
@@ -1173,12 +1389,12 @@ __global__ void mlapm_finalize2_kernel(const float2 *__restrict__ pos, const flo
     }
     if (push.world > 0) {
         // the path's one exchange, fused: the row's new state goes into EVERY rank's next-state arrays; the row's
-        // FZ_LPR lanes take one peer each, so the remote stores of a row are issued in parallel
-        const int lead = (threadIdx.x & 31) & ~(FZ_LPR - 1);
+        // LPR lanes take one peer each, so the remote stores of a row are issued in parallel
+        const int lead = (threadIdx.x & 31) & ~(LPR - 1);
         qx = __shfl_sync(0xffffffffu, qx, lead); qy = __shfl_sync(0xffffffffu, qy, lead);
         ax = __shfl_sync(0xffffffffu, ax, lead); ay = __shfl_sync(0xffffffffu, ay, lead);
         if (live)
-            for (int g = sub; g < push.world; g += FZ_LPR) {
+            for (int g = sub; g < push.world; g += LPR) {
                 push.pos[g][n] = make_float2(qx, qy);
                 push.vel[g][n] = make_float2(ax, ay);
             }
@@ -1433,22 +1649,19 @@ static int64_t cull_candidates(int64_t N) {
     const int64_t T = sym_blocks(N);
     return T * (T / 2 + 1) * MC_RPB;
 }
-// Reserved CUB scratch, computable without a device (CUB's own size query needs one).  Radix sort on DoubleBuffers
-// (onesweep): 4 passes x 256 bins of 8 B, and 256 look-back counters of 4 B per tile of >= 256 keys -- at most 4 B
-// per key.  Select, and the scan of the candidates + 1 unit counts: one 16 B tile descriptor per tile of >= 128
-// items -- at most 1 B per candidate.  64 KB for the counters, padding and alignment of all three.  The real size is checked against this at every call.
-static int64_t cull_cub_bound(int64_t N) {
-    const int64_t a = 4 * N, b = cull_candidates(N);
-    return (int64_t{1} << 16) + (a > b ? a : b);
-}
+// Reserved CUB scratch, computable without a device (CUB's own size query needs one).  Select, and the scan of the
+// candidates + 1 unit counts: one 16 B tile descriptor per tile of >= 128 items -- at most 1 B per candidate.  64 KB
+// for the counters, padding and alignment of both.  The real size is checked against this at every call.
+static int64_t cull_cub_bound(int64_t N) { return (int64_t{1} << 16) + cull_candidates(N); }
 struct CullLayout {
-    float4 *rec; long long *acc; unsigned *bad; uint32_t *key[2]; int *val[2]; int *slot;
-    float4 *cbox, *rbox, *bbox; unsigned *cflag, *rflag, *bflag; int *items, *nitems; uint16_t *masks;
+    float4 *rec; long long *acc; unsigned *bad; uint32_t *key[2]; int *val, *perm, *rank, *cnt, *dtotal, *slot;
+    float4 *cta_box, *cbox, *rbox, *bbox; unsigned *cflag, *rflag, *bflag; int *items, *nitems; uint16_t *masks;
     long long *uoff; void *temp; int64_t temp_bytes, total;
 };
-// records, accumulators (4 x int64) and flags per padded agent; keys, values (both double-buffered) and slots per
-// agent; boxes and flags per column tile, row tile and block; the work list, its masks and the scan of their
-// popcounts (14 B per candidate); CUB's scratch.  0.2 GB at N = 10^6.
+// records, accumulators (4 x int64) and flags per padded agent; the order kernel's keys (two), agents (two), ranks
+// and slots per agent, its bin counts per (bin, CTA) and totals per bin, and a box per CTA (at most one per block);
+// boxes and flags per column tile, row tile and block; the work list, its masks and the scan of their popcounts (14 B
+// per candidate); CUB's scratch.  0.2 GB at N = 10^6.
 static CullLayout cull_layout(int64_t N, void *base) {
     const int64_t T = sym_blocks(N), npad = T * MS_BLOCK;
     CullLayout l{};
@@ -1456,10 +1669,13 @@ static CullLayout cull_layout(int64_t N, void *base) {
     l.rec = static_cast<float4 *>(c.take(npad * MS_RECF * sizeof(float)));
     l.acc = static_cast<long long *>(c.take(npad * 4 * sizeof(long long)));
     l.bad = static_cast<unsigned *>(c.take(npad * sizeof(unsigned)));
-    for (int b = 0; b < 2; ++b) {
-        l.key[b] = static_cast<uint32_t *>(c.take(N * sizeof(uint32_t)));
-        l.val[b] = static_cast<int *>(c.take(N * sizeof(int)));
-    }
+    for (int b = 0; b < 2; ++b) l.key[b] = static_cast<uint32_t *>(c.take(N * sizeof(uint32_t)));
+    l.val = static_cast<int *>(c.take(N * sizeof(int)));
+    l.perm = static_cast<int *>(c.take(N * sizeof(int)));
+    l.rank = static_cast<int *>(c.take(N * sizeof(int)));
+    l.cnt = static_cast<int *>(c.take(MC_BINS * T * sizeof(int)));
+    l.dtotal = static_cast<int *>(c.take(MC_BINS * sizeof(int)));
+    l.cta_box = static_cast<float4 *>(c.take(T * sizeof(float4)));
     l.slot = static_cast<int *>(c.take(N * sizeof(int)));
     l.cbox = static_cast<float4 *>(c.take(T * MC_CPB * sizeof(float4)));
     l.rbox = static_cast<float4 *>(c.take(T * MC_RPB * sizeof(float4)));
@@ -1576,52 +1792,45 @@ static int launch_sym_pairs(int version, const float2 *p2, const float2 *v2, con
     return check_launch("mlapm_sym_kernel");
 }
 
-// Launches of one CUB radix sort of n 32-bit keys with int values on DoubleBuffers (CUB 2.x, sm_100 policy): one
-// single-tile kernel up to 256 x 19 keys, else histogram + exclusive sum + one onesweep kernel per 8-bit digit.
-static int cub_sort_launches(int64_t n, int bits) { return n <= 256 * 19 ? 1 : 2 + (bits + 7) / 8; }
-
-// Culled symmetric evaluation of the whole crowd: keys, sort, prep + boxes, work list, pair kernel.  The finalize
-// kernel follows in the caller.  No host synchronisation: the list length stays on the device.
+// Culled symmetric evaluation of the whole crowd: order + prep + boxes, work list, pair kernel.  The finalize kernel
+// follows in the caller.  No host synchronisation: the list length stays on the device.
 static int launch_sym_culled(int version, const float2 *p2, const float2 *v2, const float2 *d2, int N,
                              const MlConst &k, float rc, const CullLayout &l, float colscale, cudaStream_t st) {
     const int64_t T = sym_blocks(N), D = T / 2;
-    const int threads = 256;
-    mlapm_cull_keys_kernel<<<static_cast<unsigned>((N + threads - 1) / threads), threads, 0, st>>>(p2, N, l.key[0],
-                                                                                                     l.val[0]);
+    // co-resident grid: one CTA per resident slot, at most one per block
+    static int order_occ = 0;
+    if (order_occ == 0) {
+        int occ = 0;
+        PIML_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, mlapm_cull_order_kernel, MS_BLOCK, 0));
+        PIML_REQUIRE(occ >= 1, "piml_mlapm: mlapm_cull_order_kernel does not fit on an SM");
+        order_occ = occ;
+    }
+    int64_t ogrid = static_cast<int64_t>(order_occ) * sm_count();
+    if (ogrid > T) ogrid = T;
+    CullOrderArgs oa{p2, v2, d2, N, static_cast<int>(T), l.cta_box, l.key[0], l.key[1], l.val, l.perm, l.rank, l.cnt,
+                     l.dtotal, l.rec, l.slot, reinterpret_cast<ulonglong2 *>(l.acc), l.bad, l.cbox, l.rbox, l.bbox,
+                     l.cflag, l.rflag, l.bflag};
+    void *oargs[] = {&oa};
+    PIML_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<const void *>(&mlapm_cull_order_kernel),
+                                          dim3(static_cast<unsigned>(ogrid)), dim3(MS_BLOCK), oargs, 0, st));
     count_launch();
-    int rc_ = check_launch("mlapm_cull_keys_kernel");
-    if (rc_) return rc_;
-    cub::DoubleBuffer<uint32_t> keys(l.key[0], l.key[1]);
-    cub::DoubleBuffer<int> vals(l.val[0], l.val[1]);
-    size_t need = 0;
-    PIML_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, need, keys, vals, N, 0, 32, st));
-    PIML_REQUIRE(static_cast<int64_t>(need) <= l.temp_bytes,
-                 "piml_mlapm: CUB radix sort needs %lld bytes of scratch, %lld reserved", static_cast<long long>(need),
-                 static_cast<long long>(l.temp_bytes));
-    size_t temp_bytes = static_cast<size_t>(l.temp_bytes);
-    PIML_CUDA(cub::DeviceRadixSort::SortPairs(l.temp, temp_bytes, keys, vals, N, 0, 32, st));
-    count_launch(cub_sort_launches(N, 32));
-    mlapm_prep_cull_kernel<<<static_cast<unsigned>(T), MS_BLOCK, 0, st>>>(
-        p2, v2, d2, vals.Current(), N, l.rec, l.slot, reinterpret_cast<ulonglong2 *>(l.acc), l.bad, l.cbox, l.cflag,
-        l.rbox, l.rflag, l.bbox, l.bflag);
-    count_launch();
-    rc_ = check_launch("mlapm_prep_cull_kernel");
+    int rc_ = check_launch("mlapm_cull_order_kernel");
     if (rc_) return rc_;
     const int iT = static_cast<int>(T), iD = static_cast<int>(D);
     const CullKeep keep{l.rbox, l.bbox, l.rflag, l.bflag, iT, iD, rc};
     const int ncand = static_cast<int>(cull_candidates(N));
     cub::CountingInputIterator<int> cand(0);
-    need = 0;
+    size_t need = 0;
     PIML_CUDA(cub::DeviceSelect::If(nullptr, need, cand, l.items, l.nitems, ncand, keep, st));
     PIML_REQUIRE(static_cast<int64_t>(need) <= l.temp_bytes,
                  "piml_mlapm: CUB select needs %lld bytes of scratch, %lld reserved", static_cast<long long>(need),
                  static_cast<long long>(l.temp_bytes));
-    temp_bytes = static_cast<size_t>(l.temp_bytes);
+    size_t temp_bytes = static_cast<size_t>(l.temp_bytes);
     PIML_CUDA(cub::DeviceSelect::If(l.temp, temp_bytes, cand, l.items, l.nitems, ncand, keep, st));
     count_launch(2);                                              // tile-state init + select
     // the list's length stays on the device: a fixed grid strides over it, and the scan runs over every candidate
     // (MaskCount is 0 past the list's end), so uoff[n] = W, the live units
-    mlapm_cull_masks_kernel<<<static_cast<unsigned>(4 * sm_count()), threads, 0, st>>>(
+    mlapm_cull_masks_kernel<<<static_cast<unsigned>(4 * sm_count()), 256, 0, st>>>(
         l.items, l.nitems, l.rbox, l.rflag, l.cbox, l.cflag, iT, iD, rc, l.masks);
     count_launch();
     rc_ = check_launch("mlapm_cull_masks_kernel");
@@ -1758,9 +1967,16 @@ static int mlapm_advance_impl(const float *pos, const float *vel, const float *d
         partial = partial4;
     }
     const int threads = 256;
-    mlapm_finalize2_kernel<<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0, st>>>(
-        p2, v2, desired_speed, ds_dim, d2, r0, r1, nsplit, partial, prm->A, k.cos_t, k.sin_t, prm->version, prm->tau,
-        dt, radius, reinterpret_cast<float2 *>(action), reinterpret_cast<float2 *>(pos_new), arrived, push, symp);
+    float2 *a2 = reinterpret_cast<float2 *>(action), *q2 = reinterpret_cast<float2 *>(pos_new);
+    if (nsplit == 0)
+        mlapm_finalize2_kernel<1><<<static_cast<unsigned>((nrows + threads - 1) / threads), threads, 0, st>>>(
+            p2, v2, desired_speed, ds_dim, d2, r0, r1, nsplit, partial, prm->A, k.cos_t, k.sin_t, prm->version,
+            prm->tau, dt, radius, a2, q2, arrived, push, symp);
+    else
+        mlapm_finalize2_kernel<FZ_LPR><<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0,
+                                         st>>>(
+            p2, v2, desired_speed, ds_dim, d2, r0, r1, nsplit, partial, prm->A, k.cos_t, k.sin_t, prm->version,
+            prm->tau, dt, radius, a2, q2, arrived, push, symp);
     count_launch();
     return check_launch("mlapm_finalize2_kernel");
 }
@@ -1987,8 +2203,8 @@ extern "C" int piml_mlapm_sym_finalize_push_f32(const float *pos, const float *v
     SymPartials symp{nullptr, 0.f, static_cast<int>(pl.nI * MS_BLOCK), reinterpret_cast<const float4 *>(inbox_local),
                      world, sym_inbox_stride(N, world)};
     const int threads = 256;
-    mlapm_finalize2_kernel<<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0,
-                             static_cast<cudaStream_t>(stream)>>>(
+    mlapm_finalize2_kernel<FZ_LPR><<<static_cast<unsigned>((nrows * FZ_LPR + threads - 1) / threads), threads, 0,
+                                     static_cast<cudaStream_t>(stream)>>>(
         reinterpret_cast<const float2 *>(pos), reinterpret_cast<const float2 *>(vel), desired_speed, ds_dim,
         reinterpret_cast<const float2 *>(dest), static_cast<int>(row0), static_cast<int>(row1), pl.l.S, pl.l.partialR,
         prm->A, k.cos_t, k.sin_t, prm->version, prm->tau, dt, radius, nullptr, nullptr, arrived, push, symp);

@@ -73,7 +73,7 @@ class MLAPM:
         r0, r1 = rows if rows is not None else (0, N)
         action = torch.empty(r1 - r0, 2, dtype=torch.float32, device=dev)
         pnew = torch.empty(r1 - r0, 2, dtype=torch.float32, device=dev)
-        arrived = torch.empty(r1 - r0, dtype=torch.uint8, device=dev)
+        arrived = torch.empty(r1 - r0, dtype=torch.bool, device=dev)   # the kernel stores bytes 0 / 1
         prm = self._params()
         ws = self._workspace(N, dev, whole_crowd=(r0 == 0 and r1 == N))
         L.check(L.load().piml_mlapm_advance_ws_f32(L.ptr(pos), L.ptr(vel), L.ptr(ds), ds.shape[1], L.ptr(dest), N, r0,
@@ -81,8 +81,8 @@ class MLAPM:
                                                    L.ptr(pnew), L.ptr(arrived), L.ptr(ws), ws.numel(),
                                                    L.stream_ptr(dev)), "piml_mlapm_advance_ws_f32")
         if origin != dev:
-            return action.to(origin), pnew.to(origin), arrived.bool().to(origin)
-        return action, pnew, arrived.bool()
+            return action.to(origin), pnew.to(origin), arrived.to(origin)
+        return action, pnew, arrived
 
     def advance_scenes(self, position, velocity, desired_speed, destination, active, dt, radius=0.3, params=None):
         """`advance` for S independent scenes in one launch.  position, velocity, destination [S,N,2]; desired_speed

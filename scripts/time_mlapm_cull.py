@@ -32,10 +32,8 @@ def algo(a):
 
 
 def groups(name):
-    if "cull_keys" in name or "RadixSort" in name:
-        return "keys + sort"
-    if "prep_cull" in name:
-        return "prep + boxes"
+    if "cull_order" in name:
+        return "order + prep + boxes"
     if ("Select" in name or "Compact" in name or "Scan" in name or "InitKernel" in name
             or "cull_masks" in name):
         return "list build"
