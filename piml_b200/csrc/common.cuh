@@ -96,6 +96,15 @@ __device__ __forceinline__ void tma_bulk_g2s(void *dst_smem, const void *src_gme
                  : "memory");
 }
 
+// One thread's asynchronous 16 B global -> shared copy (cp.async, L2 only; both addresses 16 B aligned), completed by
+// cp_async_wait<k> (k = commit groups left in flight) followed by a barrier between the threads that read it.
+__device__ __forceinline__ void cp_async16(void *dst_smem, const void *src_gmem) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int K>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(K) : "memory"); }
+
 // Stage `n` 8-byte elements (float2) from gmem into smem.  Called by ALL threads of the CTA with identical
 // arguments.  If `src` is 16B aligned one elected thread issues a TMA bulk copy that completes on `bar` (and copies
 // an odd trailing element by hand); otherwise the CTA copies cooperatively.  Returns true if the consumer must wait

@@ -774,13 +774,17 @@ __global__ void __launch_bounds__(MS_BLOCK / (2 * RPS)) mlapm_sym_kernel(const f
 // of a 512-block live close together, then records in sorted order plus an axis-aligned box per 512-agent block, per
 // 128-agent row tile and per 32-agent column tile; (3) the work list: every (row tile R of
 // block I, column block J = I + d mod T) item of the circulant schedule whose boxes are within r_cut, compacted in
-// order (cub::DeviceSelect), the mask of its column tiles within r_cut, and the exclusive scan of the masks' popcounts
-// (cub::DeviceScan): the live (row tile, column tile) units; (4) a persistent pair kernel over the units; (5) the
-// finalize kernel reads each agent's sums through its sorted slot.  Row and column directions both go into the
-// crowd-wide int64 fixed-point accumulators, so the result does not depend on how the units are cut over the CTAs.
+// order (cub::DeviceSelect), the mask of its column tiles within r_cut and its unit count, and the exclusive scan of
+// the counts (cub::DeviceScan); (4) a persistent pair kernel over the units; (5) the finalize kernel reads each agent's
+// sums through its sorted slot.  Row and column directions both go into the crowd-wide int64 fixed-point accumulators,
+// so the result does not depend on how the units are cut over the CTAs.
 // Every unordered pair once: d >= 1 takes the 16 column tiles of block J in both directions; d = 0 takes the column
 // tiles of the row tiles r' > r of the own block in both directions and the row tile's own 4 column tiles in the row
 // direction only (every ordered pair of the row tile appears there); r' < r belongs to row tile r'.
+// A unit is the row tile against 32 column slots.  An own column tile is one unit.  The other column tiles of an item
+// are packed: their live columns (cull_col_live: within r_cut of the row tile's box), in list order, fill units of 32,
+// the item's last one padded with a far record.  Units stay a uniform amount of work, so the CTAs' equal unit counts
+// stay balanced; dropping the dead columns inside units instead would leave the busiest CTA as busy as before.
 // =====================================================================================================================
 constexpr int MC_RT = 128;                        // rows per row tile
 constexpr int MC_CT = 32;                         // columns per column tile: one warp of the order kernel, 1 KB
@@ -1119,7 +1123,20 @@ struct CullItem {
     }
     // first column tile of block J that the item covers: d = 0 skips the row tiles r' < r of the own block
     __device__ __forceinline__ int first_tile() const { return d == 0 ? (R % MC_RPB) * (MC_CPB / MC_RPB) : 0; }
+    // the row tile's own column tiles (d = 0), evaluated in the row direction only: the lowest tiles the item covers
+    __device__ __forceinline__ unsigned own_tiles() const {
+        return d == 0 ? ((1u << (MC_CPB / MC_RPB)) - 1u) << first_tile() : 0u;
+    }
 };
+
+// Whether column slot j, record pv = {px,py,vx,vy}, may have a pair within rc with the row tile of box a, flag fa: the
+// point against the box, rounded down as in cull_near.  A non-finite position or velocity gives the column's pairs a
+// NaN weight, not 0, so such a column is always live; padding slots (j >= N) never are.
+__device__ __forceinline__ bool cull_col_live(float4 pv, int j, int N, float4 a, unsigned fa, float rc) {
+    if (j >= N) return false;
+    const bool finite = isfinite(pv.x) && isfinite(pv.y) && isfinite(pv.z) && isfinite(pv.w);
+    return cull_near(a, fa, make_float4(pv.x, pv.y, pv.x, pv.y), finite ? 0u : MC_NEAR_ALL, rc);
+}
 
 // Keep-predicate of the work list: the row tile's box within r_cut of block J's box (circulant schedule of
 // mlapm_sym_kernel; for even T the pairs at d = T/2 belong to I < T/2).
@@ -1136,89 +1153,156 @@ struct CullKeep {
 };
 
 // masks[i] = the column tiles of block J that list item i evaluates: within r_cut of the row tile's box and allowed by
-// the d = 0 rule.  Grid-stride over the n = *nitems items (read on the device).
+// the d = 0 rule; units[i] = its units: one per own column tile, and its other tiles' live columns in units of 32
+// (rounded up).  One warp per item, lane = column tile for the mask and column for the liveness ballots; grid-stride
+// over the n = *nitems items (read on the device).
 __global__ void mlapm_cull_masks_kernel(const int *__restrict__ items, const int *__restrict__ nitems,
-                                        const float4 *__restrict__ rbox, const unsigned *__restrict__ rflag,
-                                        const float4 *__restrict__ cbox, const unsigned *__restrict__ cflag, int T,
-                                        int D, float rc, uint16_t *__restrict__ masks) {
-    const int n = *nitems;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+                                        const float4 *__restrict__ rec, int N, const float4 *__restrict__ rbox,
+                                        const unsigned *__restrict__ rflag, const float4 *__restrict__ cbox,
+                                        const unsigned *__restrict__ cflag, int T, int D, float rc,
+                                        uint16_t *__restrict__ masks, uint8_t *__restrict__ units) {
+    const int n = *nitems, lane = threadIdx.x & 31;
+    const int w0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = (gridDim.x * blockDim.x) >> 5;
+    for (int i = w0; i < n; i += nw) {
         const CullItem it(items[i], T, D);
         const float4 a = rbox[it.R];
         const unsigned fa = rflag[it.R];
-        unsigned m = 0;
-        for (int ct = it.first_tile(); ct < MC_CPB; ++ct) {
-            const int s = it.J * MC_CPB + ct;
-            if (cull_near(a, fa, cbox[s], cflag[s], rc)) m |= 1u << ct;
+        const int s = it.J * MC_CPB + lane;
+        const unsigned m = __ballot_sync(0xffffffffu, lane >= it.first_tile() && lane < MC_CPB &&
+                                                          cull_near(a, fa, cbox[s], cflag[s], rc));
+        const unsigned own = m & it.own_tiles();
+        int live = 0;
+#pragma unroll
+        for (int ct = 0; ct < MC_CPB; ++ct) {
+            if (!((m & ~own) >> ct & 1u)) continue;
+            const int j = it.J * MS_BLOCK + ct * MC_CT + lane;
+            live += __popc(__ballot_sync(0xffffffffu, cull_col_live(rec[2 * j], j, N, a, fa, rc)));
         }
-        masks[i] = static_cast<uint16_t>(m);
+        if (lane == 0) {
+            masks[i] = static_cast<uint16_t>(m);
+            units[i] = static_cast<uint8_t>(__popc(own) + (live + MC_CT - 1) / MC_CT);
+        }
     }
 }
 
-// Live units of item i for the scan: popcount of its mask; 0 past the end of the list.
-struct MaskCount {
-    const uint16_t *masks;
+// Units of item i for the scan; 0 past the end of the list.
+struct UnitCount {
+    const uint8_t *units;
     const int *nitems;
-    __device__ __forceinline__ long long operator()(int i) const { return i < *nitems ? __popc(masks[i]) : 0; }
+    __device__ __forceinline__ long long operator()(int i) const { return i < *nitems ? units[i] : 0; }
 };
 
-// The symmetric pair kernel over the live units.  Persistent, one warp per CTA: CTA b takes the units
-// [b W / G, (b+1) W / G) of the W = uoff[n] on the list (read on the device: no host sync), finds the item of its first
-// unit by binary search in the scan and walks the masks from there.  A unit is one 1 KB column tile, staged by a TMA
-// bulk copy (double buffered) and evaluated against the warp's 128 rows by the dense kernel's bodies (ms_pair_tile,
-// ms_diag_tile); each column's warp sum goes straight into the fixed-point accumulators.  Rows stay in registers while
-// consecutive units share the row tile; when it changes, and at the end, the row sums go into the same accumulators
-// with the opposite sign of the column shares (acc = column share - row share; the finalize kernel subtracts acc).
+// The symmetric pair kernel over the units.  Persistent, one warp per CTA: CTA b takes the units [b W / G, (b+1) W / G)
+// of the W = uoff[n] on the list (read on the device: no host sync) and finds the item of its first unit by binary
+// search in the scan.  It walks the list with a cursor: an own column tile is staged whole; a packed unit walks the
+// item's remaining column tiles, one column per lane, repeats the masks kernel's liveness test with a ballot and takes
+// the live columns in order until it has 32 or the item ends (short: the rest are far padding records).  Each lane
+// copies one 32 B record into the unit's stage with cp.async, one unit ahead of the compute (double buffered), and the
+// unit's column slots go beside it.  The stage runs through the dense kernel's bodies (ms_pair_tile, ms_diag_tile);
+// each column's warp sum goes straight into its slot's fixed-point accumulators (none for padding).  Rows stay in
+// registers while consecutive units share the row tile; when it changes, and at the end, the row sums go into the same
+// accumulators with the opposite sign of the column shares (acc = column share - row share; the finalize kernel
+// subtracts acc).
 template <int VERSION>
 __global__ void __launch_bounds__(MC_THREADS, 16) mlapm_sym_tiles_kernel(
-    const float4 *__restrict__ rec, const int *__restrict__ items, const int *__restrict__ nitems,
-    const uint16_t *__restrict__ masks, const long long *__restrict__ uoff, int T, int D, M2Const k,
+    const float4 *__restrict__ rec, int N, const int *__restrict__ items, const int *__restrict__ nitems,
+    const uint16_t *__restrict__ masks, const uint8_t *__restrict__ units, const long long *__restrict__ uoff,
+    const float4 *__restrict__ rbox, const unsigned *__restrict__ rflag, float rc, int T, int D, M2Const k,
     unsigned long long *__restrict__ acc, unsigned *__restrict__ bad, float colscale) {
     constexpr int RPS = MC_RT / (2 * MC_THREADS);
-    constexpr uint32_t TILE_BYTES = MC_CT * MS_RECF * sizeof(float);
+    static_assert(MC_CT == MC_THREADS, "one column slot per lane");
     __shared__ __align__(128) float4 tile[2][MC_CT * 2];
+    __shared__ int cols[2][MC_CT];
     __shared__ __align__(16) float4 red[MS_BATCH * MS_RED_STRIDE];
-    __shared__ __align__(8) uint64_t bars[2];
     const int lane = threadIdx.x;
+    const unsigned below = (1u << lane) - 1u;
     const int n = *nitems;
     const long long W = uoff[n];
     const long long u0 = W * blockIdx.x / gridDim.x, u1 = W * (blockIdx.x + 1) / gridDim.x;
     if (u1 <= u0) return;
-    int lo = 0, hi = n;                                        // uoff[lo] <= u0 < uoff[hi]
-    while (hi - lo > 1) {
-        const int mid = (lo + hi) >> 1;
-        if (uoff[mid] <= u0) lo = mid;
+    int item = 0, hi = n;                                      // uoff[item] <= u0 < uoff[hi]
+    while (hi - item > 1) {
+        const int mid = (item + hi) >> 1;
+        if (uoff[mid] <= u0) item = mid;
         else hi = mid;
     }
-    int item = lo;
-    unsigned mask = masks[item];
-    for (long long s = u0 - uoff[item]; s > 0; --s) mask &= mask - 1;
-    // the next unit in list order: row tile R, first column slot j0, whether it is one of the row tile's own tiles
-    auto next_unit = [&](int &R, int &j0, bool &diag) {
-        while (mask == 0) mask = masks[++item];
-        const int ct = __ffs(mask) - 1;
-        mask &= mask - 1;
-        const CullItem it(items[item], T, D);
+    // cursor: the item's row tile R and column block J, its column tiles not yet started (own: those that are own
+    // tiles), its packed units not yet formed, and the live columns of the last started tile not yet taken (slots
+    // jt + their bits)
+    int R, J, pk, jt = 0;
+    unsigned mask, own, live;
+    auto open = [&](int i) {
+        const CullItem it(items[i], T, D);
         R = it.R;
-        j0 = it.J * MS_BLOCK + ct * MC_CT;
-        diag = it.d == 0 && ct / (MC_CPB / MC_RPB) == it.R % MC_RPB;
+        J = it.J;
+        mask = masks[i];
+        own = mask & it.own_tiles();
+        pk = units[i] - __popc(own);
+        live = 0u;
     };
-    auto stage = [&](int j0, int buf) {
-        if (lane == 0) {
-            mbar_expect_tx(&bars[buf], TILE_BYTES);
-            tma_bulk_g2s(tile[buf], rec + static_cast<int64_t>(j0) * 2, TILE_BYTES, &bars[buf]);
+    // takes up to `want` live columns of the item's packed tiles in list order and returns how many; buf >= 0: the
+    // p-th of them goes to slot got + p of stage buf
+    auto take = [&](int want, int buf, int got) {
+        const float4 a = rbox[R];
+        const unsigned fa = rflag[R];
+        int taken = 0;
+        while (taken < want) {
+            if (live == 0u) {
+                if (mask == 0u) break;
+                jt = J * MS_BLOCK + (__ffs(mask) - 1) * MC_CT;
+                mask &= mask - 1u;
+                live = __ballot_sync(0xffffffffu, cull_col_live(rec[2 * (jt + lane)], jt + lane, N, a, fa, rc));
+                continue;
+            }
+            const bool mine = (live >> lane) & 1u;
+            const int rank = __popc(live & below), c = min(__popc(live), want - taken);
+            if (buf >= 0 && mine && rank < c) {
+                const int p = got + taken + rank;
+                const float4 *src = rec + 2 * static_cast<int64_t>(jt + lane);
+                cp_async16(&tile[buf][2 * p], src);
+                cp_async16(&tile[buf][2 * p + 1], src + 1);
+                cols[buf][p] = jt + lane;
+            }
+            live = __ballot_sync(0xffffffffu, mine && rank >= c);
+            taken += c;
+        }
+        return taken;
+    };
+    // the next unit into stage buf: its row tile Ru, whether it is an own tile
+    auto next_unit = [&](int buf, int &Ru, bool &diag) {
+        while (own == 0u && pk == 0) open(++item);
+        Ru = R;
+        diag = own != 0u;
+        if (diag) {
+            const int ct = __ffs(own) - 1;
+            own &= own - 1u;
+            mask &= ~(1u << ct);
+            const float4 *src = rec + 2 * (static_cast<int64_t>(J) * MS_BLOCK + ct * MC_CT + lane);
+            cp_async16(&tile[buf][2 * lane], src);
+            cp_async16(&tile[buf][2 * lane + 1], src + 1);
+        } else {
+            --pk;
+            if (lane >= take(MC_CT, buf, 0)) {
+                tile[buf][2 * lane] = make_float4(MS_FAR, MS_FAR, 0.f, 0.f);     // weight exactly 0 both ways
+                tile[buf][2 * lane + 1] = make_float4(0.f, 0.f, 0.f, 0.f);
+                cols[buf][lane] = -1;
+            }
         }
     };
-    if (lane == 0) {
-        mbar_init(&bars[0], 1);
-        mbar_init(&bars[1], 1);
-        mbar_fence_init();
+    // skip the s units of the item before u0: own tiles first, then 32 live columns per packed unit
+    open(item);
+    int s = static_cast<int>(u0 - uoff[item]);
+    for (; s > 0 && own != 0u; --s) {
+        mask &= ~(own & (0u - own));
+        own &= own - 1u;
     }
-    __syncwarp();
-    int R, j0;
+    pk -= s;
+    take(s * MC_CT, -1, 0);
+
+    int R0;
     bool diag;
-    next_unit(R, j0, diag);
-    stage(j0, 0);
+    next_unit(0, R0, diag);
+    cp_async_commit();
 
     MsRows<RPS> rw;
     const float2 Bl = splat(k.Bl), Cl = splat(k.Cl), Dl = splat(k.Dl);
@@ -1242,29 +1326,30 @@ __global__ void __launch_bounds__(MC_THREADS, 16) mlapm_sym_tiles_kernel(
     int Rrun = -1;
     for (int t = 0; t < cnt; ++t) {
         const int buf = t & 1;
-        int Rn = 0, jn = 0;
+        int Rn = 0;
         bool dn = false;
-        if (t + 1 < cnt) {                                     // tile[buf^1] was released by the __syncwarp below
-            next_unit(Rn, jn, dn);
-            stage(jn, buf ^ 1);
-        }
-        if (R != Rrun) {
+        if (t + 1 < cnt) next_unit(buf ^ 1, Rn, dn);           // stage buf^1 was released by the __syncwarp below
+        cp_async_commit();
+        if (R0 != Rrun) {
             if (Rrun >= 0) flush_rows(Rrun);
-            ms_load_rows<RPS, MC_THREADS>(rw, rec, static_cast<int64_t>(R) * MC_RT, lane);
-            Rrun = R;
+            ms_load_rows<RPS, MC_THREADS>(rw, rec, static_cast<int64_t>(R0) * MC_RT, lane);
+            Rrun = R0;
         }
-        mbar_wait(&bars[buf], (t >> 1) & 1);                   // the (t/2)-th use of this buffer
+        cp_async_wait<1>();                                    // this unit's copies; the next unit's stay in flight
+        __syncwarp();
         // the off-diagonal branch first: in the other order ptxas emits the diagonal loop twice
         if (!diag) {
-            const int64_t jc = j0;
+            const int *cl = cols[buf];
             ms_pair_tile<VERSION, RPS, MC_CT>(rw, tile[buf], red, lane, Bl, Cl, Dl, [&](int c, float4 a) {
-                add(jc + c, a.x, a.y, a.z, a.w, colscale);
+                const int j = cl[c];
+                if (j >= 0) add(j, a.x, a.y, a.z, a.w, colscale);
             });
         } else {
             ms_diag_tile<VERSION, RPS, MC_CT>(rw, tile[buf], Bl, Cl, Dl);
         }
         __syncwarp();
-        R = Rn; j0 = jn; diag = dn;
+        R0 = Rn;
+        diag = dn;
     }
     flush_rows(Rrun);
 }
@@ -1656,12 +1741,12 @@ static int64_t cull_cub_bound(int64_t N) { return (int64_t{1} << 16) + cull_cand
 struct CullLayout {
     float4 *rec; long long *acc; unsigned *bad; uint32_t *key[2]; int *val, *perm, *rank, *cnt, *dtotal, *slot;
     float4 *cta_box, *cbox, *rbox, *bbox; unsigned *cflag, *rflag, *bflag; int *items, *nitems; uint16_t *masks;
-    long long *uoff; void *temp; int64_t temp_bytes, total;
+    uint8_t *units; long long *uoff; void *temp; int64_t temp_bytes, total;
 };
 // records, accumulators (4 x int64) and flags per padded agent; the order kernel's keys (two), agents (two), ranks
 // and slots per agent, its bin counts per (bin, CTA) and totals per bin, and a box per CTA (at most one per block);
-// boxes and flags per column tile, row tile and block; the work list, its masks and the scan of their popcounts (14 B
-// per candidate); CUB's scratch.  0.2 GB at N = 10^6.
+// boxes and flags per column tile, row tile and block; the work list, its masks, unit counts and their scan (15 B per
+// candidate); CUB's scratch.  0.2 GB at N = 10^6.
 static CullLayout cull_layout(int64_t N, void *base) {
     const int64_t T = sym_blocks(N), npad = T * MS_BLOCK;
     CullLayout l{};
@@ -1686,6 +1771,7 @@ static CullLayout cull_layout(int64_t N, void *base) {
     l.items = static_cast<int *>(c.take(cull_candidates(N) * sizeof(int)));
     l.nitems = static_cast<int *>(c.take(sizeof(int)));
     l.masks = static_cast<uint16_t *>(c.take(cull_candidates(N) * sizeof(uint16_t)));
+    l.units = static_cast<uint8_t *>(c.take(cull_candidates(N) * sizeof(uint8_t)));
     l.uoff = static_cast<long long *>(c.take((cull_candidates(N) + 1) * sizeof(long long)));
     l.temp_bytes = cull_cub_bound(N);
     l.temp = c.take(l.temp_bytes);
@@ -1829,13 +1915,14 @@ static int launch_sym_culled(int version, const float2 *p2, const float2 *v2, co
     PIML_CUDA(cub::DeviceSelect::If(l.temp, temp_bytes, cand, l.items, l.nitems, ncand, keep, st));
     count_launch(2);                                              // tile-state init + select
     // the list's length stays on the device: a fixed grid strides over it, and the scan runs over every candidate
-    // (MaskCount is 0 past the list's end), so uoff[n] = W, the live units
-    mlapm_cull_masks_kernel<<<static_cast<unsigned>(4 * sm_count()), 256, 0, st>>>(
-        l.items, l.nitems, l.rbox, l.rflag, l.cbox, l.cflag, iT, iD, rc, l.masks);
+    // (UnitCount is 0 past the list's end), so uoff[n] = W, the units
+    mlapm_cull_masks_kernel<<<static_cast<unsigned>(8 * sm_count()), 256, 0, st>>>(
+        l.items, l.nitems, l.rec, N, l.rbox, l.rflag, l.cbox, l.cflag, iT, iD, rc, l.masks, l.units);
     count_launch();
     rc_ = check_launch("mlapm_cull_masks_kernel");
     if (rc_) return rc_;
-    const auto counts = thrust::make_transform_iterator(thrust::counting_iterator<int>(0), MaskCount{l.masks, l.nitems});
+    const auto counts =
+        thrust::make_transform_iterator(thrust::counting_iterator<int>(0), UnitCount{l.units, l.nitems});
     need = 0;
     PIML_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, need, counts, l.uoff, ncand + 1, st));
     PIML_REQUIRE(static_cast<int64_t>(need) <= l.temp_bytes,
@@ -1861,10 +1948,10 @@ static int launch_sym_culled(int version, const float2 *p2, const float2 *v2, co
     unsigned long long *acc = reinterpret_cast<unsigned long long *>(l.acc);
     if (version == 0)
         mlapm_sym_tiles_kernel<0><<<static_cast<unsigned>(grid), MC_THREADS, 0, st>>>(
-            l.rec, l.items, l.nitems, l.masks, l.uoff, iT, iD, k2, acc, l.bad, colscale);
+            l.rec, N, l.items, l.nitems, l.masks, l.units, l.uoff, l.rbox, l.rflag, rc, iT, iD, k2, acc, l.bad, colscale);
     else
         mlapm_sym_tiles_kernel<1><<<static_cast<unsigned>(grid), MC_THREADS, 0, st>>>(
-            l.rec, l.items, l.nitems, l.masks, l.uoff, iT, iD, k2, acc, l.bad, colscale);
+            l.rec, N, l.items, l.nitems, l.masks, l.units, l.uoff, l.rbox, l.rflag, rc, iT, iD, k2, acc, l.bad, colscale);
     count_launch();
     return check_launch("mlapm_sym_tiles_kernel");
 }

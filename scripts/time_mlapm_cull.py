@@ -4,9 +4,10 @@
 
 Per size: culled (algorithm 2) and dense (algorithm 3) steps alternate in one process, `rounds` x `steps` each, with
 a 160 MB L2 flush before every step outside its CUDA-event pair; min / median / max ms per step.  The dense arm at
-N >= 10^6 runs one step per round (about 0.7 s each).  Then the live units, the evaluated pairs and their rate
-against the dense kernel's, a torch.profiler run for the per-kernel split (written under --out), and 50 consecutive
-culled steps on the moving crowd.
+N >= 10^6 runs one step per round (about 0.7 s each).  Then the units W, the pair slots they evaluate and their
+rate against the dense kernel's, a torch.profiler run for the per-kernel split (written under --out), and 50
+consecutive culled steps on the moving crowd.  A unit is one 128-row tile against 32 column slots; a packed unit's
+last slots may be padding (not known on the host), so the slot pairs bound the live pairs from above.
 """
 import argparse
 import ctypes as C
@@ -24,7 +25,7 @@ import bench  # noqa: E402
 import piml_b200 as P  # noqa: E402
 from piml_b200 import _lib as L  # noqa: E402
 
-UNIT_PAIRS = 128 * 32            # (row tile, column tile) unit
+UNIT_PAIRS = 128 * 32            # (row tile, 32 column slots) unit
 
 
 def algo(a):
@@ -92,7 +93,7 @@ def main():
             ms["dense"] += run(3, dense_steps)
         res = {k: {"min": min(t), "median": statistics.median(t), "max": max(t), "n": len(t)} for k, t in ms.items()}
         res["speedup_median"] = res["dense"]["median"] / res["culled"]["median"]
-        # live units of the culled step on the bench crowd
+        # units of the culled step on the bench crowd
         run(2, 1)
         units = C.c_int64()
         L.check(L.load().piml_mlapm_cull_items(L.ptr(model._ws), N, C.byref(units)), "piml_mlapm_cull_items")
@@ -102,8 +103,8 @@ def main():
         off = units.value - diag
         ordered = off * 2 * UNIT_PAIRS + diag * UNIT_PAIRS
         res.update({"units": units.value, "unit_candidates": cand, "unit_share": units.value / cand,
-                    "unordered_pairs_evaluated": off * UNIT_PAIRS + diag * UNIT_PAIRS // 2,
-                    "ordered_pair_equivalents": ordered})
+                    "unordered_slot_pairs_evaluated": off * UNIT_PAIRS + diag * UNIT_PAIRS // 2,
+                    "ordered_slot_pair_equivalents": ordered})
         # per-kernel split (a separate, traced run)
         prof_steps = 5
         with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
@@ -124,9 +125,9 @@ def main():
         t_pair = split.get("pair kernel (culled)", {}).get("us_per_step")
         t_dense = split.get("pair kernel (dense)", {}).get("us_per_step")
         if t_pair and t_dense:
-            res["ordered_pairs_per_s_culled"] = ordered / (t_pair * 1e-6)
+            res["ordered_slot_pairs_per_s_culled"] = ordered / (t_pair * 1e-6)
             res["ordered_pairs_per_s_dense"] = float(N) * N / (t_dense * 1e-6)
-            res["rate_ratio"] = res["ordered_pairs_per_s_culled"] / res["ordered_pairs_per_s_dense"]
+            res["rate_ratio"] = res["ordered_slot_pairs_per_s_culled"] / res["ordered_pairs_per_s_dense"]
         prof.export_chrome_trace(os.path.join(a.out, f"cull_N{N}.pt.trace.json"))
         # 50 consecutive culled steps on the moving crowd
         run_ms = run(2, 50, state=[p.clone(), v.clone()])
